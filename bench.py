@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the self-play hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): raw env throughput, 65536 lockstep 2-player games per
 GPU, uniform-random legal moves, finished games re-dealt in place.  One bench "step" = one
@@ -26,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only: the benchmark writes nothing into it
 
 ENV_BYTES_PER_STEP = 330      # SURVEY.md §8d: 2 x 160 B State image + 8 B mask + 1 B action + 1 B status
 SEED = 0x5EED0001
@@ -552,6 +553,24 @@ def run_train(args, api, torch, local):
                                     "copied out inside the timed region" % (n, args.blocks)})
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, env, cnt, stream):
+    """What the timed rollouts leave a caller: the 160-byte State image of every game (az_env_export_aos) and the counters of the
+    timed steps, as float arrays (bytes and counts are exact in float32 / float64).  When the images exceed DUMP_BYTES, a fixed
+    seeded sample of the games is written; game_ids.npy names the rows either way."""
+    import numpy as np
+    img = env.export_aos(stream=stream)
+    rows = min(env.n, (DUMP_BYTES - 4096) // (img.shape[1] * 4 + 8))       # 4 KB: the three .npy headers and the counters
+    ids = np.arange(env.n) if rows == env.n else np.sort(np.random.default_rng(SEED).choice(env.n, rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "state_images.npy"), img[ids].astype(np.float32))
+    np.save(os.path.join(out_dir, "game_ids.npy"), ids.astype(np.float64))
+    np.save(os.path.join(out_dir, "counters.npy"),
+            np.array([cnt["steps"], cnt["games"], cnt["wins"][0], cnt["wins"][1], cnt["draws"], cnt["illegal"]], np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -586,11 +605,6 @@ def run_ours(args):
     env.reset(SEED, stream=sptr)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")     # > 126 MB L2
 
-    for _ in range(args.warmup):
-        env.rollout(S, stream=sptr)
-    torch.cuda.synchronize()
-    env.counters(reset=True, stream=sptr)
-
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -600,7 +614,12 @@ def run_ours(args):
         while len(sampler.lines) < 3 and time.perf_counter() - t_lead < 3.0:
             env.rollout(S, stream=sptr)
             torch.cuda.synchronize()
-        env.counters(reset=True, stream=sptr)
+    # the lead-in ran a time-dependent number of moves: deal again, so that every run with the same arguments times the same games
+    env.reset(SEED, stream=sptr)
+    for _ in range(args.warmup):
+        env.rollout(S, stream=sptr)
+    torch.cuda.synchronize()
+    env.counters(reset=True, stream=sptr)
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     barrier()
     t_wall0 = time.perf_counter()
@@ -615,6 +634,8 @@ def run_ours(args):
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     cnt = env.counters(stream=sptr)
     assert cnt["steps"] == n * S * args.steps, cnt
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, cnt, sptr)
 
     # ---- e2e: host State images in pinned memory -> device -> rollout -> host, every step.  The public calls are synchronous
     # (az_env_import_aos / az_env_rollout / az_env_export_aos return when the data is there), so a host that wants the copies of one
@@ -761,7 +782,9 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed rollout launches of the headline line; its e2e sub-line times max(3, min(K, 10)) steps and the self-play "
+                         "sub-line max(2, min(K, --sp-steps))")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--games", type=int, default=65536)
@@ -783,7 +806,11 @@ def main():
     ap.add_argument("--no-blocks20", dest="blocks20", action="store_false", help="skip the 20-block (CMake default graph) sub-line")
     ap.add_argument("--train-batch", type=int, default=512, help="training-step measurement batch (SETTINGS.BATCH_SIZE); 0 skips it")
     ap.add_argument("--play-games", type=int, default=1000, help="configs[0] match size (--cg); 0 skips it")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write rank 0's game State images and the counters "
+                                                          "of the timed steps to DIR/*.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -2,6 +2,7 @@
 // Without a GPU: constructing the service must fail loudly (no CPU fallback) -> prints NO_DEVICE_OK.
 // With a GPU: 16 threads call registerThread / predictFuture concurrently like the reference's search threads;
 // every future must equal a direct az_nn_forward of the same input -> prints SERVICE_OK <batches>.
+// Usage: test_nn_service [DIR]; with a GPU, DIR (required) receives the checkpoints the test writes.
 #include <atomic>
 #include <cmath>
 #include <cstdio>
@@ -22,7 +23,7 @@ static NNInputData make_input(unsigned k)
     return in;
 }
 
-int main()
+int main(int argc, char** argv)
 {
     static_assert(sizeof(NNInputData) == 88, "mirror layout");
     if (az_device_count() == 0) {
@@ -37,10 +38,12 @@ int main()
     bool dup = false;
     try { cluster.initPlayerGroup("az1", "model_bin_V2_2.pb"); } catch (const std::invalid_argument&) { dup = true; }   // upstream behaviour
     if (!dup) { printf("duplicate group accepted\n"); return 1; }
+    if (argc < 2) { printf("usage: %s DIR (the checkpoints the test writes go there)\n", argv[0]); return 2; }
+    const std::string ck = std::string(argv[1]) + "/az_b200_test_ckpt";
     auto nn = group->getNN(0);
-    std::filesystem::remove_all("/tmp/az_b200_test_ckpt");
-    nn->loadCheckpoint("/tmp/az_b200_test_ckpt/az1");          // missing -> random init + save (a TensorFlow checkpoint bundle)
-    if (!std::filesystem::exists("/tmp/az_b200_test_ckpt/az1.index") || !std::filesystem::exists("/tmp/az_b200_test_ckpt/az1.data-00000-of-00001")) {
+    std::filesystem::remove_all(ck);
+    nn->loadCheckpoint(ck + "/az1");          // missing -> random init + save (a TensorFlow checkpoint bundle)
+    if (!std::filesystem::exists(ck + "/az1.index") || !std::filesystem::exists(ck + "/az1.data-00000-of-00001")) {
         printf("checkpoint bundle was not written\n"); return 1; }
     const int T = 16, R = 40;
     std::atomic<int> bad{ 0 };
@@ -75,9 +78,9 @@ int main()
     group->train(data, 2);
     NNOutputData after = nn->predict(probe);
     bool moved = before.value != after.value;
-    group->saveCheckpoint("/tmp/az_b200_test_ckpt/trained");
+    group->saveCheckpoint(ck + "/trained");
     auto group2 = cluster.initPlayerGroup("az2", "model_bin_V2_2.pb");
-    group2->loadCheckpoint("/tmp/az_b200_test_ckpt/trained");
+    group2->loadCheckpoint(ck + "/trained");
     NNOutputData again = group2->getNN(0)->predict(probe);
     bool restored = again.value == after.value;
     for (int i = 0; i < 43; ++i) restored = restored && again.policy[i] == after.policy[i];
@@ -93,7 +96,7 @@ int main()
         Cluster two(AZ_NN_FP32, 2);
         two.initGpus(2);
         auto g2 = two.initPlayerGroup("pair", "model_bin_V2_2.pb");
-        g2->loadCheckpoint("/tmp/az_b200_test_ckpt/az1");
+        g2->loadCheckpoint(ck + "/az1");
         g2->getNN(0)->service().setBatchSize(32);
         g2->train(data, 1);
         NNOutputData p0 = g2->getNN(0)->predict(probe), p1 = g2->getNN(1)->predict(probe);

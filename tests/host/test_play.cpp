@@ -1,14 +1,16 @@
 // Standalone test of alphazero_risk_b200/host/az_play.hpp with a mirror of the reference's GameResults (game/game.h:10-29).
 // Without a GPU: construction must fail loudly -> NO_DEVICE_OK.  With a GPU: a 40-game match (--mcts=16, -t 2) -> PLAY_OK.
+// Usage: test_play [DIR]; with a GPU, DIR (required) receives the checkpoint the test writes.
 #include <cstdio>
 #include <cstring>
+#include <string>
 #include <vector>
 #include "az_play.hpp"
 
 struct PlayerGameResult { int win = 0; int winAndStartedGame = 0; };
 struct GameResults { int count = 0; int draw = 0; std::vector<PlayerGameResult> players = std::vector<PlayerGameResult>(2); };
 
-int main()
+int main(int argc, char** argv)
 {
     azb200::PlaySettings s;
     s.MCTS_SIMULATIONS = 16; s.THREADS_PER_MCTS = 2; s.BLOCKS = 2;
@@ -18,9 +20,11 @@ int main()
         printf("expected a failure without a GPU\n");
         return 1;
     }
+    if (argc < 2) { printf("usage: %s DIR (the checkpoint the test writes goes there)\n", argv[0]); return 2; }
+    const std::string ck = std::string(argv[1]) + "/az_b200_play_ckpt";
     azb200::DevicePlay p(s);
-    remove("/tmp/az_b200_play_ckpt.index"); remove("/tmp/az_b200_play_ckpt.data-00000-of-00001");
-    p.loadCheckpoint("/tmp/az_b200_play_ckpt");            // missing: random init kept and saved as a TensorFlow checkpoint bundle
+    remove((ck + ".index").c_str()); remove((ck + ".data-00000-of-00001").c_str());
+    p.loadCheckpoint(ck);            // missing: random init kept and saved as a TensorFlow checkpoint bundle
     GameResults a = p.playGames<GameResults>(41);          // odd request: 40 games, like Counter::hasNext(2)
     GameResults b = p.playGames<GameResults>(41);          // same seed, same weights: the match is reproducible
     bool ok = a.count == 40 && a.draw + a.players[0].win + a.players[1].win == 40 &&
@@ -29,7 +33,7 @@ int main()
     // the trainer's comparison match: a second DevicePlay holds the "old" model (here the same checkpoint), player index 1 searches
     // with its network and its own tables
     azb200::DevicePlay old(s);
-    old.loadCheckpoint("/tmp/az_b200_play_ckpt");
+    old.loadCheckpoint(ck);
     p.setOpponentNetwork(old.network());
     GameResults c = p.playGames<GameResults>(12);
     ok = ok && c.count == 12 && c.draw + c.players[0].win + c.players[1].win == 12 && p.last.opponent_turns > 0 && p.last.az_moves > 0;

@@ -30,3 +30,32 @@ def test_committed_ncu_numbers_belong_to_the_committed_kernels():
         d, why = bench.ncu_capture(kernel)
         assert d is not None, why
         assert os.path.exists(os.path.join(ROOT, d["capture"])), d["capture"]
+
+
+def test_dump_outputs_samples_a_fixed_set_of_games_above_the_cap(tmp_path, monkeypatch):
+    """--dump-outputs over DUMP_BYTES: a seeded, sorted sample of the games, the same on every call, the files within the cap"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+
+    class Env:
+        n = 4096
+
+        def export_aos(self, stream=None):
+            return (np.arange(self.n * 160) % 251).astype(np.uint8).reshape(self.n, 160)
+
+    cnt = dict(steps=7, games=3, wins=[1, 1], draws=1, illegal=0)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), Env(), cnt, None)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["counters.npy", "game_ids.npy", "state_images.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 1 << 20
+    for f in files:
+        assert (np.load(tmp_path / "a" / f) == np.load(tmp_path / "b" / f)).all(), f
+    ids, img = np.load(tmp_path / "a" / "game_ids.npy"), np.load(tmp_path / "a" / "state_images.npy")
+    assert ids.dtype == np.float64 and img.dtype == np.float32
+    assert 1000 < len(ids) < Env.n and img.shape == (len(ids), 160)
+    assert (np.diff(ids) > 0).all() and ids[0] >= 0 and ids[-1] < Env.n
+    assert (img == Env().export_aos()[ids.astype(int)]).all()
+    assert list(np.load(tmp_path / "a" / "counters.npy")) == [7, 3, 1, 1, 1, 0]

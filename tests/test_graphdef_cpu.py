@@ -16,7 +16,8 @@ from oracle import graphdef_oracle as go
 from oracle import nn_oracle as no
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_PB = "/root/reference/python/model/model_txt_V2_5.pb"
+REF_DIR = os.environ.get("AZ_REFERENCE_DIR")          # a checkout of the original project, as oracle/ref/build_ref.sh reads it
+REF_PB = os.path.join(REF_DIR, "python", "model", "model_txt_V2_5.pb") if REF_DIR else ""
 
 
 @pytest.fixture(scope="module")
@@ -112,7 +113,7 @@ def test_optimizer_wiring_and_constants(sl):
     assert regularised == sorted(n for n in no.variable_names(5) if n.endswith("/kernel")) and len(regularised) == 16
 
 
-@pytest.mark.skipif(not os.path.exists(REF_PB), reason="the reference tree is not present (GPU box)")
+@pytest.mark.skipif(not os.path.exists(REF_PB), reason="AZ_REFERENCE_DIR does not name a checkout of the original project")
 def test_committed_slices_are_what_the_extractor_produces(tmp_path, golden_dir):
     a, b = str(tmp_path / "inference.json"), str(tmp_path / "training.json")
     subprocess.check_call([sys.executable, os.path.join(golden_dir, "gen_graph_slice.py"), REF_PB, a, b], stdout=subprocess.DEVNULL)

@@ -60,6 +60,21 @@ def test_samples_file_is_the_reference_format(tmp_path):
         assert len(a) == 8 + 265 * len(snaps) and a == b
 
 
+def test_samples_file_matches_the_reference_bytes(golden_dir, tmp_path):
+    """az_samples_write_file around the records the reference's NNTrainDataStorage::saveTrainingSamples wrote (tests/golden/
+    turn_samples.npz, generator tests/golden/gen_turn_samples.py): the reference's file is the record count as uint64, then the
+    265-byte records, so writing those records must give back exactly that file"""
+    from alphazero_risk_b200 import api
+    z = np.load(os.path.join(golden_dir, "turn_samples.npz"))
+    names = [k for k in z.files if k.endswith("_records")]
+    assert len(names) == 4
+    for name in names:
+        recs = z[name]
+        path = str(tmp_path / (name + ".bin"))
+        api.write_samples_file(path, recs)
+        assert open(path, "rb").read() == np.uint64(len(recs)).tobytes() + recs.tobytes(), name
+
+
 @pytest.mark.gpu
 def test_device_recording_matches_oracle_replay():
     """az_selfplay_run with recording: every finished game's samples (state image, policy target, outcome) equal an oracle replay"""
