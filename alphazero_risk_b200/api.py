@@ -148,6 +148,9 @@ def lib():
         L.az_mcts6_root_stats.argtypes = [vp, vp, vp, vp, vp, vp]
         L.az_selfplay6_run.argtypes = [vp, C.c_int, vp]
         L.az_mcts6_counters.argtypes = [vp, C.POINTER(AzCounters6), u64, u64, u64, C.c_int, vp]
+        L.az_selfplay6_record.argtypes = [vp, C.c_size_t, C.c_int]
+        L.az_selfplay6_samples.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_uint64), vp]
+        L.az_nn_train6.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_int, C.c_uint64, vp, vp, vp]
         L.az_dist_nccl_version.argtypes = [C.POINTER(C.c_int)]
         L.az_dist_init.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(vp)]
         L.az_dist_unique_id.argtypes = [vp]
@@ -377,6 +380,14 @@ class Net:
         r = np.ascontiguousarray(records, np.uint8).reshape(-1, SAMPLE_BYTES)
         lp, lv = np.zeros(epochs, np.float32), np.zeros(epochs, np.float32)
         check(self.L.az_nn_train(self.h, _ptr(r), r.shape[0], int(epochs), int(batch_size), int(seed), _ptr(lp), _ptr(lv), stream))
+        return lp, lv
+
+    def train6(self, records, epochs, batch_size=512, seed=0, stream=None):
+        """train() on six-player SAMPLE6_BYTES records (Mcts6.samples), with the six-seat input encoding; returns per-epoch
+        (policy loss, value loss) means"""
+        r = np.ascontiguousarray(records, np.uint8).reshape(-1, SAMPLE6_BYTES)
+        lp, lv = np.zeros(epochs, np.float32), np.zeros(epochs, np.float32)
+        check(self.L.az_nn_train6(self.h, _ptr(r), r.shape[0], int(epochs), int(batch_size), int(seed), _ptr(lp), _ptr(lv), stream))
         return lp, lv
 
     def copy_state_from(self, other, stream=None):
@@ -684,6 +695,8 @@ class Dist:
 
 
 ENV6_IMAGE_BYTES = 108
+# six-player training record: image[108] | float value | float pi[43] | int8 final status | 3 zero bytes (include/az_b200.h)
+SAMPLE6_BYTES = 288
 
 
 class Env6:
@@ -780,6 +793,22 @@ class Mcts6:
 
     def selfplay(self, n_moves, stream=None):
         check(self.L.az_selfplay6_run(self.h, int(n_moves), stream))
+
+    def record(self, capacity_samples, max_moves_per_game=4096):
+        """enable training-sample recording (az_selfplay6_record) in selfplay() and search(apply_move=True).  Staging costs about
+        288 bytes x max_moves_per_game per game on the device: roughly 19 GB for 16384 games at the default 4096.  Under
+        uniform-random play a game with the default rules lasts 598 / 2690 / 3349 plies (min / median / max over 60 games), about
+        415 with max_game_rounds = 20; a game longer than max_moves_per_game is dropped whole and counted."""
+        check(self.L.az_selfplay6_record(self.h, C.c_size_t(int(capacity_samples)), int(max_moves_per_game)))
+
+    def samples(self, stream=None):
+        """finished-game samples as a [k, SAMPLE6_BYTES] uint8 array and the dropped count (az_selfplay6_samples)"""
+        n, dropped = C.c_size_t(0), C.c_uint64(0)
+        check(self.L.az_selfplay6_samples(self.h, None, C.c_size_t(0), C.byref(n), C.byref(dropped), stream))
+        out = np.empty((n.value, SAMPLE6_BYTES), np.uint8)
+        if n.value:          # an empty queue was drained (and its dropped count reset) by the query itself
+            check(self.L.az_selfplay6_samples(self.h, _ptr(out), C.c_size_t(n.value), C.byref(n), C.byref(dropped), stream))
+        return out[:n.value], int(dropped.value)
 
     def counters(self, reset=False, stream=None):
         c, sims, evals, errs = AzCounters6(), C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)

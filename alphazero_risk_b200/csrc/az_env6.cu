@@ -189,6 +189,7 @@ struct az_env6 {
     uint8_t* d_img = nullptr; uint8_t* d_action = nullptr; int8_t* d_status = nullptr; uint64_t* d_valid = nullptr; int* d_bad = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool timed = false;
+    uint64_t generation = 0;    // bumped by reset / import: a search's staged samples of the games before it are abandoned
 };
 
 // accessors for az_mcts6.cu
@@ -198,6 +199,7 @@ int az_env6_device(const az_env6* e) { return e->device; }
 uint64_t az_env6_seed(const az_env6* e) { return e->seed; }
 uint32_t az_env6_first_game(const az_env6* e) { return e->first_game; }
 const az_rules* az_env6_rules(const az_env6* e) { return &e->rules; }
+uint64_t az_env6_generation(const az_env6* e) { return e->generation; }
 
 static AzRulesDev e6_rules(const az_rules& r)
 {
@@ -252,6 +254,7 @@ extern "C" int az_env6_reset(az_env6* e, uint64_t seed, void* stream)
     AZ_REQUIRE(e != nullptr, "env is NULL");
     AzDeviceGuard guard(e->device);
     e->seed = seed;
+    e->generation++;
     k_env6_reset<<<e6_grid(e->n), E6_BLOCK, 0, (cudaStream_t)stream>>>(e->d_state, e->n, seed, e->first_game);
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
@@ -328,6 +331,7 @@ extern "C" int az_env6_import(az_env6* e, const uint8_t* h_images, void* stream)
     cudaStream_t s = (cudaStream_t)stream;
     AZ_CUDA(cudaMemcpyAsync(e->d_img, h_images, (size_t)e->n * E6_IMG, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaMemsetAsync(e->d_bad, 0, sizeof(int), s));
+    e->generation++;
     k_env6_import<<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, e->d_img, e->d_bad);
     AZ_CUDA(cudaGetLastError());
     int bad = 0;

@@ -11,12 +11,16 @@
 // warp's shared-memory state row — the six-seat rules are thread code, shared with the environment kernels —, the table work
 // (hash-window probing, node records, PUCT argmax) uses all 32 lanes.  The leaf batch goes through the same policy / value tower
 // as the two-player game (k_env6_encode6 -> az_nn_forward_dev).  Deliberately simpler than az_mcts.cu (one pool per game, no
-// virtual loss, no arena, no sample records): a throughput extension, the tower is what it spends its time in.
+// virtual loss, no arena): the tower is what it spends its time in.
+//
+// Training samples (AZ_SAMPLE6_BYTES records, az_samples6.cuh): k_mcts6_finish stages (state words, pi) per real move; the game's warp
+// turns them into records in k_mcts6_rec_end once the game has ended.
 #include <cstring>
 #include <new>
 
 #include "az_common.cuh"
 #include "az_game6.cuh"
+#include "az_samples6.cuh"
 #include "az_nn.cuh"
 #include "az_pseudo_net.h"
 
@@ -54,6 +58,14 @@ struct Mcts6Dev {
     uint64_t seed; uint32_t first_game;
     AzRulesDev rules;
     int eval_mode, temp_threshold;
+    // sample recording (az_selfplay6_record): per-game staging until the game ends
+    uint32_t* rec_state;    // [n][rec_moves][27]  state words 0..26 of the root before the move
+    float* rec_pi;          // [n][rec_moves][43]  policy target
+    uint32_t* rec_len;      // [n]                 staged samples of the running game (> rec_moves = overflowed)
+    int8_t* rec_end;        // [n]                 status of a game that ended at the last real move, else AZ_STATUS_RUNNING
+    uint8_t* rec_out;       // [rec_cap][288]      records of finished games
+    unsigned long long* rec_count;   // [2]        records in rec_out, samples dropped (staging or queue full)
+    int rec_moves; unsigned long long rec_cap;
 };
 
 struct M6Smem {
@@ -363,6 +375,16 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
             for (int i = 0; i < AZ_MOVES; ++i) { it = __fadd_rn(it, op[i]); if (it >= a) { move = i; break; } }
         }
         if (apply_move && move != AZ_NONE) {
+            if (m.rec_out) {                                 // stage (root before the move, pi); the records are written when the game ends
+                const uint32_t k = m.rec_len[gi];
+                if (k < (uint32_t)m.rec_moves) {
+                    uint32_t* rs = m.rec_state + ((size_t)gi * m.rec_moves + k) * S6_IMG_WORDS;
+                    float* rp = m.rec_pi + ((size_t)gi * m.rec_moves + k) * AZ_MOVES;
+                    for (int w = 0; w < S6_IMG_WORDS; ++w) rs[w] = row[w];
+                    for (int i = 0; i < AZ_MOVES; ++i) rp[i] = op[i];
+                }
+                m.rec_len[gi] = k + 1;                       // > rec_moves marks the game's samples as overflowed (dropped at the end)
+            }
             E6DiceWord dice; dice.w = blk.x;
             e6_move(c, T, m.rules, move, dice);
             c.ply++;
@@ -371,6 +393,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
             if (status != AZ_STATUS_RUNNING) {
                 atomicAdd(&m.counters[M6C_GAMES], 1ull);
                 if (status == AZ_STATUS_DRAW) atomicAdd(&m.counters[M6C_DRAWS], 1ull); else atomicAdd(&m.counters[M6C_WIN0 + status], 1ull);
+                if (m.rec_out) m.rec_end[gi] = (int8_t)status;    // before the re-deal: the staged samples belong to this result
                 if (auto_reset) e6_new_game(c, m.seed, game, c.ply);
             }
             m6_pack_row(c, row);
@@ -382,52 +405,57 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
     m.out_status[gi] = (int8_t)status;
 }
 
-// the six-seat network input (SIXPLAYER.md): the reference's [7][6][13] tensor with "enemy" = the seat that moves next and
-// "neutral" = every other seat; one thread per position (r6_encode of the oracle, same expressions)
+// the staged samples of every game that ended at the last real move -> records with their value targets, one contiguous block per game
+// in the output queue (az_rec_reserve: a game that overflowed its staging or does not fit is dropped whole and counted).  One warp per
+// game; the lanes write the game's records word by word.
+__global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_rec_end(Mcts6Dev m)
+{
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int gi = blockIdx.x * M6_WARPS + warp;
+    if (gi >= m.n) return;
+    const int status = m.rec_end[gi];
+    if (status == AZ_STATUS_RUNNING) return;
+    const uint32_t len = m.rec_len[gi];
+    unsigned long long base = 0;
+    int ok = 0;
+    if (lane == 0 && len > 0) ok = az_rec_reserve(m.rec_count, m.rec_cap, len, len <= (uint32_t)m.rec_moves, &base);
+    ok = __shfl_sync(M6_FULL, ok, 0);
+    base = ((unsigned long long)__shfl_sync(M6_FULL, (uint32_t)(base >> 32), 0) << 32) | __shfl_sync(M6_FULL, (uint32_t)base, 0);
+    if (ok) {
+        const uint32_t* rs = m.rec_state + (size_t)gi * m.rec_moves * S6_IMG_WORDS;
+        const float* rp = m.rec_pi + (size_t)gi * m.rec_moves * AZ_MOVES;
+        uint32_t* dst = (uint32_t*)(m.rec_out + base * S6_BYTES);
+        for (uint32_t j = (uint32_t)lane; j < len * S6_WORDS; j += 32) {
+            const uint32_t i = j / S6_WORDS, k = j % S6_WORDS;
+            dst[j] = s6_record_word(rs + (size_t)i * S6_IMG_WORDS, rp + (size_t)i * AZ_MOVES, status, (int)k);
+        }
+    }
+    if (lane == 0) { m.rec_len[gi] = 0; m.rec_end[gi] = AZ_STATUS_RUNNING; }
+}
+
+// the six-seat network input (SIXPLAYER.md, e6_encode_position); one thread per position
 __global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict__ st, int n, float* __restrict__ x)
 {
     const int gi = blockIdx.x * 128 + threadIdx.x;
     if (gi >= n) return;
     uint32_t row[E6_WORDS];
     for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * n + gi];
-    const uint8_t* army = (const uint8_t*)row; const uint8_t* owner = (const uint8_t*)(row + 11);
     const uint32_t cur = (row[24] >> 16) & 0xffu, phase = (row[25] >> 8) & 0xffu, attacks = (row[23] >> 24) & 0xffu, allow = (row[23] >> 16) & 0xffu;
-    uint64_t own[E6_PLAYERS] = { 0, 0, 0, 0, 0, 0 };
-    int own_total = 0, other_total = 0;
-    for (int i = 0; i < AZ_LANDS; ++i) {
-        own[owner[i]] |= 1ull << i;
-        if (owner[i] == cur) own_total += army[i]; else other_total += army[i];
-    }
-    uint32_t nx = cur;
-    for (int k = 0; k < E6_PLAYERS; ++k) { nx = nx + 1 == E6_PLAYERS ? 0u : nx + 1; if (own[nx]) break; }
-    const float ref = (float)az_reinforcement_value(own[cur]);
-    float oref = 0.0f;
-    for (uint32_t p = 0; p < E6_PLAYERS; ++p) if (p != cur && own[p]) oref = __fadd_rn(oref, (float)az_reinforcement_value(own[p]));
-    const float army_share = __fdiv_rn((float)own_total, __fadd_rn((float)own_total, (float)other_total));
-    const float reinf_share = __fdiv_rn(ref, __fadd_rn(ref, oref));
-    float att = __fdiv_rn((float)attacks, 8.0f); att = att > 1.0f ? 1.0f : att;
-    float* out = x + (size_t)gi * AZ_INPUT_FLOATS;
-    for (int i = 0; i < AZ_LANDS; ++i) {
-        float* f = out + i * 13;
-        const float a = __fdiv_rn((float)army[i], 32.0f);
-        f[0] = owner[i] == cur ? a : 0.0f;
-        f[1] = (owner[i] == nx && nx != cur) ? a : 0.0f;
-        f[2] = (owner[i] != cur && owner[i] != nx) ? a : 0.0f;
-        f[3] = army_share; f[4] = reinf_share; f[5] = att; f[6] = allow ? 1.0f : 0.0f;
-        for (uint32_t k = 0; k < 6; ++k) f[7 + k] = phase == k ? 1.0f : 0.0f;
-    }
+    e6_encode_position((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, x + (size_t)gi * AZ_INPUT_FLOATS);
 }
 
 // ---------------------------------------------------------------- host side
 struct az_env6;
 uint32_t* az_env6_state_ptr(az_env6* e); int az_env6_n(const az_env6* e); int az_env6_device(const az_env6* e);
 uint64_t az_env6_seed(const az_env6* e); uint32_t az_env6_first_game(const az_env6* e); const az_rules* az_env6_rules(const az_env6* e);
+uint64_t az_env6_generation(const az_env6* e);
 
 struct az_mcts6 {
     az_env6* env = nullptr; az_nn* nn = nullptr;
     int evaluator = M6_EVAL_NN, precision = AZ_NN_FP32, device = 0, sims = 0;
     Mcts6Dev d;
     float* d_x = nullptr;
+    uint64_t rec_generation = 0;    // the env's deal generation the staged samples belong to
     std::vector<void*> allocs;
 };
 
@@ -506,8 +534,12 @@ static int m6_search_once(az_mcts6* mc, int pick_mode, int apply_move, int auto_
     Mcts6Dev& d = mc->d;
     if (mc->evaluator == M6_EVAL_NN && !mc->nn->finalized) { int frc = az_nn_finalize(mc->nn); if (frc) return frc; }
     d.seed = az_env6_seed(mc->env); d.first_game = az_env6_first_game(mc->env);
-    const uint64_t* tab = az_device_tables();
     const int grid = (d.n + M6_WARPS - 1) / M6_WARPS;
+    if (d.rec_out && mc->rec_generation != az_env6_generation(mc->env)) {    // games re-dealt or imported since: their staged samples go
+        AZ_CUDA(cudaMemsetAsync(d.rec_len, 0, sizeof(uint32_t) * (size_t)d.n, s));
+        mc->rec_generation = az_env6_generation(mc->env);
+    }
+    const uint64_t* tab = az_device_tables();
     k_mcts6_begin<<<grid, M6_WARPS * 32, 0, s>>>(d);
     k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, -1);
     AZ_CUDA(cudaGetLastError());
@@ -519,6 +551,10 @@ static int m6_search_once(az_mcts6* mc, int pick_mode, int apply_move, int auto_
     }
     k_mcts6_finish<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, pick_mode, apply_move, auto_reset);
     AZ_CUDA(cudaGetLastError());
+    if (d.rec_out && apply_move) {
+        k_mcts6_rec_end<<<grid, M6_WARPS * 32, 0, s>>>(d);
+        AZ_CUDA(cudaGetLastError());
+    }
     return AZ_OK;
 }
 
@@ -560,6 +596,52 @@ extern "C" int az_selfplay6_run(az_mcts6* mc, int n_moves, void* stream)
     AZ_REQUIRE(n_moves >= 0, "n_moves must be >= 0");
     AzDeviceGuard guard(mc->device);
     for (int i = 0; i < n_moves; ++i) { int rc = m6_search_once(mc, 1, 1, 1, (cudaStream_t)stream); if (rc) return rc; }
+    return AZ_OK;
+}
+
+// ---- six-player training samples (az_samples6.cuh)
+extern "C" int az_selfplay6_record(az_mcts6* mc, size_t capacity_samples, int max_moves_per_game)
+{
+    AZ_REQUIRE(mc != nullptr, "mcts is NULL");
+    AZ_REQUIRE(capacity_samples > 0 && max_moves_per_game > 0, "capacity_samples and max_moves_per_game must be positive");
+    AZ_REQUIRE(mc->d.rec_out == nullptr, "recording is already enabled on this handle");
+    AzDeviceGuard guard(mc->device);
+    Mcts6Dev& d = mc->d;
+    const size_t n = (size_t)d.n;
+    int rc = 0;
+    rc |= m6_alloc(mc, &d.rec_state, n * (size_t)max_moves_per_game * S6_IMG_WORDS, false);
+    rc |= m6_alloc(mc, &d.rec_pi, n * (size_t)max_moves_per_game * AZ_MOVES, false);
+    rc |= m6_alloc(mc, &d.rec_len, n);
+    rc |= m6_alloc(mc, &d.rec_end, n, false);
+    rc |= m6_alloc(mc, &d.rec_count, (size_t)2);
+    uint8_t* out = nullptr;
+    rc |= m6_alloc(mc, &out, capacity_samples * (size_t)S6_BYTES, false);
+    if (rc) { d.rec_out = nullptr; return AZ_ERR_CUDA; }
+    AZ_CUDA(cudaMemset(d.rec_end, 0xff, n));           // AZ_STATUS_RUNNING: no game has ended
+    d.rec_moves = max_moves_per_game; d.rec_cap = capacity_samples;
+    mc->rec_generation = az_env6_generation(mc->env);
+    d.rec_out = out;                                   // set last: the kernels record iff rec_out != NULL
+    return AZ_OK;
+}
+
+extern "C" int az_selfplay6_samples(az_mcts6* mc, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream)
+{
+    AZ_REQUIRE(mc && n_out, "NULL argument");
+    AZ_REQUIRE(mc->d.rec_out != nullptr, "az_selfplay6_record has not been called");
+    AzDeviceGuard guard(mc->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned long long h[2];
+    AZ_CUDA(cudaMemcpyAsync(h, mc->d.rec_count, sizeof h, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
+    AZ_REQUIRE(h[0] <= mc->d.rec_cap, "sample queue corrupted: committed count exceeds the capacity");
+    const size_t have = (size_t)h[0];                  // committed records: az_rec_reserve never reserves past the capacity
+    if (h_dropped) *h_dropped = h[1];
+    *n_out = have;
+    if (!h_records && have) return AZ_OK;              // size query; with an empty queue the call drains (resets the dropped count)
+    AZ_REQUIRE(max_records >= have, "h_records is too small: query the size with h_records = NULL first");
+    if (have) AZ_CUDA(cudaMemcpyAsync(h_records, mc->d.rec_out, have * (size_t)S6_BYTES, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaMemsetAsync(mc->d.rec_count, 0, sizeof h, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
     return AZ_OK;
 }
 

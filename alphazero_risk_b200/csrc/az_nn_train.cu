@@ -29,6 +29,7 @@
 
 #include "az_common.cuh"
 #include "az_nn.cuh"
+#include "az_samples6.cuh"
 #include "az_tc_gemm.cuh"
 
 #define TR_CH AZ_NN_CH
@@ -747,6 +748,20 @@ __global__ void __launch_bounds__(64) k_tr_unpack_samples(const uint8_t* __restr
     if (threadIdx.x < 43) { uint32_t u = 0; for (int k = 0; k < 4; ++k) u |= (uint32_t)r[92 + 4 * threadIdx.x + k] << (8 * k); tp[(size_t)b * 43 + threadIdx.x] = __uint_as_float(u); }
 }
 
+// six-player records (az_samples6.cuh) -> the six-seat input planes of each record's image (e6_encode_position, the encoding the
+// six-player search evaluates its leaves with) + value and policy targets; one thread per sample
+__global__ void __launch_bounds__(128) k_tr_unpack_samples6(const uint8_t* __restrict__ rec, const uint32_t* __restrict__ order, int n,
+                                                            float* __restrict__ x, float* __restrict__ tp, float* __restrict__ tv)
+{
+    const int b = blockIdx.x * 128 + threadIdx.x;
+    if (b >= n) return;
+    const uint8_t* r = rec + (size_t)order[b] * S6_BYTES;
+    e6_encode_position(r, r + AZ_LANDS, r[S6_CUR], r[S6_PHASE], r[S6_ATTACKS], r[S6_ALLOW_DRAW], x + (size_t)b * AZ_INPUT_FLOATS);
+    const float* f = (const float*)r;                       // records are 4-byte aligned (288-byte stride)
+    tv[b] = f[S6_VALUE / 4];
+    for (int i = 0; i < AZ_MOVES; ++i) tp[(size_t)b * AZ_MOVES + i] = f[S6_PI / 4 + i];
+}
+
 // ---------------------------------------------------------------- host side
 static bool is_moving(const std::string& name)
 {
@@ -1047,26 +1062,32 @@ extern "C" int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_targ
     return AZ_OK;
 }
 
-// AlphaZeroNN::train (alphazero_nn.cpp:351-410): `epochs` passes over the samples in shuffled order, whole batches of batch_size only
-// (:372 batchCount = size / BATCH_SIZE).  Samples are the packed records az_selfplay_samples returns (the reference's file layout).
-// The reference shuffles with its process-wide std engine (irreproducible, src/rng.h:16); here: Fisher-Yates on splitmix64(seed).
-extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
-                           float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream)
+// the record -> (input planes, targets) step of a training loop: batch b of an epoch unpacks the n records order[0..n) of d_rec
+typedef void (*TrUnpack)(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s);
+static void tr_unpack_samples(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s)
 {
-    AZ_REQUIRE(nn && h_records, "NULL argument");
-    AZ_REQUIRE(epochs >= 1 && batch_size >= 2, "epochs must be >= 1 and batch_size >= 2");
-    AZ_REQUIRE(n_records >= (size_t)batch_size, "fewer samples than one batch");
-    AzDeviceGuard guard(nn->device);
-    cudaStream_t s = (cudaStream_t)stream;
+    k_tr_unpack_samples<<<(unsigned)n, 64, 0, s>>>(d_rec, d_order, n, x, tp, tv);
+}
+static void tr_unpack_samples6(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s)
+{
+    k_tr_unpack_samples6<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv);
+}
+
+// AlphaZeroNN::train (alphazero_nn.cpp:351-410): `epochs` passes over the samples in shuffled order, whole batches of batch_size only
+// (:372 batchCount = size / BATCH_SIZE), on records of rec_bytes each that `unpack` turns into a batch.
+// The reference shuffles with its process-wide std engine (irreproducible, src/rng.h:16); here: Fisher-Yates on splitmix64(seed).
+static int train_records(az_nn* nn, const char* who, const uint8_t* h_records, size_t n_records, size_t rec_bytes, TrUnpack unpack,
+                         int epochs, int batch_size, uint64_t seed, float* h_epoch_loss_policy, float* h_epoch_loss_value, cudaStream_t s)
+{
     AzTrainState* t = train_state(nn);
     AZ_REQUIRE(t != nullptr, "out of host memory");
     int rc = train_reserve(nn, t, batch_size); if (rc) return rc;
     uint8_t* d_rec = nullptr; uint32_t* d_order = nullptr; double* d_acc = nullptr;
-    AZ_CUDA(cudaMalloc(&d_rec, n_records * (size_t)AZ_SAMPLE_BYTES));
+    AZ_CUDA(cudaMalloc(&d_rec, n_records * rec_bytes));
     if (cudaMalloc(&d_order, sizeof(uint32_t) * n_records) != cudaSuccess || cudaMalloc(&d_acc, 2 * sizeof(double)) != cudaSuccess) {
         cudaFree(d_rec); cudaFree(d_order); az_set_error("out of device memory"); return AZ_ERR_CUDA;
     }
-    cudaError_t ce = cudaMemcpyAsync(d_rec, h_records, n_records * (size_t)AZ_SAMPLE_BYTES, cudaMemcpyHostToDevice, s);
+    cudaError_t ce = cudaMemcpyAsync(d_rec, h_records, n_records * rec_bytes, cudaMemcpyHostToDevice, s);
     std::vector<uint32_t> order(n_records);
     for (size_t i = 0; i < n_records; ++i) order[i] = (uint32_t)i;
     uint64_t st = seed;
@@ -1083,7 +1104,7 @@ extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records
         // the batches of an epoch are enqueued back to back; the losses are accumulated on the device and read once per epoch
         if (ce == cudaSuccess) ce = cudaMemsetAsync(d_acc, 0, 2 * sizeof(double), s);
         for (size_t b = 0; b < batches && ce == cudaSuccess && rc == AZ_OK; ++b) {
-            k_tr_unpack_samples<<<(unsigned)batch_size, 64, 0, s>>>(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv);
+            unpack(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv, s);
             rc = train_step_dev(nn, t->d_x, t->d_tp, t->d_tv, batch_size, nullptr, s);
             if (rc == AZ_OK) k_tr_loss_accum<<<1, 32, 0, s>>>(t->d_loss, d_acc);
         }
@@ -1095,8 +1116,38 @@ extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records
     }
     cudaStreamSynchronize(s);
     cudaFree(d_rec); cudaFree(d_order); cudaFree(d_acc);
-    if (ce != cudaSuccess) { az_set_error("az_nn_train: %s", cudaGetErrorString(ce)); return AZ_ERR_CUDA; }
+    if (ce != cudaSuccess) { az_set_error("%s: %s", who, cudaGetErrorString(ce)); return AZ_ERR_CUDA; }
     return rc;
+}
+
+// Samples are the packed records az_selfplay_samples returns (the reference's file layout).
+extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
+                           float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream)
+{
+    AZ_REQUIRE(nn && h_records, "NULL argument");
+    AZ_REQUIRE(epochs >= 1 && batch_size >= 2, "epochs must be >= 1 and batch_size >= 2");
+    AZ_REQUIRE(n_records >= (size_t)batch_size, "fewer samples than one batch");
+    AzDeviceGuard guard(nn->device);
+    return train_records(nn, "az_nn_train", h_records, n_records, AZ_SAMPLE_BYTES, tr_unpack_samples, epochs, batch_size, seed,
+                         h_epoch_loss_policy, h_epoch_loss_value, (cudaStream_t)stream);
+}
+
+// The same loop on six-player records (az_selfplay6_samples); the input planes are the six-seat encoding of each record's image.
+extern "C" int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
+                            float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream)
+{
+    AZ_REQUIRE(nn && h_records, "NULL argument");
+    AZ_REQUIRE(epochs >= 1 && batch_size >= 2, "epochs must be >= 1 and batch_size >= 2");
+    AZ_REQUIRE(n_records >= (size_t)batch_size, "fewer samples than one batch");
+    for (size_t i = 0; i < n_records; ++i) {                // the encoder indexes per-seat tables with these bytes
+        const uint8_t* r = h_records + i * S6_BYTES;
+        bool ok = r[S6_CUR] < E6_PLAYERS;
+        for (int l = 0; l < AZ_LANDS; ++l) ok = ok && r[AZ_LANDS + l] < E6_PLAYERS;
+        if (!ok) { az_set_error("az_nn_train6: record %zu holds a seat outside 0..5", i); return AZ_ERR_INVALID_ARG; }
+    }
+    AzDeviceGuard guard(nn->device);
+    return train_records(nn, "az_nn_train6", h_records, n_records, S6_BYTES, tr_unpack_samples6, epochs, batch_size, seed,
+                         h_epoch_loss_policy, h_epoch_loss_value, (cudaStream_t)stream);
 }
 
 // AZ_NN_FP32 (default): every contraction on the fp32 pipes — the parity path.  AZ_NN_BF16: forward convolutions, data gradients and

@@ -349,6 +349,25 @@ AZ_API int az_mcts6_search(az_mcts6* mcts, int pick_mode, int apply_move, uint32
 AZ_API int az_mcts6_root_stats(az_mcts6* mcts, float* h_q, float* h_p, uint32_t* h_sumn, int32_t* h_table, void* stream);
 AZ_API int az_selfplay6_run(az_mcts6* mcts, int n_moves, void* stream);      /* n_moves moves of every game, finished games re-dealt */
 AZ_API int az_mcts6_counters(az_mcts6* mcts, az_counters6* h_out, uint64_t* h_sims, uint64_t* h_evals, uint64_t* h_errors, int reset, void* stream);
+/* ---- six-player training samples.  A record format of this project (the reference's 88-byte NNInputData has no room for six owners),
+   AZ_SAMPLE6_BYTES per sample, every field 4-byte aligned:
+     bytes 0..107    the root position BEFORE the move as its AZ_ENV6_IMAGE_BYTES image (az_env6_export's bytes; seat to move = byte 98)
+     bytes 108..111  float value target: 1 when the seat to move won, 0 after a draw, -1/5 (the search's -v / 5 with v = 1) otherwise
+     bytes 112..283  float policy target[43]: the search's pi for that move (az_mcts6_search's h_pi), bit for bit
+     byte  284       int8 final status of the game (winner seat 0..5 or AZ_STATUS_DRAW); bytes 285..287 zero */
+#define AZ_SAMPLE6_BYTES 288
+/* enable recording in az_selfplay6_run / az_mcts6_search(apply_move != 0), both pick modes: every real move stages one sample per game
+   (max_moves_per_game per game on the device, about 288 bytes each); when a game ends its samples go to an output queue of
+   capacity_samples records as one contiguous block with their value targets.  A game that overflows its staging area or does not fit
+   the queue is dropped whole and counted.  Staged samples of games abandoned by az_env6_reset / az_env6_import are discarded.
+   Recording changes nothing the search computes. */
+AZ_API int az_selfplay6_record(az_mcts6* mcts, size_t capacity_samples, int max_moves_per_game);
+/* drains the six-player queue: the calling convention of az_selfplay_samples with AZ_SAMPLE6_BYTES records */
+AZ_API int az_selfplay6_samples(az_mcts6* mcts, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream);
+/* az_nn_train on AZ_SAMPLE6_BYTES records: the same shuffled epochs, whole batches, per-epoch mean losses and training precisions; the
+   input planes are the six-seat encoding of az_env6_encode, built on the device from each record's image */
+AZ_API int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
+                        float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
 
 /* ---------------------------------------------------------------- multi-GPU (SURVEY.md 8e): NCCL over NVLink / NVSwitch, never inside a search
    Games shard over GPUs by contiguous global id (first_game_id of az_env_create) and never migrate; every GPU holds a full copy of
