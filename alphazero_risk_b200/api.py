@@ -151,6 +151,10 @@ def lib():
         L.az_selfplay6_record.argtypes = [vp, C.c_size_t, C.c_int]
         L.az_selfplay6_samples.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_uint64), vp]
         L.az_nn_train6.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_int, C.c_uint64, vp, vp, vp]
+        L.az_arena6_create.argtypes = [vp, C.POINTER(vp), C.c_int, vp, C.c_int, C.POINTER(vp)]
+        L.az_arena6_destroy.argtypes = [vp]
+        L.az_arena6_play.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(AzArena6Results), vp, vp, vp]
+        L.az_arena6_active_slots.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
         L.az_dist_nccl_version.argtypes = [C.POINTER(C.c_int)]
         L.az_dist_init.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(vp)]
         L.az_dist_unique_id.argtypes = [vp]
@@ -815,3 +819,55 @@ class Mcts6:
         check(self.L.az_mcts6_counters(self.h, C.byref(c), C.byref(sims), C.byref(evals), C.byref(errs), int(reset), stream))
         return dict(steps=int(c.steps), games=int(c.games), draws=int(c.draws), wins=[int(c.wins[i]) for i in range(6)], sims=int(sims.value),
                     evals=int(evals.value), errors=int(errs.value))
+
+
+class AzArena6Results(C.Structure):
+    """mirror of az_arena6_results"""
+    _fields_ = [("count", C.c_uint64), ("draw", C.c_uint64), ("win", C.c_uint64 * 6), ("win_seat", C.c_uint64 * 6),
+                ("moves", C.c_uint64 * 6), ("sims", C.c_uint64), ("evals", C.c_uint64), ("ticks", C.c_uint64), ("errors", C.c_uint64)]
+
+    def as_dict(self):
+        return dict(count=int(self.count), draw=int(self.draw), win=[int(v) for v in self.win], win_seat=[int(v) for v in self.win_seat],
+                    moves=[int(v) for v in self.moves], sims=int(self.sims), evals=int(self.evals), ticks=int(self.ticks),
+                    errors=int(self.errors))
+
+
+class Arena6:
+    """six-player matches on the device (az_arena6_*, SIXPLAYER.md §4): `agents` are Mcts6 handles over `env` or None (the
+    uniform-random player), seat_agent[s] = the agent index that holds seat s; with rotate_seats the six games of a group share
+    one deal and rotate the seats"""
+
+    def __init__(self, env, agents, seat_agent, rotate_seats=True):
+        self.L, self.env, self.agents = lib(), env, list(agents)
+        hs = (C.c_void_p * max(1, len(self.agents)))(*[a.h if a is not None else None for a in self.agents])
+        seats = np.ascontiguousarray(seat_agent, np.uint8)
+        assert seats.shape == (6,)
+        h = C.c_void_p()
+        check(self.L.az_arena6_create(env.h, hs, len(self.agents), _ptr(seats), int(rotate_seats), C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.az_arena6_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def play(self, n_games, seed, first_game=0, stream=None):
+        """match games first_game .. first_game + n_games - 1: the result tallies plus per-game `status` (winner seat or STATUS_DRAW)
+        and `plies`"""
+        r = AzArena6Results()
+        st, pl = np.empty(int(n_games), np.int8), np.empty(int(n_games), np.uint32)
+        check(self.L.az_arena6_play(self.h, int(first_game), int(n_games), int(seed), C.byref(r), _ptr(st), _ptr(pl), stream))
+        out = r.as_dict()
+        out.update(status=st, plies=pl)
+        return out
+
+    def active_slots(self):
+        """slots that held a game at each tick of the last play()"""
+        n = C.c_size_t(0)
+        check(self.L.az_arena6_active_slots(self.h, None, C.c_size_t(0), C.byref(n)))
+        out = np.empty(n.value, np.uint32)
+        if n.value:
+            check(self.L.az_arena6_active_slots(self.h, _ptr(out), C.c_size_t(n.value), C.byref(n)))
+        return out

@@ -30,3 +30,30 @@ struct ArenaDev {
 };
 
 int az_launch_arena_advance(const ArenaDev& a, const az_rules* rules, cudaStream_t s);   // az_env.cu
+// ascending list of the slots with flags[slot] == want: the leaf-batch compaction of both arenas.  The kernel is defined in az_mcts.cu;
+// az_launch_arena_list (az_mcts6.cu) launches it for the six-player arena.
+__global__ void k_arena_list(const uint8_t* __restrict__ flags, int n, int want, int32_t* __restrict__ out);
+int az_launch_arena_list(const uint8_t* flags, int n, int want, int32_t* out, cudaStream_t s);
+
+// ---------------------------------------------------------------- six-player arena (az_arena6_*, SIXPLAYER.md §4)
+// shared by az_env6.cu (k_arena6_advance) and az_mcts6.cu (host loop)
+enum { A6_COUNT = 0, A6_DRAW = 1, A6_WIN0 = 2, A6_WIN_SEAT0 = 8, A6_MOVES0 = 14, A6_CLAIMED = 20, A6_ACTIVE = 21, A6_WAIT0 = 22, A6_N = 28 };
+enum { A6_FREE = 0, A6_PLAYING = 1, A6_DONE = 2 };
+
+struct Arena6Dev {
+    int n;                      // slots of the env
+    uint32_t first_game;        // match game ids first_game .. first_game + n_games - 1
+    uint64_t n_games, seed;
+    uint32_t* state;            // env6 SoA [28][n]
+    uint8_t* slot;              // [n]  A6_FREE (claims a game next), A6_PLAYING, A6_DONE (no game left)
+    uint32_t* slot_game;        // [n]  match game id of the slot's game
+    uint8_t* to_move;           // [n]  agent whose searcher moves next in this slot (0xff = none this tick)
+    int8_t* out_status;         // [n_games]  per match game: winner seat or AZ_STATUS_DRAW
+    uint32_t* out_plies;        // [n_games]  and its plies
+    unsigned long long* res;    // [A6_N]
+    uint32_t seat_agent;        // agent index of seat s in bits 4s .. 4s + 3
+    uint8_t searcher;           // bit a: agent a is a searcher (else the uniform-random player)
+    uint8_t rotate;
+};
+
+int az_launch_arena6_advance(const Arena6Dev& a, const az_rules* rules, cudaStream_t s);   // az_env6.cu

@@ -16,6 +16,7 @@
 #include <new>
 
 #include "az_common.cuh"
+#include "az_arena.cuh"
 
 #define E6_BLOCK 128                    // configs[3] has 16384 games per GPU: 128 blocks = four warps on 128 of the 148 SMs (256: 64 SMs)
 #include "az_game6.cuh"
@@ -178,6 +179,78 @@ __global__ void __launch_bounds__(E6_BLOCK) k_env6_import(uint32_t* __restrict__
     e6_store(c, sm, st, n, gi);
 }
 
+// ---------------------------------------------------------------- six-player arena (SIXPLAYER.md §4): everything between two searches
+// One thread per slot: tally the slot's finished game (per-game status and plies on the device), claim the next match game from
+// the shared counter and deal it (deal of game id g - g % 6 with rotation, else g; ply 0), play the uniform-random player's plies
+// (az_env6_rollout's rule keyed by the match game id), and stop when a searcher's seat is to move: to_move = that agent.  At most
+// 64 iterations per launch, like k_arena_advance.  res[A6_ACTIVE] counts the slots that hold a game afterwards, res[A6_WAIT0 + a]
+// those waiting for agent a's search.
+__global__ void __launch_bounds__(E6_BLOCK) k_arena6_advance(Arena6Dev a, const uint64_t* __restrict__ g_tab, AzRulesDev rules)
+{
+    __shared__ E6Smem sm;
+    __shared__ unsigned s_cnt[1 + 2 * E6_PLAYERS];    // active slots, waiting slots per agent, random plies per agent
+    if (threadIdx.x < 1 + 2 * E6_PLAYERS) s_cnt[threadIdx.x] = 0;
+    const AzTables T = e6_stage(sm, g_tab);           // (its barrier also orders the zeroing above)
+    const int gi = blockIdx.x * E6_BLOCK + threadIdx.x;
+    int slot = gi < a.n ? a.slot[gi] : A6_DONE;
+    if (slot != A6_DONE) {
+        E6Ctx c;
+        uint32_t game = 0, r = 0;
+        int wait = 0xff;
+        if (slot == A6_PLAYING) { e6_load(c, sm, a.state, a.n, gi); game = a.slot_game[gi]; r = a.rotate ? game % E6_PLAYERS : 0u; }
+        else e6_bind(c, sm);
+        for (int it = 0; it < 64; ++it) {
+            if (slot == A6_PLAYING) {
+                const int st = e6_status(c.g, rules);
+                if (st != AZ_STATUS_RUNNING) {
+                    const uint32_t k = game - a.first_game;
+                    atomicAdd(&a.res[A6_COUNT], 1ull);
+                    if (st == AZ_STATUS_DRAW) atomicAdd(&a.res[A6_DRAW], 1ull);
+                    else {
+                        atomicAdd(&a.res[A6_WIN0 + ((a.seat_agent >> (4 * (((uint32_t)st + r) % E6_PLAYERS))) & 0xfu)], 1ull);
+                        atomicAdd(&a.res[A6_WIN_SEAT0 + st], 1ull);
+                    }
+                    a.out_status[k] = (int8_t)st; a.out_plies[k] = c.ply;
+                    slot = A6_FREE;
+                }
+            }
+            if (slot == A6_FREE) {
+                const unsigned long long k = atomicAdd(&a.res[A6_CLAIMED], 1ull);
+                if (k >= a.n_games) { slot = A6_DONE; break; }
+                game = a.first_game + (uint32_t)k;
+                r = a.rotate ? game % E6_PLAYERS : 0u;
+                for (int w = 0; w < 22; ++w) sm.col[w * E6_BLOCK + threadIdx.x] = 0;
+                e6_new_game(c, a.seed, game - r, 0);
+                c.ply = 0;
+                slot = A6_PLAYING;
+                continue;
+            }
+            const uint32_t agent = (a.seat_agent >> (4 * ((c.g.cur + r) % E6_PLAYERS))) & 0xfu;
+            if ((a.searcher >> agent) & 1u) { wait = (int)agent; break; }
+            const uint64_t valid = e6_valid(c.g, T, rules);
+            const az_u32x4 blk = az_rng_block(a.seed, game, c.ply, AZ_STREAM_REAL, 0);
+            const int action = az_nth_set_bit(valid, az_mulhi32(blk.y, (uint32_t)__popcll(valid)));
+            { E6DiceWord dice; dice.w = blk.x; e6_move(c, T, rules, action, dice); }
+            c.ply++;
+            atomicAdd(&s_cnt[1 + E6_PLAYERS + agent], 1u);
+        }
+        if (slot == A6_PLAYING) {
+            e6_store(c, sm, a.state, a.n, gi);
+            a.slot_game[gi] = game;
+            atomicAdd(&s_cnt[0], 1u);
+            if (wait != 0xff) atomicAdd(&s_cnt[1 + wait], 1u);
+        }
+        a.slot[gi] = (uint8_t)slot;
+        a.to_move[gi] = (uint8_t)wait;
+    }
+    __syncthreads();
+    if (threadIdx.x < 1 + 2 * E6_PLAYERS && s_cnt[threadIdx.x]) {
+        const int i = threadIdx.x;
+        const int dst = i == 0 ? A6_ACTIVE : i <= E6_PLAYERS ? A6_WAIT0 + i - 1 : A6_MOVES0 + i - 1 - E6_PLAYERS;
+        atomicAdd(&a.res[dst], (unsigned long long)s_cnt[i]);
+    }
+}
+
 // ---------------------------------------------------------------- C ABI
 struct az_env6 {
     int n = 0, device = 0;
@@ -207,6 +280,13 @@ static AzRulesDev e6_rules(const az_rules& r)
     d.max_game_rounds = r.max_game_rounds; d.min_unit_move = r.min_unit_move; return d;
 }
 static inline int e6_grid(int n) { return (n + E6_BLOCK - 1) / E6_BLOCK; }
+
+int az_launch_arena6_advance(const Arena6Dev& a, const az_rules* rules, cudaStream_t s)
+{
+    k_arena6_advance<<<e6_grid(a.n), E6_BLOCK, 0, s>>>(a, az_device_tables(), e6_rules(*rules));
+    AZ_CUDA(cudaGetLastError());
+    return AZ_OK;
+}
 
 extern "C" int az_env6_create(int n_games, const az_rules* rules, int device, uint32_t first_game_id, az_env6** out)
 {

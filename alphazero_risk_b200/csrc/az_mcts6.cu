@@ -11,7 +11,8 @@
 // warp's shared-memory state row — the six-seat rules are thread code, shared with the environment kernels —, the table work
 // (hash-window probing, node records, PUCT argmax) uses all 32 lanes.  The leaf batch goes through the same policy / value tower
 // as the two-player game (k_env6_encode6 -> az_nn_forward_dev).  Deliberately simpler than az_mcts.cu (one pool per game, no
-// virtual loss, no arena): the tower is what it spends its time in.
+// virtual loss): the tower is what it spends its time in.  The six-player arena (az_arena6_*, end of this file) restricts a search to
+// the games waiting for its searcher and compacts their leaf batch.
 //
 // Training samples (AZ_SAMPLE6_BYTES records, az_samples6.cuh): k_mcts6_finish stages (state words, pi) per real move; the game's warp
 // turns them into records in k_mcts6_rec_end once the game has ended.
@@ -19,6 +20,7 @@
 #include <new>
 
 #include "az_common.cuh"
+#include "az_arena.cuh"
 #include "az_game6.cuh"
 #include "az_samples6.cuh"
 #include "az_nn.cuh"
@@ -66,6 +68,9 @@ struct Mcts6Dev {
     uint8_t* rec_out;       // [rec_cap][288]      records of finished games
     unsigned long long* rec_count;   // [2]        records in rec_out, samples dropped (staging or queue full)
     int rec_moves; unsigned long long rec_cap;
+    // six-player arena (az_arena6_play sets these around a search; NULL = every game, ids first_game + gi)
+    const uint8_t* sel; int sel_value;    // only games with sel[gi] == sel_value search
+    const uint32_t* game_id;              // [n] the game id of the descents' dice and the real move, replacing first_game + gi
 };
 
 struct M6Smem {
@@ -109,6 +114,8 @@ __device__ __forceinline__ uint64_t m6_hash(uint32_t kw, int lane)
     }
     return az_pn_mix(h);
 }
+__device__ __forceinline__ bool m6_skip(const Mcts6Dev& m, int gi) { return m.sel && m.sel[gi] != (uint8_t)m.sel_value; }
+__device__ __forceinline__ uint32_t m6_game(const Mcts6Dev& m, int gi) { return m.game_id ? m.game_id[gi] : m.first_game + (uint32_t)gi; }
 __device__ __forceinline__ uint32_t* m6_node(const Mcts6Dev& m, int gi, uint32_t idx) { return m.nodes + ((size_t)gi * m.cap + idx) * M6_NODE_WORDS; }
 
 // the node of the position whose key words sit in lanes 0..26 (kw), or -1; empty_slot = where an insert would go
@@ -258,7 +265,7 @@ __device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int gi, uint32_t* 
     __syncwarp();
     E6Ctx c; m6_bind(c, row, scratch);
     AzDicePhilox dice;
-    if (lane == 0) { m6_unpack_row(c, row); dice.init(m.seed, m.first_game + (uint32_t)gi, c.ply, (uint32_t)(sim < 0 ? 0 : sim)); }
+    if (lane == 0) { m6_unpack_row(c, row); dice.init(m.seed, m6_game(m, gi), c.ply, (uint32_t)(sim < 0 ? 0 : sim)); }
     uint32_t depth = 0;
     for (;;) {
         int st = 0; uint64_t valid = 0; uint32_t mover = 0;
@@ -302,7 +309,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_begin(Mcts6Dev m)
 {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int gi = blockIdx.x * M6_WARPS + warp;
-    if (gi >= m.n) return;
+    if (gi >= m.n || m6_skip(m, gi)) return;
     uint32_t* ix = m.index + (size_t)gi * m.H;
     for (int i = lane; i < m.H; i += 32) ix[i] = 0u;
     if (lane == 0) { m.count[gi] = 0u; m.pending[gi] = 0; m.path_len[gi] = 0u; m.term_value[gi] = 0.0f; m.term_seat[gi] = 0; }
@@ -316,7 +323,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_sim(Mcts6Dev m, const u
     const AzTables T = az_tables_from_smem(sm.tab);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int gi = blockIdx.x * M6_WARPS + warp;
-    if (gi >= m.n) return;
+    if (gi >= m.n || m6_skip(m, gi)) return;
     m6_complete(m, gi, sm.row[warp], lane);
     m6_descend(m, gi, sm.row[warp], sm.scratch[warp], T, round, lane);
 }
@@ -332,7 +339,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
     const AzTables T = az_tables_from_smem(sm.tab);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int gi = blockIdx.x * M6_WARPS + warp;
-    if (gi >= m.n) return;
+    if (gi >= m.n || m6_skip(m, gi)) return;
     uint32_t* row = sm.row[warp];
     m6_complete(m, gi, row, lane);
     __syncwarp();
@@ -347,7 +354,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
     m6_unpack_row(c, row);
     int status = e6_status(c.g, m.rules);
     int move = AZ_NONE;
-    const uint32_t game = m.first_game + (uint32_t)gi;
+    const uint32_t game = m6_game(m, gi);
     uint32_t* ov = m.out_visits + (size_t)gi * AZ_MOVES; float* op = m.out_pi + (size_t)gi * AZ_MOVES;
     float* oq = m.out_q + (size_t)gi * AZ_MOVES; float* opp = m.out_p + (size_t)gi * AZ_MOVES;
     for (int i = 0; i < AZ_MOVES; ++i) { ov[i] = 0u; op[i] = 0.0f; oq[i] = 0.0f; opp[i] = 0.0f; }
@@ -433,15 +440,40 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_rec_end(Mcts6Dev m)
     if (lane == 0) { m.rec_len[gi] = 0; m.rec_end[gi] = AZ_STATUS_RUNNING; }
 }
 
-// the six-seat network input (SIXPLAYER.md, e6_encode_position); one thread per position
+// the six-seat network input (SIXPLAYER.md, e6_encode_position) of game gi of the SoA state st [28][n]
+__device__ __forceinline__ void m6_encode_game(const uint32_t* __restrict__ st, int n, int gi, float* __restrict__ out)
+{
+    uint32_t row[E6_WORDS];
+    for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * n + gi];
+    const uint32_t cur = (row[24] >> 16) & 0xffu, phase = (row[25] >> 8) & 0xffu, attacks = (row[23] >> 24) & 0xffu, allow = (row[23] >> 16) & 0xffu;
+    e6_encode_position((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, out);
+}
+// one thread per position
 __global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict__ st, int n, float* __restrict__ x)
 {
     const int gi = blockIdx.x * 128 + threadIdx.x;
     if (gi >= n) return;
-    uint32_t row[E6_WORDS];
-    for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * n + gi];
-    const uint32_t cur = (row[24] >> 16) & 0xffu, phase = (row[25] >> 8) & 0xffu, attacks = (row[23] >> 24) & 0xffu, allow = (row[23] >> 16) & 0xffu;
-    e6_encode_position((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, x + (size_t)gi * AZ_INPUT_FLOATS);
+    m6_encode_game(st, n, gi, x + (size_t)gi * AZ_INPUT_FLOATS);
+}
+
+// arena leaf batches: row i = the leaf of game games[i] (the games that search this tick), and the network's outputs back to them
+__global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __restrict__ st, int n, const int32_t* __restrict__ games, int count,
+                                                          float* __restrict__ x)
+{
+    const int i = blockIdx.x * 128 + threadIdx.x;
+    if (i >= count) return;
+    m6_encode_game(st, n, games[i], x + (size_t)i * AZ_INPUT_FLOATS);
+}
+__global__ void __launch_bounds__(256) k_mcts6_scatter_evals(const float* __restrict__ pol_c, const float* __restrict__ val_c,
+                                                             const int32_t* __restrict__ games, int count, float* __restrict__ pol,
+                                                             float* __restrict__ val)
+{
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= count * (AZ_MOVES + 1)) return;
+    const int c = i / (AZ_MOVES + 1), e = i - c * (AZ_MOVES + 1);
+    const size_t g = (size_t)games[c];
+    if (e < AZ_MOVES) pol[g * AZ_MOVES + e] = pol_c[(size_t)c * AZ_MOVES + e];
+    else val[g] = val_c[c];
 }
 
 // ---------------------------------------------------------------- host side
@@ -456,6 +488,10 @@ struct az_mcts6 {
     Mcts6Dev d;
     float* d_x = nullptr;
     uint64_t rec_generation = 0;    // the env's deal generation the staged samples belong to
+    // arena: only the listed games go through the network (az_arena6_play sets these around a search; the buffers are the arena's)
+    const int32_t* eval_games = nullptr;    // ascending list of the searching games
+    int eval_count = 0;                     // its length; 0 = every game is evaluated
+    float* eval_pol = nullptr; float* eval_val = nullptr;   // compacted outputs [count][43], [count]
     std::vector<void*> allocs;
 };
 
@@ -524,6 +560,15 @@ static int m6_evaluate(az_mcts6* mc, cudaStream_t s)
 {
     if (mc->evaluator != M6_EVAL_NN) return AZ_OK;
     Mcts6Dev& d = mc->d;
+    if (mc->eval_count > 0 && mc->eval_count < d.n) {
+        const int m = mc->eval_count;
+        k_env6_encode_list<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, d.n, mc->eval_games, m, mc->d_x);
+        AZ_CUDA(cudaGetLastError());
+        int rc = az_nn_forward_dev(mc->nn, mc->d_x, m, mc->eval_pol, mc->eval_val, mc->precision, s); if (rc) return rc;
+        k_mcts6_scatter_evals<<<(m * (AZ_MOVES + 1) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, m, d.nn_policy, d.nn_value);
+        AZ_CUDA(cudaGetLastError());
+        return AZ_OK;
+    }
     k_env6_encode<<<(d.n + 127) / 128, 128, 0, s>>>(d.leaf_state, d.n, mc->d_x);
     AZ_CUDA(cudaGetLastError());
     return az_nn_forward_dev(mc->nn, mc->d_x, d.n, d.nn_policy, d.nn_value, mc->precision, s);
@@ -676,5 +721,159 @@ extern "C" int az_env6_encode(az_env6* e, float* h_x, void* stream)
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
     cudaFree(d_x);
     if (ce != cudaSuccess) { az_set_error("az_env6_encode: %s", cudaGetErrorString(ce)); return AZ_ERR_CUDA; }
+    return AZ_OK;
+}
+
+// ---------------------------------------------------------------- six-player arena (SIXPLAYER.md §4)
+// k_arena6_advance (az_env6.cu) tallies, deals and plays the random player's plies; each tick then runs one search per searcher
+// restricted to the slots waiting for it (Mcts6Dev::sel over to_move), with the slots' match game ids as the search's game ids, and
+// its leaf batches compacted to those slots.  A searcher's move can hand the turn to another agent: that slot waits for the next tick.
+struct az_arena6 {
+    az_env6* env = nullptr;
+    az_mcts6* agent[E6_PLAYERS] = {};    // NULL = the uniform-random player
+    int n_agents = 0;
+    Arena6Dev a;
+    int32_t* d_list = nullptr;           // slots waiting for the searcher of this search (leaf-batch compaction)
+    float* d_pol_c = nullptr; float* d_val_c = nullptr;   // compacted network outputs [n][43], [n]
+    int8_t* d_status = nullptr; uint32_t* d_plies = nullptr; uint64_t games_cap = 0;   // per match game
+    std::vector<uint32_t> active;        // active slots of every tick of the last match
+    std::vector<void*> allocs;
+};
+
+int az_launch_arena_list(const uint8_t* flags, int n, int want, int32_t* out, cudaStream_t s)
+{
+    k_arena_list<<<1, 1024, 0, s>>>(flags, n, want, out);
+    AZ_CUDA(cudaGetLastError());
+    return AZ_OK;
+}
+
+template <class T> static int a6_alloc(az_arena6* ar, T** p, size_t count)
+{
+    AZ_CUDA(cudaMalloc(p, sizeof(T) * count));
+    AZ_CUDA(cudaMemset(*p, 0, sizeof(T) * count));
+    ar->allocs.push_back(*p);
+    return AZ_OK;
+}
+
+extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_agents, const uint8_t* seat_agent, int rotate_seats, az_arena6** out)
+{
+    AZ_REQUIRE(env && agents && seat_agent && out, "NULL argument");
+    AZ_REQUIRE(n_agents >= 1 && n_agents <= E6_PLAYERS, "n_agents must be in 1..6");
+    for (int i = 0; i < n_agents; ++i) {
+        if (!agents[i]) continue;
+        AZ_REQUIRE(agents[i]->env == env, "every searcher must be built over the arena's env (the agents share its game states)");
+        for (int j = 0; j < i; ++j) AZ_REQUIRE(agents[j] != agents[i], "the same az_mcts6 handle appears twice (each agent owns its tables)");
+    }
+    unsigned held = 0;
+    for (int s = 0; s < E6_PLAYERS; ++s) {
+        AZ_REQUIRE(seat_agent[s] < n_agents, "seat_agent entry out of range (must be < n_agents)");
+        held |= 1u << seat_agent[s];
+    }
+    AZ_REQUIRE(held == (1u << n_agents) - 1u, "every agent must hold at least one seat");
+    AzDeviceGuard guard(az_env6_device(env));
+    az_arena6* ar = new (std::nothrow) az_arena6();
+    AZ_REQUIRE(ar != nullptr, "out of host memory");
+    ar->env = env; ar->n_agents = n_agents;
+    Arena6Dev& a = ar->a;
+    memset(&a, 0, sizeof a);
+    a.n = az_env6_n(env); a.state = az_env6_state_ptr(env); a.rotate = rotate_seats ? 1 : 0;
+    for (int s = 0; s < E6_PLAYERS; ++s) a.seat_agent |= (uint32_t)seat_agent[s] << (4 * s);
+    for (int i = 0; i < n_agents; ++i) { ar->agent[i] = agents[i]; if (agents[i]) a.searcher |= (uint8_t)(1u << i); }
+    const size_t n = (size_t)a.n;
+    int rc = 0;
+    rc |= a6_alloc(ar, &a.slot, n); rc |= a6_alloc(ar, &a.slot_game, n); rc |= a6_alloc(ar, &a.to_move, n);
+    rc |= a6_alloc(ar, &a.res, (size_t)A6_N); rc |= a6_alloc(ar, &ar->d_list, n);
+    rc |= a6_alloc(ar, &ar->d_pol_c, n * AZ_MOVES); rc |= a6_alloc(ar, &ar->d_val_c, n);
+    if (rc) { for (void* p : ar->allocs) cudaFree(p); delete ar; return AZ_ERR_CUDA; }
+    *out = ar;
+    return AZ_OK;
+}
+
+extern "C" int az_arena6_destroy(az_arena6* ar)
+{
+    if (!ar) return AZ_OK;
+    AzDeviceGuard guard(az_env6_device(ar->env));
+    for (void* p : ar->allocs) cudaFree(p);
+    cudaFree(ar->d_status); cudaFree(ar->d_plies);
+    delete ar;
+    return AZ_OK;
+}
+
+extern "C" int az_arena6_play(az_arena6* ar, uint64_t first_game, uint64_t n_games, uint64_t seed, az_arena6_results* h_out,
+                              int8_t* h_status, uint32_t* h_plies, void* stream)
+{
+    AZ_REQUIRE(ar && h_out, "NULL argument");
+    Arena6Dev& a = ar->a;
+    for (int i = 0; i < ar->n_agents; ++i)
+        AZ_REQUIRE(!ar->agent[i] || !ar->agent[i]->d.rec_out, "a searcher with sample recording enabled cannot play in an arena");
+    AZ_REQUIRE(!a.rotate || (first_game % E6_PLAYERS == 0 && n_games % E6_PLAYERS == 0),
+               "with rotate_seats, first_game and n_games must be multiples of 6 (whole rotation groups)");
+    AZ_REQUIRE(first_game <= (1ull << 32) && n_games <= (1ull << 32) - first_game, "first_game + n_games must not exceed 2^32 (32-bit game ids)");
+    AzDeviceGuard guard(az_env6_device(ar->env));
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n_games > ar->games_cap) {
+        cudaFree(ar->d_status); cudaFree(ar->d_plies);
+        ar->d_status = nullptr; ar->d_plies = nullptr; ar->games_cap = 0;
+        AZ_CUDA(cudaMalloc(&ar->d_status, n_games));
+        AZ_CUDA(cudaMalloc(&ar->d_plies, sizeof(uint32_t) * n_games));
+        ar->games_cap = n_games;
+    }
+    int rc = az_env6_reset(ar->env, seed, stream); if (rc) return rc;
+    a.seed = seed; a.first_game = (uint32_t)first_game; a.n_games = n_games; a.out_status = ar->d_status; a.out_plies = ar->d_plies;
+    const size_t n = (size_t)a.n;
+    AZ_CUDA(cudaMemsetAsync(a.slot, A6_FREE, n, s));
+    AZ_CUDA(cudaMemsetAsync(a.res, 0, sizeof(unsigned long long) * A6_N, s));
+    for (int i = 0; i < ar->n_agents; ++i)
+        if (ar->agent[i]) AZ_CUDA(cudaMemsetAsync(ar->agent[i]->d.counters, 0, sizeof(unsigned long long) * M6C_N, s));
+    const az_rules* rules = az_env6_rules(ar->env);
+    unsigned long long cnt[1 + E6_PLAYERS];                              // A6_ACTIVE, A6_WAIT0 ..
+    ar->active.clear();
+    for (;;) {
+        AZ_CUDA(cudaMemsetAsync(a.res + A6_ACTIVE, 0, sizeof cnt, s));
+        rc = az_launch_arena6_advance(a, rules, s); if (rc) return rc;
+        AZ_CUDA(cudaMemcpyAsync(cnt, a.res + A6_ACTIVE, sizeof cnt, cudaMemcpyDeviceToHost, s));
+        AZ_CUDA(cudaStreamSynchronize(s));
+        if (cnt[0] == 0) break;
+        ar->active.push_back((uint32_t)cnt[0]);
+        for (int i = 0; i < ar->n_agents; ++i) {
+            az_mcts6* mc = ar->agent[i];
+            if (!mc || !cnt[1 + i]) continue;
+            if (mc->evaluator == M6_EVAL_NN && cnt[1 + i] < (unsigned long long)a.n) {
+                rc = az_launch_arena_list(a.to_move, a.n, i, ar->d_list, s); if (rc) return rc;
+                mc->eval_games = ar->d_list; mc->eval_count = (int)cnt[1 + i]; mc->eval_pol = ar->d_pol_c; mc->eval_val = ar->d_val_c;
+            }
+            mc->d.sel = a.to_move; mc->d.sel_value = i; mc->d.game_id = a.slot_game;
+            rc = m6_search_once(mc, 0, 1, 0, s);                            // argmax, the move applied, no re-deal
+            mc->d.sel = nullptr; mc->d.sel_value = 0; mc->d.game_id = nullptr;
+            mc->eval_games = nullptr; mc->eval_count = 0; mc->eval_pol = nullptr; mc->eval_val = nullptr;
+            if (rc) return rc;
+        }
+    }
+    unsigned long long r[A6_N], c[E6_PLAYERS][M6C_N];
+    memset(c, 0, sizeof c);
+    AZ_CUDA(cudaMemcpyAsync(r, a.res, sizeof r, cudaMemcpyDeviceToHost, s));
+    for (int i = 0; i < ar->n_agents; ++i)
+        if (ar->agent[i]) AZ_CUDA(cudaMemcpyAsync(c[i], ar->agent[i]->d.counters, sizeof c[i], cudaMemcpyDeviceToHost, s));
+    if (h_status && n_games) AZ_CUDA(cudaMemcpyAsync(h_status, ar->d_status, n_games, cudaMemcpyDeviceToHost, s));
+    if (h_plies && n_games) AZ_CUDA(cudaMemcpyAsync(h_plies, ar->d_plies, sizeof(uint32_t) * n_games, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
+    memset(h_out, 0, sizeof *h_out);
+    h_out->count = r[A6_COUNT]; h_out->draw = r[A6_DRAW];
+    for (int p = 0; p < E6_PLAYERS; ++p) {
+        h_out->win[p] = r[A6_WIN0 + p]; h_out->win_seat[p] = r[A6_WIN_SEAT0 + p];
+        h_out->moves[p] = ar->agent[p] ? c[p][M6C_STEPS] : r[A6_MOVES0 + p];
+        h_out->sims += c[p][M6C_SIMS]; h_out->evals += c[p][M6C_EVALS]; h_out->errors += c[p][M6C_OVERFLOW];
+    }
+    h_out->ticks = ar->active.size();
+    return AZ_OK;
+}
+
+extern "C" int az_arena6_active_slots(az_arena6* ar, uint32_t* h_active, size_t max_ticks, size_t* n_out)
+{
+    AZ_REQUIRE(ar && n_out, "NULL argument");
+    *n_out = ar->active.size();
+    if (!h_active) return AZ_OK;
+    AZ_REQUIRE(max_ticks >= ar->active.size(), "h_active is too small: query the size with h_active = NULL first");
+    if (!ar->active.empty()) memcpy(h_active, ar->active.data(), sizeof(uint32_t) * ar->active.size());
     return AZ_OK;
 }

@@ -368,6 +368,34 @@ AZ_API int az_selfplay6_samples(az_mcts6* mcts, uint8_t* h_records, size_t max_r
    input planes are the six-seat encoding of az_env6_encode, built on the device from each record's image */
 AZ_API int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                         float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
+/* ---- six-player arena (SIXPLAYER.md §4): seat-rotated matches between searchers and the uniform-random player over one env6.
+   An agent is an az_mcts6 handle over `env` (argmax play, table cleared per search) or NULL = the uniform-random player
+   (az_env6_rollout's rule).  seat_agent[s] = the agent index that holds seat s; every agent holds at least one seat.  Match game g
+   (first_game <= g < first_game + n_games) starts from the deal of game id d (e6_new_game(seed, d, 0)) with ply 0; with rotate_seats
+   d = g - g % 6 and seat s is played by seat_agent[(s + g % 6) % 6] (the six games of a group share one deal, every agent sits in
+   every seat), without it d = g and seat s by seat_agent[s].  All randomness of a ply is keyed by (seed, g, ply), so a game's
+   result depends only on (seed, g, agents), never on the slot that played it or the env's size: a multi-GPU match is disjoint
+   first_game ranges plus az_dist_gather_stats over the result struct (all uint64_t). */
+typedef struct az_arena6 az_arena6;
+typedef struct az_arena6_results {
+    uint64_t count, draw;
+    uint64_t win[6];        /* by agent index */
+    uint64_t win_seat[6];   /* by seat */
+    uint64_t moves[6];      /* plies played, by agent index */
+    uint64_t sims, evals, ticks, errors;   /* errors = the searchers' overflow counters, must be 0 */
+} az_arena6_results;
+/* agents[i] == NULL: the uniform-random player.  Rejects handles over another env, the same handle twice, n_agents outside 1..6,
+   seat_agent entries >= n_agents and agents without a seat */
+AZ_API int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_agents, const uint8_t* seat_agent /*[6]*/,
+                            int rotate_seats, az_arena6** out);
+AZ_API int az_arena6_destroy(az_arena6* arena);
+/* resets the env with `seed` and zeroes the searchers' counters, then plays the match over the env's slots.  h_status / h_plies: NULL
+   or [n_games], per match game (winner seat 0..5 or AZ_STATUS_DRAW; plies).  Rejects handles with recording enabled, with rotation
+   first_game or n_games not a multiple of 6, and first_game + n_games > 2^32.  The handles search stand-alone as before afterwards. */
+AZ_API int az_arena6_play(az_arena6* arena, uint64_t first_game, uint64_t n_games, uint64_t seed, az_arena6_results* h_out,
+                          int8_t* h_status, uint32_t* h_plies, void* stream);
+/* the number of slots that held a game at each tick of the last az_arena6_play (*n_out = its ticks; h_active = NULL: size query) */
+AZ_API int az_arena6_active_slots(az_arena6* arena, uint32_t* h_active, size_t max_ticks, size_t* n_out);
 
 /* ---------------------------------------------------------------- multi-GPU (SURVEY.md 8e): NCCL over NVLink / NVSwitch, never inside a search
    Games shard over GPUs by contiguous global id (first_game_id of az_env_create) and never migrate; every GPU holds a full copy of
