@@ -5,13 +5,16 @@
 // reference's AlphaZeroMCTS (player/alpha_zero/alphazero_mcts.cpp: PUCT :67-119, search :322-377, addValue :8-21, policy from the
 // visit counts :121-148, move choice :379-412) with the two changes SIXPLAYER.md states: the table is cleared before every search
 // (no trimNodes carry-over), and a leaf's scalar value belongs to the seat to move there — on the way up a node whose mover is
-// that seat receives +v, every other node -v / 5.  One descent per tree per leaf batch (THREADS_PER_MCTS = 1 semantics).
+// that seat receives +v, every other node -v / 5.  az_rules.concurrent_descents = K descents per tree per leaf batch in the two-player
+// lockstep schedule (az_mcts.cu, SIXPLAYER.md §2; checker oracle/risk6_lockstep.c): descent j of round r uses the dice of simulation
+// r * K + j and selects after descents 0..j-1 under the active_N rule; the round's leaves are evaluated as one batch of K * n positions,
+// then expanded and backed up in descent order.  K = 1 is the one-descent search (THREADS_PER_MCTS = 1 semantics).
 //
 // Mapping: one warp per game.  The game logic of a descent (status, legal mask, transition: az_game6.cuh) runs on lane 0 over the
 // warp's shared-memory state row — the six-seat rules are thread code, shared with the environment kernels —, the table work
 // (hash-window probing, node records, PUCT argmax) uses all 32 lanes.  The leaf batch goes through the same policy / value tower
-// as the two-player game (k_env6_encode6 -> az_nn_forward_dev).  Deliberately simpler than az_mcts.cu (one pool per game, no
-// virtual loss): the tower is what it spends its time in.  The six-player arena (az_arena6_*, end of this file) restricts a search to
+// as the two-player game (k_env6_encode -> az_nn_forward_dev).  Deliberately simpler than az_mcts.cu (one pool per game, no tree
+// reuse between searches): the tower is what it spends its time in.  The six-player arena (az_arena6_*, end of this file) restricts a search to
 // the games waiting for its searcher and compacts their leaf batch.
 //
 // Training samples (AZ_SAMPLE6_BYTES records, az_samples6.cuh): k_mcts6_finish stages (state words, pi) per real move; the game's warp
@@ -41,18 +44,19 @@ enum { M6C_SIMS = 0, M6C_EVALS = 1, M6C_OVERFLOW = 2, M6C_STEPS = 3, M6C_GAMES =
 
 struct Mcts6Dev {
     int n, cap, H, dmax;
-    uint32_t* nodes;        // [n][cap][M6_NODE_WORDS]
+    int K;                  // descents per tree per round (az_rules.concurrent_descents); descent slot = j * n + game
+    uint32_t* nodes;        // [n][cap][M6_NODE_WORDS]; the N word of a move: N in the low 24 bits, active_N in the top byte
     uint32_t* index;        // [n][H]   0 = empty, else tag16 << 16 | (node + 1)
     uint32_t* count;        // [n]
-    uint32_t* path;         // [n][dmax]  node | move << 16 | mover << 22
-    uint32_t* path_len;     // [n]
-    uint32_t* leaf_state;   // [28][n]
-    uint64_t* leaf_valid;   // [n]
-    int32_t* pending;       // [n]
-    float* term_value;      // [n]   value of a descent that ended in a finished game
-    int32_t* term_seat;     // [n]   and the seat it belongs to
-    float* nn_policy;       // [n][43]
-    float* nn_value;        // [n]
+    uint32_t* path;         // [K*n][dmax]  node | move << 16 | mover << 22
+    uint32_t* path_len;     // [K*n]
+    uint32_t* leaf_state;   // [28][K*n]
+    uint64_t* leaf_valid;   // [K*n]
+    int32_t* pending;       // [K*n]
+    float* term_value;      // [K*n]   value of a descent that ended in a finished game
+    int32_t* term_seat;     // [K*n]   and the seat it belongs to
+    float* nn_policy;       // [K*n][43]
+    float* nn_value;        // [K*n]
     uint32_t* root_state;   // the env6 state [28][n]
     uint32_t* out_visits; float* out_pi; uint8_t* out_move; int8_t* out_status; float* out_q; float* out_p; uint32_t* out_sumn; int32_t* out_table;
     unsigned long long* counters;
@@ -143,52 +147,74 @@ __device__ __forceinline__ int m6_lookup(const Mcts6Dev& m, int gi, uint64_t h, 
     return -1;
 }
 
-// getNextBestMoveAndSetVisited (alphazero_mcts.cpp:67-119), ascending move index on ties; one descent at a time: no active_N
-__device__ __forceinline__ int m6_select(const Mcts6Dev& m, const uint32_t* nd, int lane)
+// getNextBestMoveAndSetVisited (alphazero_mcts.cpp:67-119), ascending move index on ties.  A move with N == 0 && active_N == 1 (one
+// descent of the round is about to open it) is passed over (:91-93); if nothing else can be chosen the best such move is requested
+// again (:108-111).  The chosen move's active_N is incremented.  With K = 1 no mark is ever 1 at selection: the plain argmax.
+__device__ __forceinline__ int m6_select(const Mcts6Dev& m, uint32_t* nd, int lane)
 {
     const uint64_t valid = (uint64_t)nd[M6_VALID] | ((uint64_t)nd[M6_VALID + 1] << 32);
     const float sq = __fsqrt_rn(__fadd_rn(1.0f, (float)nd[M6_SUMN]));
-    float bu = -INFINITY; int bi = 64;
+    float bu = -INFINITY, du = -INFINITY; int bi = 64, di = 64;
 #pragma unroll
     for (int k = 0; k < 2; ++k) {
         const int i = lane + 32 * k;
         if (i < AZ_MOVES && ((valid >> i) & 1ull)) {
             const float P = __uint_as_float(nd[M6_P + i]), Q = __uint_as_float(nd[M6_Q + i]);
+            const uint32_t nw = nd[M6_N + i], N = nw & 0xffffffu;
             const float noiseP = __fadd_rn(__fmul_rn(m.c1, P), m.c2);
             const float v = __fmul_rn(__fmul_rn(noiseP, m.cpuct), sq);
-            const float u = __fadd_rn(Q, __fdiv_rn(v, __fadd_rn(1.0f, (float)nd[M6_N + i])));
-            if (u > bu) { bu = u; bi = i; }
+            const float u = __fadd_rn(Q, __fdiv_rn(v, __fadd_rn(1.0f, (float)N)));
+            if (N == 0u && (nw >> 24) == 1u) { if (u > du) { du = u; di = i; } }
+            else if (u > bu) { bu = u; bi = i; }
         }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
-        const float ou = __shfl_xor_sync(M6_FULL, bu, o); const int oi = __shfl_xor_sync(M6_FULL, bi, o);
+        float ou = __shfl_xor_sync(M6_FULL, bu, o); int oi = __shfl_xor_sync(M6_FULL, bi, o);
         if (ou > bu || (ou == bu && oi < bi)) { bu = ou; bi = oi; }
+        ou = __shfl_xor_sync(M6_FULL, du, o); oi = __shfl_xor_sync(M6_FULL, di, o);
+        if (ou > du || (ou == du && oi < di)) { du = ou; di = oi; }
     }
+    if (bi == 64) bi = di;
+    __syncwarp();
+    if (lane == 0 && bi < AZ_MOVES) nd[M6_N + bi] += 1u << 24;
     return bi;
 }
 
-// addValue up the recorded path: +v for the nodes of the seat the leaf value belongs to, -v / 5 for every other node
-__device__ __forceinline__ void m6_backup(const Mcts6Dev& m, int gi, float v, uint32_t seat, uint32_t len, int lane)
+// addValue up the recorded path of descent slot `slot`: +v for the nodes of the seat the leaf value belongs to, -v / 5 for every other
+// node; each step takes the descent's active_N mark off its move
+__device__ __forceinline__ void m6_backup(const Mcts6Dev& m, int slot, int gi, float v, uint32_t seat, uint32_t len, int lane)
 {
     __syncwarp();
     if (lane == 0) {
         const float other = __fdiv_rn(-v, 5.0f);
         for (int d = (int)len - 1; d >= 0; --d) {
-            const uint32_t e = m.path[(size_t)gi * m.dmax + d];
+            const uint32_t e = m.path[(size_t)slot * m.dmax + d];
             const uint32_t idx = e & 0xffffu, mv = (e >> 16) & 63u, mover = (e >> 22) & 7u;
             const float val = mover == seat ? v : other;
             uint32_t* nd = m6_node(m, gi, idx);
-            const uint32_t N = nd[M6_N + mv];
+            const uint32_t nw = nd[M6_N + mv], N = nw & 0xffffffu;
             const float Q = __uint_as_float(nd[M6_Q + mv]);
             const float q = N == 0 ? val : __fdiv_rn(__fadd_rn(__fmul_rn((float)N, Q), val), (float)(N + 1u));
             nd[M6_Q + mv] = __float_as_uint(q);
-            nd[M6_N + mv] = N + 1u;
+            nd[M6_N + mv] = (N + 1u) | (((nw >> 24) - 1u) << 24);
             nd[M6_SUMN] += 1u;
         }
         if (len > 0) atomicAdd(&m.counters[M6C_SIMS], 1ull);
-        m.path_len[gi] = 0;
+        m.path_len[slot] = 0;
     }
+    __syncwarp();
+}
+
+// a descent that overflowed the path: its marks come off without a backup (it is counted as an error, not as a simulation)
+__device__ __forceinline__ void m6_unmark(const Mcts6Dev& m, int slot, int gi, uint32_t len, int lane)
+{
+    __syncwarp();
+    if (lane == 0)
+        for (uint32_t d = 0; d < len; ++d) {
+            const uint32_t e = m.path[(size_t)slot * m.dmax + d];
+            m6_node(m, gi, e & 0xffffu)[M6_N + ((e >> 16) & 63u)] -= 1u << 24;
+        }
     __syncwarp();
 }
 
@@ -200,23 +226,24 @@ __device__ __forceinline__ uint64_t m6_pn_key(const uint32_t* row)
     return az_pn_key(land, (int)((row[24] >> 16) & 0xffu), (int)(row[24] & 0xffffu), (int)((row[25] >> 8) & 0xffu));
 }
 
-// complete the descent of the previous round: expand the queued leaf with the evaluator's output (StateSimulations ctor :26-42 after
-// NNOutputData::normalize, alphazero_nn_data.cpp:3-27), or take the finished game's value, and back it up
-__device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int gi, uint32_t* row, int lane)
+// complete descent slot `slot` of the previous round: expand the queued leaf with the evaluator's output (StateSimulations ctor :26-42
+// after NNOutputData::normalize, alphazero_nn_data.cpp:3-27), or take the finished game's value, and back it up.  A leaf an earlier
+// descent of the round has added is not inserted again (StateSimulationsStorage::add :203-215); its own value is still backed up.
+__device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int slot, int gi, uint32_t* row, int lane)
 {
-    const uint32_t len = m.path_len[gi];
-    float v = m.term_value[gi];
-    uint32_t seat = (uint32_t)m.term_seat[gi];
-    if (m.pending[gi]) {
+    const uint32_t len = m.path_len[slot];
+    float v = m.term_value[slot];
+    uint32_t seat = (uint32_t)m.term_seat[slot];
+    if (m.pending[slot]) {
         __syncwarp();
-        if (lane < E6_WORDS) row[lane] = m.leaf_state[(size_t)lane * m.n + gi];
+        if (lane < E6_WORDS) row[lane] = m.leaf_state[(size_t)lane * m.K * m.n + slot];
         __syncwarp();
-        const uint64_t valid = m.leaf_valid[gi];
+        const uint64_t valid = m.leaf_valid[slot];
         float p0 = 0.0f, p1 = 0.0f, value;
         if (m.eval_mode == M6_EVAL_NN) {
-            p0 = m.nn_policy[(size_t)gi * AZ_MOVES + lane];
-            if (lane + 32 < AZ_MOVES) p1 = m.nn_policy[(size_t)gi * AZ_MOVES + 32 + lane];
-            value = m.nn_value[gi];
+            p0 = m.nn_policy[(size_t)slot * AZ_MOVES + lane];
+            if (lane + 32 < AZ_MOVES) p1 = m.nn_policy[(size_t)slot * AZ_MOVES + 32 + lane];
+            value = m.nn_value[slot];
         } else if (m.eval_mode == M6_EVAL_PSEUDO) {
             const uint64_t key = m6_pn_key(row);
             p0 = az_pn_policy(key, lane);
@@ -252,13 +279,14 @@ __device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int gi, uint32_t*
         } else if (found < 0 && lane == 0) atomicAdd(&m.counters[M6C_OVERFLOW], 1ull);
         v = value;
         seat = (row[24] >> 16) & 0xffu;                      // the seat to move at the leaf
-        if (lane == 0) { m.pending[gi] = 0; atomicAdd(&m.counters[M6C_EVALS], 1ull); }
+        if (lane == 0) { m.pending[slot] = 0; atomicAdd(&m.counters[M6C_EVALS], 1ull); }
     }
-    m6_backup(m, gi, v, seat, len, lane);
+    m6_backup(m, slot, gi, v, seat, len, lane);
 }
 
-// one descent from the root (AlphaZeroMCTS::search :322-377 as a loop); sim < 0: only make sure the root is in the table
-__device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int gi, uint32_t* row, uint32_t* scratch, const AzTables& T, int sim, int lane)
+// one descent from the root into descent slot `slot` (AlphaZeroMCTS::search :322-377 as a loop); sim < 0: only make sure the root is
+// in the table.  A descent that ends in a finished game backs up at once; one that reaches an unseen position queues it.
+__device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int slot, int gi, uint32_t* row, uint32_t* scratch, const AzTables& T, int sim, int lane)
 {
     __syncwarp();
     if (lane < E6_WORDS) row[lane] = m.root_state[(size_t)lane * m.n + gi];
@@ -276,8 +304,8 @@ __device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int gi, uint32_t* 
         if (st != AZ_STATUS_RUNNING) {                       // a finished game: its value belongs to the winner (a draw is worth 0 to everyone)
             const float tv = st == AZ_STATUS_DRAW ? 0.0f : 1.0f;
             const uint32_t seat = st == AZ_STATUS_DRAW ? mover : (uint32_t)st;
-            if (lane == 0) { m.term_value[gi] = tv; m.term_seat[gi] = (int32_t)seat; m.pending[gi] = 0; }
-            m6_backup(m, gi, tv, seat, depth, lane);
+            if (lane == 0) { m.term_value[slot] = tv; m.term_seat[slot] = (int32_t)seat; m.pending[slot] = 0; }
+            m6_backup(m, slot, gi, tv, seat, depth, lane);
             depth = 0;
             break;
         }
@@ -286,22 +314,26 @@ __device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int gi, uint32_t* 
         int ins;
         const int idx = m6_lookup(m, gi, h, kw, lane, ins);
         if (idx < 0) {                                       // unseen position: queue it for the evaluator
-            if (lane < E6_WORDS) m.leaf_state[(size_t)lane * m.n + gi] = row[lane];
-            if (lane == 0) { m.leaf_valid[gi] = valid; m.pending[gi] = 1; m.term_value[gi] = 0.0f; m.term_seat[gi] = (int32_t)mover; }
+            if (lane < E6_WORDS) m.leaf_state[(size_t)lane * m.K * m.n + slot] = row[lane];
+            if (lane == 0) { m.leaf_valid[slot] = valid; m.pending[slot] = 1; m.term_value[slot] = 0.0f; m.term_seat[slot] = (int32_t)mover; }
             break;
         }
-        if (sim < 0) { if (lane == 0) m.pending[gi] = 0; break; }
-        if ((int)depth >= m.dmax) { if (lane == 0) { atomicAdd(&m.counters[M6C_OVERFLOW], 1ull); m.pending[gi] = 0; m.term_value[gi] = 0.0f; } depth = 0; break; }
+        if (sim < 0) { if (lane == 0) m.pending[slot] = 0; break; }
+        if ((int)depth >= m.dmax) {
+            m6_unmark(m, slot, gi, depth, lane);
+            if (lane == 0) { atomicAdd(&m.counters[M6C_OVERFLOW], 1ull); m.pending[slot] = 0; m.term_value[slot] = 0.0f; }
+            depth = 0; break;
+        }
         const int mv = m6_select(m, m6_node(m, gi, (uint32_t)idx), lane);
         if (lane == 0) {
-            m.path[(size_t)gi * m.dmax + depth] = (uint32_t)idx | ((uint32_t)mv << 16) | (mover << 22);
+            m.path[(size_t)slot * m.dmax + depth] = (uint32_t)idx | ((uint32_t)mv << 16) | (mover << 22);
             e6_move(c, T, m.rules, mv, dice);
             m6_pack_row(c, row);
         }
         __syncwarp();
         depth++;
     }
-    if (lane == 0) m.path_len[gi] = depth;
+    if (lane == 0) m.path_len[slot] = depth;
     __syncwarp();
 }
 
@@ -312,10 +344,16 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_begin(Mcts6Dev m)
     if (gi >= m.n || m6_skip(m, gi)) return;
     uint32_t* ix = m.index + (size_t)gi * m.H;
     for (int i = lane; i < m.H; i += 32) ix[i] = 0u;
-    if (lane == 0) { m.count[gi] = 0u; m.pending[gi] = 0; m.path_len[gi] = 0u; m.term_value[gi] = 0.0f; m.term_seat[gi] = 0; }
+    if (lane == 0) m.count[gi] = 0u;
+    if (lane < m.K) {
+        const size_t slot = (size_t)lane * m.n + gi;
+        m.pending[slot] = 0; m.path_len[slot] = 0u; m.term_value[slot] = 0.0f; m.term_seat[slot] = 0;
+    }
 }
 
-__global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_sim(Mcts6Dev m, const uint64_t* __restrict__ g_tab, int round)
+// one round: complete the K descents of the previous round in order, then (do_descent) start the K descents of this one in order;
+// round < 0: the root round.  Bounded to the register budget of five blocks per SM, which K = 1 had without the bound.
+__global__ void __launch_bounds__(M6_WARPS * 32, 5) k_mcts6_sim(Mcts6Dev m, const uint64_t* __restrict__ g_tab, int round, int do_descent)
 {
     __shared__ M6Smem sm;
     for (int i = threadIdx.x; i < AZ_TABLE_U64; i += blockDim.x) sm.tab[i] = g_tab[i];
@@ -324,8 +362,10 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_sim(Mcts6Dev m, const u
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int gi = blockIdx.x * M6_WARPS + warp;
     if (gi >= m.n || m6_skip(m, gi)) return;
-    m6_complete(m, gi, sm.row[warp], lane);
-    m6_descend(m, gi, sm.row[warp], sm.scratch[warp], T, round, lane);
+    for (int j = 0; j < m.K; ++j) m6_complete(m, j * m.n + gi, gi, sm.row[warp], lane);    // the previous round, in descent order
+    if (!do_descent) return;
+    if (round < 0) m6_descend(m, gi, gi, sm.row[warp], sm.scratch[warp], T, -1, lane);        // the root round: slot 0 only
+    else for (int j = 0; j < m.K; ++j) m6_descend(m, j * m.n + gi, gi, sm.row[warp], sm.scratch[warp], T, round * m.K + j, lane);
 }
 
 // after the last simulation: root statistics (calculateMoveProbability :121-148), move choice (pickHigestWeightedMove :397-412 /
@@ -341,7 +381,7 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
     const int gi = blockIdx.x * M6_WARPS + warp;
     if (gi >= m.n || m6_skip(m, gi)) return;
     uint32_t* row = sm.row[warp];
-    m6_complete(m, gi, row, lane);
+    m6_complete(m, gi, gi, row, lane);          // slot 0; with K > 1 the host has completed the last round's slots already
     __syncwarp();
     if (lane < E6_WORDS) row[lane] = m.root_state[(size_t)lane * m.n + gi];
     __syncwarp();
@@ -364,8 +404,9 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_finish(Mcts6Dev m, cons
         const uint64_t valid = (uint64_t)nd[M6_VALID] | ((uint64_t)nd[M6_VALID + 1] << 32);
         float sum = 0.0f;
         for (int i = 0; i < AZ_MOVES; ++i) if ((valid >> i) & 1ull) {
-            ov[i] = nd[M6_N + i]; oq[i] = __uint_as_float(nd[M6_Q + i]); opp[i] = __uint_as_float(nd[M6_P + i]);
-            op[i] = (float)nd[M6_N + i]; sum = __fadd_rn(sum, op[i]);
+            const uint32_t N = nd[M6_N + i] & 0xffffffu;         // the top byte is active_N
+            ov[i] = N; oq[i] = __uint_as_float(nd[M6_Q + i]); opp[i] = __uint_as_float(nd[M6_P + i]);
+            op[i] = (float)N; sum = __fadd_rn(sum, op[i]);
         }
         for (int i = 0; i < AZ_MOVES; ++i) op[i] = __fdiv_rn(op[i], sum);
         m.out_sumn[gi] = nd[M6_SUMN];
@@ -440,40 +481,43 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_rec_end(Mcts6Dev m)
     if (lane == 0) { m.rec_len[gi] = 0; m.rec_end[gi] = AZ_STATUS_RUNNING; }
 }
 
-// the six-seat network input (SIXPLAYER.md, e6_encode_position) of game gi of the SoA state st [28][n]
-__device__ __forceinline__ void m6_encode_game(const uint32_t* __restrict__ st, int n, int gi, float* __restrict__ out)
+// the six-seat network input (SIXPLAYER.md, e6_encode_position) of column i of the SoA state st [28][stride]
+__device__ __forceinline__ void m6_encode_game(const uint32_t* __restrict__ st, int stride, int i, float* __restrict__ out)
 {
     uint32_t row[E6_WORDS];
-    for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * n + gi];
+    for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * stride + i];
     const uint32_t cur = (row[24] >> 16) & 0xffu, phase = (row[25] >> 8) & 0xffu, attacks = (row[23] >> 24) & 0xffu, allow = (row[23] >> 16) & 0xffu;
     e6_encode_position((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, out);
 }
-// one thread per position
-__global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict__ st, int n, float* __restrict__ x)
-{
-    const int gi = blockIdx.x * 128 + threadIdx.x;
-    if (gi >= n) return;
-    m6_encode_game(st, n, gi, x + (size_t)gi * AZ_INPUT_FLOATS);
-}
-
-// arena leaf batches: row i = the leaf of game games[i] (the games that search this tick), and the network's outputs back to them
-__global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __restrict__ st, int n, const int32_t* __restrict__ games, int count,
-                                                          float* __restrict__ x)
+// one thread per position: columns 0..count-1 of the SoA state st [28][stride]
+__global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict__ st, int stride, int count, float* __restrict__ x)
 {
     const int i = blockIdx.x * 128 + threadIdx.x;
     if (i >= count) return;
-    m6_encode_game(st, n, games[i], x + (size_t)i * AZ_INPUT_FLOATS);
+    m6_encode_game(st, stride, i, x + (size_t)i * AZ_INPUT_FLOATS);
+}
+
+// arena leaf batches: row j * count + k = the leaf of descent slot j * n + games[k] (games = the games that search this tick, k_used =
+// descent slots per game in the batch, leaf state stride K * n), and the network's outputs back to those slots
+__global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __restrict__ st, int stride, int n, const int32_t* __restrict__ games,
+                                                          int count, int k_used, float* __restrict__ x)
+{
+    const int i = blockIdx.x * 128 + threadIdx.x;
+    if (i >= count * k_used) return;
+    const int j = i / count, k = i - j * count;
+    m6_encode_game(st, stride, j * n + games[k], x + (size_t)i * AZ_INPUT_FLOATS);
 }
 __global__ void __launch_bounds__(256) k_mcts6_scatter_evals(const float* __restrict__ pol_c, const float* __restrict__ val_c,
-                                                             const int32_t* __restrict__ games, int count, float* __restrict__ pol,
-                                                             float* __restrict__ val)
+                                                             const int32_t* __restrict__ games, int count, int n, int k_used,
+                                                             float* __restrict__ pol, float* __restrict__ val)
 {
     const int i = blockIdx.x * 256 + threadIdx.x;
-    if (i >= count * (AZ_MOVES + 1)) return;
+    if (i >= count * k_used * (AZ_MOVES + 1)) return;
     const int c = i / (AZ_MOVES + 1), e = i - c * (AZ_MOVES + 1);
-    const size_t g = (size_t)games[c];
-    if (e < AZ_MOVES) pol[g * AZ_MOVES + e] = pol_c[(size_t)c * AZ_MOVES + e];
-    else val[g] = val_c[c];
+    const int j = c / count, k = c - j * count;
+    const size_t slot = (size_t)j * n + games[k];
+    if (e < AZ_MOVES) pol[slot * AZ_MOVES + e] = pol_c[(size_t)c * AZ_MOVES + e];
+    else val[slot] = val_c[c];
 }
 
 // ---------------------------------------------------------------- host side
@@ -513,6 +557,9 @@ extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int preci
     const int T = r->threads_per_mcts < 1 ? 1 : r->threads_per_mcts;
     const int sims = r->mcts_simulations - (r->mcts_simulations % T);
     AZ_REQUIRE(sims >= 1 && sims <= 60000, "mcts_simulations - mcts_simulations % threads_per_mcts must be in 1..60000");
+    const int K = r->concurrent_descents < 1 ? 1 : r->concurrent_descents;
+    AZ_REQUIRE(K <= 16, "concurrent_descents must be <= 16");
+    AZ_REQUIRE(sims % K == 0, "the simulation count (mcts_simulations - mcts_simulations % threads_per_mcts) must be a multiple of concurrent_descents");
     AzDeviceGuard guard(az_env6_device(env));
     if (evaluator == M6_EVAL_NN && !nn->finalized) { int frc = az_nn_finalize(nn); if (frc) return frc; }
     az_mcts6* mc = new (std::nothrow) az_mcts6();
@@ -520,23 +567,23 @@ extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int preci
     mc->env = env; mc->nn = nn; mc->evaluator = evaluator; mc->precision = precision; mc->device = az_env6_device(env); mc->sims = sims;
     Mcts6Dev& d = mc->d;
     memset(&d, 0, sizeof d);
-    d.n = az_env6_n(env);
+    d.n = az_env6_n(env); d.K = K;
     d.cap = sims + 2;                                       // the table is cleared per search: the root + one node per simulation
     d.H = 64; while (d.H < 2 * d.cap) d.H <<= 1;
     d.dmax = 192;
-    const size_t n = (size_t)d.n;
+    const size_t n = (size_t)d.n, ns = n * (size_t)K;     // ns = descent slots = the leaf batch of a simulation round
     int rc = 0;
     rc |= m6_alloc(mc, &d.nodes, n * d.cap * M6_NODE_WORDS, false);
     rc |= m6_alloc(mc, &d.index, n * d.H); rc |= m6_alloc(mc, &d.count, n);
-    rc |= m6_alloc(mc, &d.path, n * d.dmax); rc |= m6_alloc(mc, &d.path_len, n);
-    rc |= m6_alloc(mc, &d.leaf_state, n * E6_WORDS); rc |= m6_alloc(mc, &d.leaf_valid, n); rc |= m6_alloc(mc, &d.pending, n);
-    rc |= m6_alloc(mc, &d.term_value, n); rc |= m6_alloc(mc, &d.term_seat, n);
-    rc |= m6_alloc(mc, &d.nn_policy, n * AZ_MOVES); rc |= m6_alloc(mc, &d.nn_value, n);
+    rc |= m6_alloc(mc, &d.path, ns * d.dmax); rc |= m6_alloc(mc, &d.path_len, ns);
+    rc |= m6_alloc(mc, &d.leaf_state, ns * E6_WORDS); rc |= m6_alloc(mc, &d.leaf_valid, ns); rc |= m6_alloc(mc, &d.pending, ns);
+    rc |= m6_alloc(mc, &d.term_value, ns); rc |= m6_alloc(mc, &d.term_seat, ns);
+    rc |= m6_alloc(mc, &d.nn_policy, ns * AZ_MOVES); rc |= m6_alloc(mc, &d.nn_value, ns);
     rc |= m6_alloc(mc, &d.out_visits, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_pi, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_q, n * AZ_MOVES);
     rc |= m6_alloc(mc, &d.out_p, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_move, n); rc |= m6_alloc(mc, &d.out_status, n);
     rc |= m6_alloc(mc, &d.out_sumn, n); rc |= m6_alloc(mc, &d.out_table, n);
     rc |= m6_alloc(mc, &d.counters, (size_t)M6C_N);
-    if (evaluator == M6_EVAL_NN) rc |= m6_alloc(mc, &mc->d_x, n * AZ_INPUT_FLOATS);
+    if (evaluator == M6_EVAL_NN) rc |= m6_alloc(mc, &mc->d_x, ns * AZ_INPUT_FLOATS);
     if (rc) { for (void* p : mc->allocs) cudaFree(p); delete mc; return AZ_ERR_CUDA; }
     d.root_state = az_env6_state_ptr(env);
     d.c1 = 1.0f - r->dir_noise_epsi; d.c2 = r->dir_noise_epsi * r->dir_noise_value; d.cpuct = r->cpuct;
@@ -556,22 +603,26 @@ extern "C" int az_mcts6_destroy(az_mcts6* mc)
     return AZ_OK;
 }
 
-static int m6_evaluate(az_mcts6* mc, cudaStream_t s)
+// the leaves of the first k_used descent slots of every game (K for a simulation round, 1 for the root round: it uses slot 0 only)
+static int m6_evaluate(az_mcts6* mc, cudaStream_t s, int k_used)
 {
     if (mc->evaluator != M6_EVAL_NN) return AZ_OK;
     Mcts6Dev& d = mc->d;
+    const int ns = d.K * d.n;                            // the stride of the SoA leaf state
     if (mc->eval_count > 0 && mc->eval_count < d.n) {
-        const int m = mc->eval_count;
-        k_env6_encode_list<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, d.n, mc->eval_games, m, mc->d_x);
+        const int c = mc->eval_count, m = c * k_used;
+        k_env6_encode_list<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, d.n, mc->eval_games, c, k_used, mc->d_x);
         AZ_CUDA(cudaGetLastError());
         int rc = az_nn_forward_dev(mc->nn, mc->d_x, m, mc->eval_pol, mc->eval_val, mc->precision, s); if (rc) return rc;
-        k_mcts6_scatter_evals<<<(m * (AZ_MOVES + 1) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, m, d.nn_policy, d.nn_value);
+        k_mcts6_scatter_evals<<<(m * (AZ_MOVES + 1) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, c, d.n, k_used,
+                                                                             d.nn_policy, d.nn_value);
         AZ_CUDA(cudaGetLastError());
         return AZ_OK;
     }
-    k_env6_encode<<<(d.n + 127) / 128, 128, 0, s>>>(d.leaf_state, d.n, mc->d_x);
+    const int m = d.n * k_used;                          // slots j * n + game: the first k_used * n of them
+    k_env6_encode<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, m, mc->d_x);
     AZ_CUDA(cudaGetLastError());
-    return az_nn_forward_dev(mc->nn, mc->d_x, d.n, d.nn_policy, d.nn_value, mc->precision, s);
+    return az_nn_forward_dev(mc->nn, mc->d_x, m, d.nn_policy, d.nn_value, mc->precision, s);
 }
 
 static int m6_search_once(az_mcts6* mc, int pick_mode, int apply_move, int auto_reset, cudaStream_t s)
@@ -586,14 +637,15 @@ static int m6_search_once(az_mcts6* mc, int pick_mode, int apply_move, int auto_
     }
     const uint64_t* tab = az_device_tables();
     k_mcts6_begin<<<grid, M6_WARPS * 32, 0, s>>>(d);
-    k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, -1);
+    k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, -1, 1);
     AZ_CUDA(cudaGetLastError());
-    int rc = m6_evaluate(mc, s); if (rc) return rc;
-    for (int i = 0; i < mc->sims; ++i) {
-        k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, i);
+    int rc = m6_evaluate(mc, s, 1); if (rc) return rc;
+    for (int i = 0; i < mc->sims / d.K; ++i) {               // rounds of K descents per tree
+        k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, i, 1);
         AZ_CUDA(cudaGetLastError());
-        rc = m6_evaluate(mc, s); if (rc) return rc;
+        rc = m6_evaluate(mc, s, d.K); if (rc) return rc;
     }
+    if (d.K > 1) k_mcts6_sim<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, 0, 0);     // the last round's K completions; k_mcts6_finish does slot 0
     k_mcts6_finish<<<grid, M6_WARPS * 32, 0, s>>>(d, tab, pick_mode, apply_move, auto_reset);
     AZ_CUDA(cudaGetLastError());
     if (d.rec_out && apply_move) {
@@ -715,7 +767,7 @@ extern "C" int az_env6_encode(az_env6* e, float* h_x, void* stream)
     const int n = az_env6_n(e);
     float* d_x = nullptr;
     AZ_CUDA(cudaMalloc(&d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS));
-    k_env6_encode<<<(n + 127) / 128, 128, 0, s>>>(az_env6_state_ptr(e), n, d_x);
+    k_env6_encode<<<(n + 127) / 128, 128, 0, s>>>(az_env6_state_ptr(e), n, n, d_x);
     cudaError_t ce = cudaGetLastError();
     if (ce == cudaSuccess) ce = cudaMemcpyAsync(h_x, d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS, cudaMemcpyDeviceToHost, s);
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
@@ -734,7 +786,7 @@ struct az_arena6 {
     int n_agents = 0;
     Arena6Dev a;
     int32_t* d_list = nullptr;           // slots waiting for the searcher of this search (leaf-batch compaction)
-    float* d_pol_c = nullptr; float* d_val_c = nullptr;   // compacted network outputs [n][43], [n]
+    float* d_pol_c = nullptr; float* d_val_c = nullptr;   // compacted network outputs [K*n][43], [K*n] (K = the searchers' descents per tree)
     int8_t* d_status = nullptr; uint32_t* d_plies = nullptr; uint64_t games_cap = 0;   // per match game
     std::vector<uint32_t> active;        // active slots of every tick of the last match
     std::vector<void*> allocs;
@@ -780,10 +832,12 @@ extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_age
     for (int s = 0; s < E6_PLAYERS; ++s) a.seat_agent |= (uint32_t)seat_agent[s] << (4 * s);
     for (int i = 0; i < n_agents; ++i) { ar->agent[i] = agents[i]; if (agents[i]) a.searcher |= (uint8_t)(1u << i); }
     const size_t n = (size_t)a.n;
+    size_t ns = n;                                                      // the largest compacted leaf batch: K * n
+    for (int i = 0; i < n_agents; ++i) if (agents[i] && n * (size_t)agents[i]->d.K > ns) ns = n * (size_t)agents[i]->d.K;
     int rc = 0;
     rc |= a6_alloc(ar, &a.slot, n); rc |= a6_alloc(ar, &a.slot_game, n); rc |= a6_alloc(ar, &a.to_move, n);
     rc |= a6_alloc(ar, &a.res, (size_t)A6_N); rc |= a6_alloc(ar, &ar->d_list, n);
-    rc |= a6_alloc(ar, &ar->d_pol_c, n * AZ_MOVES); rc |= a6_alloc(ar, &ar->d_val_c, n);
+    rc |= a6_alloc(ar, &ar->d_pol_c, ns * AZ_MOVES); rc |= a6_alloc(ar, &ar->d_val_c, ns);
     if (rc) { for (void* p : ar->allocs) cudaFree(p); delete ar; return AZ_ERR_CUDA; }
     *out = ar;
     return AZ_OK;

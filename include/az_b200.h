@@ -340,8 +340,11 @@ AZ_API int az_env6_counters(az_env6* env, az_counters6* h_out, int reset, void* 
    seat (SIXPLAYER.md), so the same tower evaluates it */
 AZ_API int az_env6_encode(az_env6* env, float* h_x, void* stream);
 /* the six-player SEARCH of SIXPLAYER.md: the reference's MCTS with the table cleared before every search and the six-seat value rule
-   (a leaf's value belongs to the seat to move there: +v for that seat's nodes on the path, -v / 5 for the others); one descent per tree
-   per leaf batch (THREADS_PER_MCTS = 1 semantics), hyper-parameters from the env's az_rules, evaluators and precisions as az_mcts_create */
+   (a leaf's value belongs to the seat to move there: +v for that seat's nodes on the path, -v / 5 for the others); K =
+   max(1, concurrent_descents) descents per tree per leaf batch under the reference's active_N rule, the two-player lockstep schedule
+   (SIXPLAYER.md §2; K = 1 by default = THREADS_PER_MCTS = 1 semantics), hyper-parameters from the env's az_rules, evaluators and
+   precisions as az_mcts_create.  az_mcts6_create rejects K > 16 and a simulation count (mcts_simulations - mcts_simulations %
+   threads_per_mcts) that K does not divide.  Self-play, both pick modes, sample recording and the arena use the env's K. */
 typedef struct az_mcts6 az_mcts6;
 AZ_API int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int precision, az_mcts6** out);
 AZ_API int az_mcts6_destroy(az_mcts6* mcts);
