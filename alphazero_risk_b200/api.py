@@ -74,6 +74,9 @@ def lib():
         L.az_env_counters.argtypes = [vp, C.POINTER(AzCounters), C.c_int, vp]
         L.az_env_last_kernel_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.az_nn_create.argtypes = [C.c_int, C.c_int, C.POINTER(vp)]
+        L.az_nn_create_value.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
+        L.az_nn_value_outputs.argtypes = [vp]
+        L.az_nn_value_outputs.restype = C.c_int
         L.az_nn_destroy.argtypes = [vp]
         L.az_nn_blocks.argtypes = [vp]
         L.az_nn_num_vars.argtypes = [vp]
@@ -303,13 +306,15 @@ FP32, BF16 = 0, 1
 
 
 class Net:
-    """the policy/value conv ResNet (az_nn_*); weights keyed by the reference graph's TF variable names"""
+    """the policy/value conv ResNet (az_nn_*); weights keyed by the reference graph's TF variable names.  value_outputs = 6: the
+    six-seat value vector of SIXPLAYER.md §2 (output k = the value of seat (cur + k) % 6); 1 = the reference graph"""
 
-    def __init__(self, blocks=5, device=0, seed=None):
+    def __init__(self, blocks=5, device=0, seed=None, value_outputs=1):
         self.L = lib()
         h = C.c_void_p()
-        check(self.L.az_nn_create(int(blocks), device, C.byref(h)))
+        check(self.L.az_nn_create_value(int(blocks), int(value_outputs), device, C.byref(h)))
         self.h, self.blocks, self.device = h, int(blocks), device
+        self.value_outputs = int(self.L.az_nn_value_outputs(h))
         if seed is not None:
             self.init_random(seed)
 
@@ -359,9 +364,11 @@ class Net:
         check(self.L.az_nn_finalize(self.h))
 
     def forward(self, x, precision=FP32, stream=None):
+        """(policy [n, 43], value [n] with one value output, [n, 6] with six)"""
         a = np.ascontiguousarray(x, np.float32).reshape(-1, INPUT_FLOATS)
         n = a.shape[0]
-        pol, val = np.empty((n, MOVES), np.float32), np.empty(n, np.float32)
+        pol = np.empty((n, MOVES), np.float32)
+        val = np.empty(n, np.float32) if self.value_outputs == 1 else np.empty((n, self.value_outputs), np.float32)
         check(self.L.az_nn_forward(self.h, _ptr(a), n, _ptr(pol), _ptr(val), precision, stream))
         return pol, val
 
@@ -370,11 +377,12 @@ class Net:
 
     # ---- training step and checkpoints (AlphaZeroNN::train / saveCheckpoint / loadCheckpoint)
     def train_step(self, x, target_policy, target_value, stream=None):
-        """one optimizer step on a batch; returns (policy loss, value loss)"""
+        """one optimizer step on a batch; target_value [n] (one value output) or [n, 6] (six); returns (policy loss, value loss)"""
         a = np.ascontiguousarray(x, np.float32).reshape(-1, INPUT_FLOATS)
         tp = np.ascontiguousarray(target_policy, np.float32).reshape(-1, MOVES)
-        tv = np.ascontiguousarray(target_value, np.float32).reshape(-1)
-        assert tp.shape[0] == a.shape[0] == tv.shape[0]
+        tv = np.ascontiguousarray(target_value, np.float32)
+        assert tv.shape == ((a.shape[0],) if self.value_outputs == 1 else (a.shape[0], self.value_outputs)), tv.shape
+        assert tp.shape[0] == a.shape[0]
         lp, lv = C.c_float(), C.c_float()
         check(self.L.az_nn_train_step(self.h, _ptr(a), _ptr(tp), _ptr(tv), a.shape[0], C.byref(lp), C.byref(lv), stream))
         return float(lp.value), float(lv.value)
@@ -388,7 +396,8 @@ class Net:
 
     def train6(self, records, epochs, batch_size=512, seed=0, stream=None):
         """train() on six-player SAMPLE6_BYTES records (Mcts6.samples), with the six-seat input encoding; returns per-epoch
-        (policy loss, value loss) means"""
+        (policy loss, value loss) means.  With six value outputs target k of a record is the value of seat (cur + k) % 6 under the
+        record's final status"""
         r = np.ascontiguousarray(records, np.uint8).reshape(-1, SAMPLE6_BYTES)
         lp, lv = np.zeros(epochs, np.float32), np.zeros(epochs, np.float32)
         check(self.L.az_nn_train6(self.h, _ptr(r), r.shape[0], int(epochs), int(batch_size), int(seed), _ptr(lp), _ptr(lv), stream))
@@ -479,6 +488,7 @@ class Checkpoint:
 
 
 EVAL_NN, EVAL_PSEUDO, EVAL_UNIFORM = 0, 1, 2
+EVAL_PSEUDO6 = 3    # six-player search only: the pseudo evaluator with the six-seat value vector (include/az_pseudo_net.h)
 OPPONENT_SCRIPT, OPPONENT_RANDOM, OPPONENT_ALPHAZERO = 1, 2, 3
 SCRIPT_INIT = 0x00ffffff
 

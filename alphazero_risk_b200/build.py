@@ -18,11 +18,13 @@ COMMON = ["-std=c++17", "-O3", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler",
           "-I" + os.path.join(ROOT, "include"), "-I" + CSRC]
 # per translation unit flags: the game / tree code must round exactly like the reference's
 # x86 build (no FMA contraction); the network kernels may fuse.
+# A unit may include another .cu whose bytes must stay as they are (profiles/traffic.json keys its ncu captures by source hashes):
+# INCLUDED lists those files, so that a change to them rebuilds the unit.
 UNITS = {
     "az_env.cu": ["-fmad=false"],
-    "az_mcts.cu": ["-fmad=false"],
+    "az_mcts_value6.cu": ["-fmad=false"],    # az_mcts.cu (included unchanged) + az_mcts_create's six-output check
     "az_nn.cu": [],
-    "az_nn_tc.cu": [],
+    "az_nn_tc_value6.cu": [],                # az_nn_tc.cu (included unchanged) + the six-output value tail
     "az_tc_gemm.cu": [],
     "az_nn_train.cu": ["-fmad=false"],   # training step: plain fp32, same roundings whatever the compiler would contract
     "az_ckpt.cpp": [],       # host only: TensorFlow V2 checkpoint bundles
@@ -30,6 +32,9 @@ UNITS = {
     "az_mcts6.cu": ["-fmad=false"],  # six-player search: reference roundings (no FMA contraction), like az_mcts.cu
     "az_dist.cu": [],        # NCCL weight broadcast + statistics gather (NCCL itself is dlopen'ed at run time)
 }
+
+
+INCLUDED = {"az_mcts_value6.cu": ["az_mcts.cu"], "az_nn_tc_value6.cu": ["az_nn_tc.cu"]}
 
 
 def _newer(src_files, target):
@@ -51,7 +56,7 @@ def build(force=False, verbose=False):
             continue
         obj = os.path.join(OBJ, os.path.splitext(unit)[0] + ".o")
         objs.append(obj)
-        if force or _newer([src] + headers, obj):
+        if force or _newer([src] + [os.path.join(CSRC, f) for f in INCLUDED.get(unit, [])] + headers, obj):
             cmd = [nvcc] + ARCH + COMMON + extra + os.environ.get("AZ_B200_NVCC_FLAGS", "").split() + \
                   (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
             procs.append((unit, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))

@@ -9,6 +9,8 @@
 // lockstep schedule (az_mcts.cu, SIXPLAYER.md §2; checker oracle/risk6_lockstep.c): descent j of round r uses the dice of simulation
 // r * K + j and selects after descents 0..j-1 under the active_N rule; the round's leaves are evaluated as one batch of K * n positions,
 // then expanded and backed up in descent order.  K = 1 is the one-descent search (THREADS_PER_MCTS = 1 semantics).
+// An evaluator with a six-seat value vector (a 6-output network, AZ_EVAL_PSEUDO6; SIXPLAYER.md §2) gives each leaf v[6] relative to its
+// seat to move L, and a path node whose mover is s receives v[(s - L + 6) % 6] instead; a finished game backs up as above.
 //
 // Mapping: one warp per game.  The game logic of a descent (status, legal mask, transition: az_game6.cuh) runs on lane 0 over the
 // warp's shared-memory state row — the six-seat rules are thread code, shared with the environment kernels —, the table work
@@ -19,6 +21,7 @@
 //
 // Training samples (AZ_SAMPLE6_BYTES records, az_samples6.cuh): k_mcts6_finish stages (state words, pi) per real move; the game's warp
 // turns them into records in k_mcts6_rec_end once the game has ended.
+#include <algorithm>
 #include <cstring>
 #include <new>
 
@@ -39,7 +42,7 @@
 #define M6_P 32
 #define M6_Q 76
 #define M6_N 120
-enum { M6_EVAL_NN = 0, M6_EVAL_PSEUDO = 1, M6_EVAL_UNIFORM = 2 };
+enum { M6_EVAL_NN = 0, M6_EVAL_PSEUDO = 1, M6_EVAL_UNIFORM = 2, M6_EVAL_PSEUDO6 = 3 };
 enum { M6C_SIMS = 0, M6C_EVALS = 1, M6C_OVERFLOW = 2, M6C_STEPS = 3, M6C_GAMES = 4, M6C_DRAWS = 5, M6C_WIN0 = 6, M6C_N = 12 };
 
 struct Mcts6Dev {
@@ -56,7 +59,8 @@ struct Mcts6Dev {
     float* term_value;      // [K*n]   value of a descent that ended in a finished game
     int32_t* term_seat;     // [K*n]   and the seat it belongs to
     float* nn_policy;       // [K*n][43]
-    float* nn_value;        // [K*n]
+    float* nn_value;        // [K*n][vo]   the evaluator's value (vector) per descent slot
+    int vo;                 // value components per leaf: 1 (the scalar rule) or 6 (per-seat backup)
     uint32_t* root_state;   // the env6 state [28][n]
     uint32_t* out_visits; float* out_pi; uint8_t* out_move; int8_t* out_status; float* out_q; float* out_p; uint32_t* out_sumn; int32_t* out_table;
     unsigned long long* counters;
@@ -182,8 +186,9 @@ __device__ __forceinline__ int m6_select(const Mcts6Dev& m, uint32_t* nd, int la
 }
 
 // addValue up the recorded path of descent slot `slot`: +v for the nodes of the seat the leaf value belongs to, -v / 5 for every other
-// node; each step takes the descent's active_N mark off its move
-__device__ __forceinline__ void m6_backup(const Mcts6Dev& m, int slot, int gi, float v, uint32_t seat, uint32_t len, int lane)
+// node; with a value vector vec (NULL: the scalar rule; seat = the leaf's seat to move) a node whose mover is s receives
+// vec[(s - seat + 6) % 6].  Each step takes the descent's active_N mark off its move
+__device__ __forceinline__ void m6_backup(const Mcts6Dev& m, int slot, int gi, float v, uint32_t seat, uint32_t len, int lane, const float* vec)
 {
     __syncwarp();
     if (lane == 0) {
@@ -191,7 +196,7 @@ __device__ __forceinline__ void m6_backup(const Mcts6Dev& m, int slot, int gi, f
         for (int d = (int)len - 1; d >= 0; --d) {
             const uint32_t e = m.path[(size_t)slot * m.dmax + d];
             const uint32_t idx = e & 0xffffu, mv = (e >> 16) & 63u, mover = (e >> 22) & 7u;
-            const float val = mover == seat ? v : other;
+            const float val = vec ? vec[(mover + E6_PLAYERS - seat) % E6_PLAYERS] : (mover == seat ? v : other);
             uint32_t* nd = m6_node(m, gi, idx);
             const uint32_t nw = nd[M6_N + mv], N = nw & 0xffffffu;
             const float Q = __uint_as_float(nd[M6_Q + mv]);
@@ -234,6 +239,7 @@ __device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int slot, int gi,
     const uint32_t len = m.path_len[slot];
     float v = m.term_value[slot];
     uint32_t seat = (uint32_t)m.term_seat[slot];
+    const float* vec = nullptr;
     if (m.pending[slot]) {
         __syncwarp();
         if (lane < E6_WORDS) row[lane] = m.leaf_state[(size_t)lane * m.K * m.n + slot];
@@ -243,12 +249,13 @@ __device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int slot, int gi,
         if (m.eval_mode == M6_EVAL_NN) {
             p0 = m.nn_policy[(size_t)slot * AZ_MOVES + lane];
             if (lane + 32 < AZ_MOVES) p1 = m.nn_policy[(size_t)slot * AZ_MOVES + 32 + lane];
-            value = m.nn_value[slot];
-        } else if (m.eval_mode == M6_EVAL_PSEUDO) {
+            value = m.nn_value[(size_t)slot * m.vo];
+        } else if (m.eval_mode == M6_EVAL_PSEUDO || m.eval_mode == M6_EVAL_PSEUDO6) {
             const uint64_t key = m6_pn_key(row);
             p0 = az_pn_policy(key, lane);
             if (lane + 32 < AZ_MOVES) p1 = az_pn_policy(key, lane + 32);
             value = az_pn_value(key);
+            if (m.eval_mode == M6_EVAL_PSEUDO6 && lane < E6_PLAYERS) m.nn_value[(size_t)slot * E6_PLAYERS + lane] = az_pn_value6(key, lane);
         } else { p0 = 1.0f / 43.0f; p1 = lane + 32 < AZ_MOVES ? 1.0f / 43.0f : 0.0f; value = 0.0f; }
         if (!((valid >> lane) & 1ull)) p0 = 0.0f;
         if (lane + 32 >= AZ_MOVES || !((valid >> (lane + 32)) & 1ull)) p1 = 0.0f;
@@ -280,8 +287,9 @@ __device__ __forceinline__ void m6_complete(const Mcts6Dev& m, int slot, int gi,
         v = value;
         seat = (row[24] >> 16) & 0xffu;                      // the seat to move at the leaf
         if (lane == 0) { m.pending[slot] = 0; atomicAdd(&m.counters[M6C_EVALS], 1ull); }
+        if (m.vo == E6_PLAYERS) vec = m.nn_value + (size_t)slot * E6_PLAYERS;   // m6_backup's __syncwarp orders the lanes' writes
     }
-    m6_backup(m, slot, gi, v, seat, len, lane);
+    m6_backup(m, slot, gi, v, seat, len, lane, vec);
 }
 
 // one descent from the root into descent slot `slot` (AlphaZeroMCTS::search :322-377 as a loop); sim < 0: only make sure the root is
@@ -305,7 +313,7 @@ __device__ __forceinline__ void m6_descend(const Mcts6Dev& m, int slot, int gi, 
             const float tv = st == AZ_STATUS_DRAW ? 0.0f : 1.0f;
             const uint32_t seat = st == AZ_STATUS_DRAW ? mover : (uint32_t)st;
             if (lane == 0) { m.term_value[slot] = tv; m.term_seat[slot] = (int32_t)seat; m.pending[slot] = 0; }
-            m6_backup(m, slot, gi, tv, seat, depth, lane);
+            m6_backup(m, slot, gi, tv, seat, depth, lane, nullptr);
             depth = 0;
             break;
         }
@@ -498,7 +506,7 @@ __global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict_
 }
 
 // arena leaf batches: row j * count + k = the leaf of descent slot j * n + games[k] (games = the games that search this tick, k_used =
-// descent slots per game in the batch, leaf state stride K * n), and the network's outputs back to those slots
+// descent slots per game in the batch, leaf state stride K * n), and the network's outputs (policy [43], value [vo]) back to those slots
 __global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __restrict__ st, int stride, int n, const int32_t* __restrict__ games,
                                                           int count, int k_used, float* __restrict__ x)
 {
@@ -508,16 +516,16 @@ __global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __rest
     m6_encode_game(st, stride, j * n + games[k], x + (size_t)i * AZ_INPUT_FLOATS);
 }
 __global__ void __launch_bounds__(256) k_mcts6_scatter_evals(const float* __restrict__ pol_c, const float* __restrict__ val_c,
-                                                             const int32_t* __restrict__ games, int count, int n, int k_used,
+                                                             const int32_t* __restrict__ games, int count, int n, int k_used, int vo,
                                                              float* __restrict__ pol, float* __restrict__ val)
 {
     const int i = blockIdx.x * 256 + threadIdx.x;
-    if (i >= count * k_used * (AZ_MOVES + 1)) return;
-    const int c = i / (AZ_MOVES + 1), e = i - c * (AZ_MOVES + 1);
+    if (i >= count * k_used * (AZ_MOVES + vo)) return;
+    const int c = i / (AZ_MOVES + vo), e = i - c * (AZ_MOVES + vo);
     const int j = c / count, k = c - j * count;
     const size_t slot = (size_t)j * n + games[k];
     if (e < AZ_MOVES) pol[slot * AZ_MOVES + e] = pol_c[(size_t)c * AZ_MOVES + e];
-    else val[slot] = val_c[c];
+    else val[slot * vo + (e - AZ_MOVES)] = val_c[(size_t)c * vo + (e - AZ_MOVES)];
 }
 
 // ---------------------------------------------------------------- host side
@@ -535,7 +543,7 @@ struct az_mcts6 {
     // arena: only the listed games go through the network (az_arena6_play sets these around a search; the buffers are the arena's)
     const int32_t* eval_games = nullptr;    // ascending list of the searching games
     int eval_count = 0;                     // its length; 0 = every game is evaluated
-    float* eval_pol = nullptr; float* eval_val = nullptr;   // compacted outputs [count][43], [count]
+    float* eval_pol = nullptr; float* eval_val = nullptr;   // compacted outputs [count][43], [count][vo]
     std::vector<void*> allocs;
 };
 
@@ -550,7 +558,7 @@ template <class T> static int m6_alloc(az_mcts6* mc, T** p, size_t count, bool z
 extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int precision, az_mcts6** out)
 {
     AZ_REQUIRE(env && out, "NULL argument");
-    AZ_REQUIRE(evaluator >= M6_EVAL_NN && evaluator <= M6_EVAL_UNIFORM, "unknown evaluator");
+    AZ_REQUIRE(evaluator >= M6_EVAL_NN && evaluator <= M6_EVAL_PSEUDO6, "unknown evaluator");
     AZ_REQUIRE(evaluator != M6_EVAL_NN || nn != nullptr, "evaluator AZ_EVAL_NN needs a network");
     AZ_REQUIRE(precision == AZ_NN_FP32 || precision == AZ_NN_BF16, "unknown precision");
     const az_rules* r = az_env6_rules(env);
@@ -568,6 +576,7 @@ extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int preci
     Mcts6Dev& d = mc->d;
     memset(&d, 0, sizeof d);
     d.n = az_env6_n(env); d.K = K;
+    d.vo = evaluator == M6_EVAL_PSEUDO6 ? E6_PLAYERS : evaluator == M6_EVAL_NN ? nn->value_outputs : 1;
     d.cap = sims + 2;                                       // the table is cleared per search: the root + one node per simulation
     d.H = 64; while (d.H < 2 * d.cap) d.H <<= 1;
     d.dmax = 192;
@@ -578,7 +587,7 @@ extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int preci
     rc |= m6_alloc(mc, &d.path, ns * d.dmax); rc |= m6_alloc(mc, &d.path_len, ns);
     rc |= m6_alloc(mc, &d.leaf_state, ns * E6_WORDS); rc |= m6_alloc(mc, &d.leaf_valid, ns); rc |= m6_alloc(mc, &d.pending, ns);
     rc |= m6_alloc(mc, &d.term_value, ns); rc |= m6_alloc(mc, &d.term_seat, ns);
-    rc |= m6_alloc(mc, &d.nn_policy, ns * AZ_MOVES); rc |= m6_alloc(mc, &d.nn_value, ns);
+    rc |= m6_alloc(mc, &d.nn_policy, ns * AZ_MOVES); rc |= m6_alloc(mc, &d.nn_value, ns * (size_t)d.vo);
     rc |= m6_alloc(mc, &d.out_visits, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_pi, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_q, n * AZ_MOVES);
     rc |= m6_alloc(mc, &d.out_p, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_move, n); rc |= m6_alloc(mc, &d.out_status, n);
     rc |= m6_alloc(mc, &d.out_sumn, n); rc |= m6_alloc(mc, &d.out_table, n);
@@ -614,8 +623,8 @@ static int m6_evaluate(az_mcts6* mc, cudaStream_t s, int k_used)
         k_env6_encode_list<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, d.n, mc->eval_games, c, k_used, mc->d_x);
         AZ_CUDA(cudaGetLastError());
         int rc = az_nn_forward_dev(mc->nn, mc->d_x, m, mc->eval_pol, mc->eval_val, mc->precision, s); if (rc) return rc;
-        k_mcts6_scatter_evals<<<(m * (AZ_MOVES + 1) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, c, d.n, k_used,
-                                                                             d.nn_policy, d.nn_value);
+        k_mcts6_scatter_evals<<<(m * (AZ_MOVES + d.vo) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, c, d.n, k_used,
+                                                                                d.vo, d.nn_policy, d.nn_value);
         AZ_CUDA(cudaGetLastError());
         return AZ_OK;
     }
@@ -786,7 +795,7 @@ struct az_arena6 {
     int n_agents = 0;
     Arena6Dev a;
     int32_t* d_list = nullptr;           // slots waiting for the searcher of this search (leaf-batch compaction)
-    float* d_pol_c = nullptr; float* d_val_c = nullptr;   // compacted network outputs [K*n][43], [K*n] (K = the searchers' descents per tree)
+    float* d_pol_c = nullptr; float* d_val_c = nullptr;   // compacted network outputs [K*n][43], [K*n][vo] (K = the searchers' descents per tree)
     int8_t* d_status = nullptr; uint32_t* d_plies = nullptr; uint64_t games_cap = 0;   // per match game
     std::vector<uint32_t> active;        // active slots of every tick of the last match
     std::vector<void*> allocs;
@@ -832,12 +841,15 @@ extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_age
     for (int s = 0; s < E6_PLAYERS; ++s) a.seat_agent |= (uint32_t)seat_agent[s] << (4 * s);
     for (int i = 0; i < n_agents; ++i) { ar->agent[i] = agents[i]; if (agents[i]) a.searcher |= (uint8_t)(1u << i); }
     const size_t n = (size_t)a.n;
-    size_t ns = n;                                                      // the largest compacted leaf batch: K * n
-    for (int i = 0; i < n_agents; ++i) if (agents[i] && n * (size_t)agents[i]->d.K > ns) ns = n * (size_t)agents[i]->d.K;
+    size_t ns = n, nv = n;                                              // the largest compacted leaf batch: K * n, and its values K * n * vo
+    for (int i = 0; i < n_agents; ++i) if (agents[i]) {
+        ns = std::max(ns, n * (size_t)agents[i]->d.K);
+        nv = std::max(nv, n * (size_t)agents[i]->d.K * (size_t)agents[i]->d.vo);
+    }
     int rc = 0;
     rc |= a6_alloc(ar, &a.slot, n); rc |= a6_alloc(ar, &a.slot_game, n); rc |= a6_alloc(ar, &a.to_move, n);
     rc |= a6_alloc(ar, &a.res, (size_t)A6_N); rc |= a6_alloc(ar, &ar->d_list, n);
-    rc |= a6_alloc(ar, &ar->d_pol_c, ns * AZ_MOVES); rc |= a6_alloc(ar, &ar->d_val_c, ns);
+    rc |= a6_alloc(ar, &ar->d_pol_c, ns * AZ_MOVES); rc |= a6_alloc(ar, &ar->d_val_c, nv);
     if (rc) { for (void* p : ar->allocs) cudaFree(p); delete ar; return AZ_ERR_CUDA; }
     *out = ar;
     return AZ_OK;

@@ -5,7 +5,8 @@
 // BOARD-ROW axis (7 parameters: build_graph.py:68 passes axis=1 on an NHWC tensor) -> ReLU ->
 // BLOCKS x {conv3x3, BN(256), ReLU, conv3x3, BN(256), +skip, ReLU} -> policy head conv1x1->2, BN,
 // ReLU, flatten(84, NHWC order), dense 43 + bias, softmax ; value head conv1x1->1, BN, ReLU,
-// flatten(42), dense 256 + bias, ReLU, dense 1 + bias, tanh.  Inference BN:
+// flatten(42), dense 256 + bias, ReLU, dense 1 + bias, tanh (dense value_outputs = 6 for the six-seat value vector of
+// SIXPLAYER.md §2, each output through tanh).  Inference BN:
 // y = (x - moving_mean) * (gamma * rsqrt(moving_variance + 0.001)) + beta.
 // Replaces the TensorFlow session->Run of neural_network/alphazero_nn.cpp:247-248, :339-340.
 #include <cmath>
@@ -59,8 +60,8 @@ static void build_inventory(az_nn* nn)
     add_bn(nn, "bn_v", 1);
     add_var(nn, "dense_1/kernel", { 42, 256 }, glorot(42, 256), 0.0f);
     add_var(nn, "dense_1/bias", { 256 }, 0.0f, 0.0f);
-    add_var(nn, "dense_2/kernel", { 256, 1 }, glorot(256, 1), 0.0f);
-    add_var(nn, "dense_2/bias", { 1 }, 0.0f, 0.0f);
+    add_var(nn, "dense_2/kernel", { 256, nn->value_outputs }, glorot(256, nn->value_outputs), 0.0f);
+    add_var(nn, "dense_2/bias", { nn->value_outputs }, 0.0f, 0.0f);
 }
 
 const float* az_nn_host_var(const az_nn* nn, const std::string& name)
@@ -185,10 +186,12 @@ __device__ __forceinline__ float warp_sum(float v)
     return v;
 }
 
+// VO = value outputs (AzHeadParams::vo); with VO = 1 the arithmetic is the one-output graph's, operation for operation
+template <int VO>
 __global__ void __launch_bounds__(256) k_nn_heads_fp32(const float* __restrict__ act, int n, AzHeadParams hp,
-                                                        float* __restrict__ policy /*[n][43]*/, float* __restrict__ value /*[n]*/)
+                                                        float* __restrict__ policy /*[n][43]*/, float* __restrict__ value /*[n][VO]*/)
 {
-    __shared__ float s_pi[84], s_v[42], s_h[256], s_logit[43], s_red[8];
+    __shared__ float s_pi[84], s_v[42], s_h[256], s_logit[43], s_red[VO][8];
     const int b = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     // 1x1 convs: every warp takes cells warp, warp+8, ...
     for (int p = warp; p < 42; p += 8) {
@@ -220,14 +223,17 @@ __global__ void __launch_bounds__(256) k_nn_heads_fp32(const float* __restrict__
         s_h[threadIdx.x] = fmaxf(s, 0.0f);
     }
     __syncthreads();
-    // dense 256 -> 1 (+bias, tanh)
-    float part = warp_sum(s_h[threadIdx.x] * hp.dense2_w[threadIdx.x]);
-    if (lane == 0) s_red[warp] = part;
+    // dense 256 -> VO (+bias, tanh)
+#pragma unroll
+    for (int k = 0; k < VO; ++k) {
+        const float part = warp_sum(s_h[threadIdx.x] * hp.dense2_w[threadIdx.x * VO + k]);
+        if (lane == 0) s_red[k][warp] = part;
+    }
     __syncthreads();
-    if (threadIdx.x == 0) {
-        float s = hp.dense2_b[0];
-        for (int i = 0; i < 8; ++i) s += s_red[i];
-        value[b] = tanhf(s);
+    if (threadIdx.x < VO) {
+        float s = hp.dense2_b[threadIdx.x];
+        for (int i = 0; i < 8; ++i) s += s_red[threadIdx.x][i];
+        value[(size_t)b * VO + threadIdx.x] = tanhf(s);
     }
     // softmax over 43 logits
     if (warp == 0) {
@@ -250,17 +256,18 @@ static int upload(float** d, const float* h, size_t count)
     return AZ_OK;
 }
 
-extern "C" int az_nn_create(int blocks, int device, az_nn** out)
+extern "C" int az_nn_create_value(int blocks, int value_outputs, int device, az_nn** out)
 {
     AZ_REQUIRE(out != nullptr, "out is NULL");
     AZ_REQUIRE(blocks >= 1 && blocks <= 26, "blocks must be in [1, 26]");
+    AZ_REQUIRE(value_outputs == 1 || value_outputs == 6, "value_outputs must be 1 or 6");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); az_set_error("no CUDA device: libaz_b200 has no CPU fallback"); return AZ_ERR_NO_DEVICE; }
     AZ_REQUIRE(device >= 0 && device < ndev, "device index out of range");
     AzDeviceGuard guard(device);
     az_nn* nn = new (std::nothrow) az_nn();
     AZ_REQUIRE(nn != nullptr, "out of host memory");
-    nn->blocks = blocks; nn->device = device;
+    nn->blocks = blocks; nn->device = device; nn->value_outputs = value_outputs;
     build_inventory(nn);
     int8_t nb[42 * 9];
     for (int p = 0; p < 42; ++p)
@@ -274,6 +281,8 @@ extern "C" int az_nn_create(int blocks, int device, az_nn** out)
     *out = nn;
     return AZ_OK;
 }
+
+extern "C" int az_nn_create(int blocks, int device, az_nn** out) { return az_nn_create_value(blocks, 1, device, out); }
 
 extern "C" int az_nn_destroy(az_nn* nn)
 {
@@ -290,6 +299,7 @@ extern "C" int az_nn_destroy(az_nn* nn)
 extern "C" int az_nn_num_vars(const az_nn* nn) { return nn ? (int)nn->vars.size() : 0; }
 extern "C" size_t az_nn_num_params(const az_nn* nn) { return nn ? nn->blob.size() : 0; }
 extern "C" int az_nn_blocks(const az_nn* nn) { return nn ? nn->blocks : 0; }
+extern "C" int az_nn_value_outputs(const az_nn* nn) { return nn ? nn->value_outputs : 0; }
 
 extern "C" int az_nn_var_info(const az_nn* nn, int i, const char** name, size_t* count, int* rank, int* shape4)
 {
@@ -406,7 +416,7 @@ int az_nn_reserve(az_nn* nn, int n)
     for (int i = 0; i < 3; ++i) AZ_CUDA(cudaMalloc(&nn->d_act[i], sizeof(float) * (size_t)n * 42 * AZ_NN_CH));
     AZ_CUDA(cudaMalloc(&nn->d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS));
     AZ_CUDA(cudaMalloc(&nn->d_policy, sizeof(float) * (size_t)n * 43));
-    AZ_CUDA(cudaMalloc(&nn->d_value, sizeof(float) * (size_t)n));
+    AZ_CUDA(cudaMalloc(&nn->d_value, sizeof(float) * (size_t)n * nn->value_outputs));
     nn->cap = n;
     return AZ_OK;
 }
@@ -419,6 +429,7 @@ AzHeadParams az_nn_head_params(const az_nn* nn)
     hp.v_w = az_nn_dev_var(nn, "v/kernel"); hp.bn_v = az_nn_dev_var(nn, "bn_v/gamma");
     hp.dense1_w = az_nn_dev_var(nn, "dense_1/kernel"); hp.dense1_b = az_nn_dev_var(nn, "dense_1/bias");
     hp.dense2_w = az_nn_dev_var(nn, "dense_2/kernel"); hp.dense2_b = az_nn_dev_var(nn, "dense_2/bias");
+    hp.vo = nn->value_outputs;
     return hp;
 }
 
@@ -441,7 +452,8 @@ static int forward_fp32(az_nn* nn, const float* d_x, int n, float* d_policy, flo
         int o = cur; cur = nxt; nxt = o;
     }
     float* a = buf[cur];
-    k_nn_heads_fp32<<<n, 256, 0, s>>>(a, n, az_nn_head_params(nn), d_policy, d_value);
+    if (nn->value_outputs == 6) k_nn_heads_fp32<6><<<n, 256, 0, s>>>(a, n, az_nn_head_params(nn), d_policy, d_value);
+    else k_nn_heads_fp32<1><<<n, 256, 0, s>>>(a, n, az_nn_head_params(nn), d_policy, d_value);
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
 }
@@ -454,6 +466,7 @@ extern "C" int az_nn_forward_dev(az_nn* nn, const float* d_x, int n, float* d_po
     AzDeviceGuard guard(nn->device);
     int rc = finalize(nn); if (rc) return rc;
     rc = az_nn_reserve(nn, n); if (rc) return rc;
+    if (precision == AZ_NN_BF16 && nn->value_outputs == 6) return az_nn_tc_forward_value6(nn, d_x, n, d_policy, d_value, (cudaStream_t)stream);
     if (precision == AZ_NN_BF16) return az_nn_tc_forward(nn, d_x, nullptr, n, d_policy, d_value, (cudaStream_t)stream);
     return forward_fp32(nn, d_x, n, d_policy, d_value, (cudaStream_t)stream);
 }
@@ -470,7 +483,7 @@ extern "C" int az_nn_forward(az_nn* nn, const float* h_x, int n, float* h_policy
     rc = az_nn_forward_dev(nn, nn->d_x, n, nn->d_policy, nn->d_value, precision, stream);
     if (rc) return rc;
     AZ_CUDA(cudaMemcpyAsync(h_policy, nn->d_policy, sizeof(float) * (size_t)n * 43, cudaMemcpyDeviceToHost, s));
-    AZ_CUDA(cudaMemcpyAsync(h_value, nn->d_value, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaMemcpyAsync(h_value, nn->d_value, sizeof(float) * (size_t)n * nn->value_outputs, cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaStreamSynchronize(s));
     return AZ_OK;
 }

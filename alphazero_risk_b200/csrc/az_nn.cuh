@@ -23,6 +23,7 @@ struct AzVar {
 
 struct AzHeadParams {
     const float *pi_w, *bn_pi, *dense_w, *dense_b, *v_w, *bn_v, *dense1_w, *dense1_b, *dense2_w, *dense2_b;
+    int vo;                           // value outputs: 1, or 6 (seat (cur + k) % 6); dense2_w is [256][vo]
 };
 
 struct AzTcState;   // az_nn_tc.cu
@@ -30,6 +31,7 @@ struct AzTrainState; // az_nn_train.cu
 
 struct az_nn {
     int blocks = 5, device = 0;
+    int value_outputs = 1;            // 1 = the reference graph; 6 = the six-seat value vector (SIXPLAYER.md §2)
     std::vector<AzVar> vars;
     std::map<std::string, int> index;
     std::vector<float> blob;          // every variable, fp32, TF layouts (HWIO kernels), inventory order
@@ -59,6 +61,8 @@ void az_nn_tc_release(az_nn* nn);
 // shared_device: another forward shares the device right now (no programmatic dependent launch between the layers, see az_nn_tc.cu)
 int az_nn_tc_forward(az_nn* nn, const float* d_x, const uint32_t* d_env_state, int n, float* d_policy, float* d_value, cudaStream_t s,
                      int state_stride = 0, int scratch_set = 0, bool shared_device = false);
+// the same forward for a network with six value outputs: value [n][6] (az_nn_tc_value6.cu)
+int az_nn_tc_forward_value6(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, cudaStream_t s);
 
 // raw 3x3 convolution of the training step on the tower kernel (az_nn_tc.cu): fp32 [n * 42][256] in, fp32 HWIO device weights
 // [9][256][256] (flip = 1: the data gradient's kernel), fp32 [n * 42][256] out; bf16 operands, fp32 accumulation

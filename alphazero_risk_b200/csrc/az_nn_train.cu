@@ -6,7 +6,7 @@
 //   forward with FusedBatchNormV3(is_training = true): batch mean / biased batch variance, epsilon 0.001; moving statistics move to the
 //   batch mean and the unbiased batch variance with momentum 0.99; the stem's BatchNorm runs over the board-row axis (7 groups);
 //   loss = softmax cross-entropy(policy logits, target pi) [batch mean] + mean squared error(tanh value, target z) + 0.001 * sum of the
-//   squared kernels; Adam(lr 0.001, beta1 0.9, beta2 0.999, epsilon 1e-8) in TensorFlow's formulation.
+//   squared kernels (a six-output value head, SIXPLAYER.md §2: the mean over all n * 6 squared errors); Adam(lr 0.001, beta1 0.9, beta2 0.999, epsilon 1e-8) in TensorFlow's formulation.
 // AlphaZeroNN::saveCheckpoint / loadCheckpoint (alphazero_nn.cpp:189-214) exchange the 163 tensors of the graph's Saver: variables, BN
 // moving statistics, Adam slots "<var>/optimize" (m) and "<var>/optimize_1" (v), beta1_power, beta2_power (az_ckpt.cpp holds the format).
 //
@@ -76,18 +76,18 @@ struct AzTrainState {
     float* d_wT = nullptr;                             // [9][256][256] flipped + transposed kernel of the layer being back-propagated
     float* d_wpart = nullptr;                          // [TR_WG_SPLITS][9][256][256]
     float *d_hz = nullptr, *d_hg = nullptr;            // heads: raw 1x1 outputs / gradients [cap*42][4] (pi0, pi1, v, unused)
-    float *d_hfeat = nullptr;                          // per board: s_pi[84] dlogit[43] s_v[42] h[256] dh[256] dout[1] loss[2] -> 684 floats
+    float *d_hfeat = nullptr;                          // per board: s_pi[84] dlogit[43] s_v[42] h[256] dh[256] dout[vo <= 6] loss[2]
     float *d_hpart = nullptr;                          // [TR_STAT_CHUNKS][256][3] 1x1 kernel gradient partials
-    float *d_tp = nullptr, *d_tv = nullptr, *d_loss = nullptr;
+    float *d_tp = nullptr, *d_tv = nullptr, *d_loss = nullptr;   // d_tv: [cap][value outputs]
 };
-#define HF_STRIDE 688
+#define HF_STRIDE 696
 #define HF_SPI 0
 #define HF_DLOGIT 84
 #define HF_SV 128
 #define HF_H 172
 #define HF_DH 428
-#define HF_DOUT 684
-#define HF_LOSS 685
+#define HF_DOUT 684      // [vo]
+#define HF_LOSS 690
 
 __constant__ int8_t c_tnb[42 * 9];       // neighbour of board cell p for tap t, -1 outside the board (SAME padding)
 
@@ -550,10 +550,11 @@ __global__ void __launch_bounds__(256) k_tr_head_stats(const float* __restrict__
 
 // one block per board: BN + ReLU of the three head channels, dense layers, softmax / tanh, the two losses, and the backward pass down to
 // the gradient with respect to the BN outputs (masked by the ReLU) -> hg.  The per-board vectors the weight gradients need go to hfeat.
+// hp.vo value outputs: tv [n][vo], the value loss is the mean over the n * vo squared errors, dh = sum_k dout_k * dense_2[:, k]
 __global__ void __launch_bounds__(256) k_tr_head_board(const float* __restrict__ hz, const float* __restrict__ hstats, AzHeadParams hp, const float* __restrict__ tp,
                                                         const float* __restrict__ tv, int n, float* __restrict__ hg, float* __restrict__ hfeat)
 {
-    __shared__ float s_pi[84], s_v[42], s_h[256], s_dh[256], s_logit[43], s_dlogit[43], s_red[8], s_do;
+    __shared__ float s_pi[84], s_v[42], s_h[256], s_dh[256], s_logit[43], s_dlogit[43], s_red[6][8], s_do[6], s_d2[6];
     const int b = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     float* hf = hfeat + (size_t)b * HF_STRIDE;
     if (threadIdx.x < 42) {
@@ -576,16 +577,21 @@ __global__ void __launch_bounds__(256) k_tr_head_board(const float* __restrict__
         s_h[threadIdx.x] = fmaxf(s, 0.0f);
     }
     __syncthreads();
-    float part = tr_warp_sum(s_h[threadIdx.x] * hp.dense2_w[threadIdx.x]);
-    if (lane == 0) s_red[warp] = part;
+    const int vo = hp.vo;
+    for (int k = 0; k < vo; ++k) {
+        const float part = tr_warp_sum(s_h[threadIdx.x] * hp.dense2_w[threadIdx.x * vo + k]);
+        if (lane == 0) s_red[k][warp] = part;
+    }
     __syncthreads();
-    const float inv_n = 1.0f / (float)n;
-    if (threadIdx.x == 0) {
-        float s = hp.dense2_b[0];
-        for (int i = 0; i < 8; ++i) s += s_red[i];
-        const float v = tanhf(s), d = v - tv[b];
-        s_do = 2.0f * d * inv_n * (1.0f - v * v);               // d(mean squared error) / d(pre-tanh output)
-        hf[HF_DOUT] = s_do; hf[HF_LOSS + 1] = d * d;
+    const float inv_n = 1.0f / (float)n, inv_nv = 1.0f / (float)(n * vo);
+    if (threadIdx.x < vo) {
+        const int k = threadIdx.x;
+        float s = hp.dense2_b[k];
+        for (int i = 0; i < 8; ++i) s += s_red[k][i];
+        const float v = tanhf(s), d = v - tv[(size_t)b * vo + k];
+        s_do[k] = 2.0f * d * inv_nv * (1.0f - v * v);           // d(mean squared error) / d(pre-tanh output)
+        s_d2[k] = d * d;
+        hf[HF_DOUT + k] = s_do[k];
     }
     if (warp == 1) {                                             // softmax cross-entropy of this board and its logit gradient
         const float l0 = s_logit[lane], l1 = lane < 11 ? s_logit[32 + lane] : -INFINITY;
@@ -602,7 +608,16 @@ __global__ void __launch_bounds__(256) k_tr_head_board(const float* __restrict__
         if (lane == 0) hf[HF_LOSS] = loss;
     }
     __syncthreads();
-    s_dh[threadIdx.x] = s_h[threadIdx.x] > 0.0f ? s_do * hp.dense2_w[threadIdx.x] : 0.0f;
+    if (threadIdx.x == 0) {                                      // this board's squared errors, in component order
+        float l = s_d2[0];
+        for (int k = 1; k < vo; ++k) l += s_d2[k];
+        hf[HF_LOSS + 1] = l;
+    }
+    {
+        float g = s_do[0] * hp.dense2_w[threadIdx.x * vo];
+        for (int k = 1; k < vo; ++k) g += s_do[k] * hp.dense2_w[threadIdx.x * vo + k];
+        s_dh[threadIdx.x] = s_h[threadIdx.x] > 0.0f ? g : 0.0f;
+    }
     __syncthreads();
     if (threadIdx.x < 84) {                                      // gradient w.r.t. the flattened policy features
         float s = 0.0f;
@@ -622,8 +637,9 @@ __global__ void __launch_bounds__(256) k_tr_head_board(const float* __restrict__
     hf[HF_DH + threadIdx.x] = s_dh[threadIdx.x];
 }
 
-// gradients of the dense layers: one thread per output element, boards summed in order
-__global__ void __launch_bounds__(256) k_tr_head_dense_grad(const float* __restrict__ hfeat, int n, float* __restrict__ g_dense_w, float* __restrict__ g_dense_b,
+// gradients of the dense layers: one thread per output element, boards summed in order; vo value outputs (dense_2 is [256][vo])
+#define TR_HEAD_D1_END (84 * 43 + 43 + 42 * 256 + 256)
+__global__ void __launch_bounds__(256) k_tr_head_dense_grad(const float* __restrict__ hfeat, int n, int vo, float* __restrict__ g_dense_w, float* __restrict__ g_dense_b,
                                                              float* __restrict__ g_d1_w, float* __restrict__ g_d1_b, float* __restrict__ g_d2_w, float* __restrict__ g_d2_b,
                                                              float* __restrict__ loss2)
 {
@@ -632,14 +648,14 @@ __global__ void __launch_bounds__(256) k_tr_head_dense_grad(const float* __restr
     if (i < 84 * 43) { a_off = HF_SPI + i / 43; b_off = HF_DLOGIT + i % 43; dst = g_dense_w + i; }
     else if (i < 84 * 43 + 43) { a_off = -1; b_off = HF_DLOGIT + (i - 84 * 43); dst = g_dense_b + (i - 84 * 43); }
     else if (i < 84 * 43 + 43 + 42 * 256) { const int k = i - (84 * 43 + 43); a_off = HF_SV + k / 256; b_off = HF_DH + k % 256; dst = g_d1_w + k; }
-    else if (i < 84 * 43 + 43 + 42 * 256 + 256) { const int k = i - (84 * 43 + 43 + 42 * 256); a_off = -1; b_off = HF_DH + k; dst = g_d1_b + k; }
-    else if (i < 84 * 43 + 43 + 42 * 256 + 512) { const int k = i - (84 * 43 + 43 + 42 * 256 + 256); a_off = HF_H + k; b_off = HF_DOUT; dst = g_d2_w + k; }
-    else if (i == 84 * 43 + 43 + 42 * 256 + 512) { a_off = -1; b_off = HF_DOUT; dst = g_d2_b; }
-    else if (i <= 84 * 43 + 43 + 42 * 256 + 514) {               // the two batch losses (means)
-        const int k = i - (84 * 43 + 43 + 42 * 256 + 513);
+    else if (i < TR_HEAD_D1_END) { const int k = i - (84 * 43 + 43 + 42 * 256); a_off = -1; b_off = HF_DH + k; dst = g_d1_b + k; }
+    else if (i < TR_HEAD_D1_END + 256 * vo) { const int k = i - TR_HEAD_D1_END; a_off = HF_H + k / vo; b_off = HF_DOUT + k % vo; dst = g_d2_w + k; }
+    else if (i < TR_HEAD_D1_END + 257 * vo) { const int k = i - (TR_HEAD_D1_END + 256 * vo); a_off = -1; b_off = HF_DOUT + k; dst = g_d2_b + k; }
+    else if (i < TR_HEAD_D1_END + 257 * vo + 2) {                // the two batch losses (means: over n boards, over n * vo value errors)
+        const int k = i - (TR_HEAD_D1_END + 257 * vo);
         float s = 0.0f;
         for (int b = 0; b < n; ++b) s += hfeat[(size_t)b * HF_STRIDE + HF_LOSS + k];
-        loss2[k] = s / (float)n;
+        loss2[k] = s / (float)(k == 1 ? n * vo : n);
         return;
     } else return;
     float s = 0.0f;
@@ -649,7 +665,7 @@ __global__ void __launch_bounds__(256) k_tr_head_dense_grad(const float* __restr
     }
     *dst = s;
 }
-#define TR_HEAD_DENSE_ELEMS (84 * 43 + 43 + 42 * 256 + 515)
+static inline int tr_head_dense_elems(int vo) { return TR_HEAD_D1_END + 257 * vo + 2; }
 
 // BN backward of the head channels per row, then the gradient into the tower output: dA[r][c] = sum_k dz[r][k] * W[c][k].
 // dz overwrites hg (the 1x1 kernels' gradient needs it).  One warp per row.
@@ -749,16 +765,18 @@ __global__ void __launch_bounds__(64) k_tr_unpack_samples(const uint8_t* __restr
 }
 
 // six-player records (az_samples6.cuh) -> the six-seat input planes of each record's image (e6_encode_position, the encoding the
-// six-player search evaluates its leaves with) + value and policy targets; one thread per sample
+// six-player search evaluates its leaves with) + value and policy targets; one thread per sample.  vo = 6: tv [n][6], target k =
+// s6_value(status, (cur + k) % 6) (component 0 is the record's stored value)
 __global__ void __launch_bounds__(128) k_tr_unpack_samples6(const uint8_t* __restrict__ rec, const uint32_t* __restrict__ order, int n,
-                                                            float* __restrict__ x, float* __restrict__ tp, float* __restrict__ tv)
+                                                            float* __restrict__ x, float* __restrict__ tp, float* __restrict__ tv, int vo)
 {
     const int b = blockIdx.x * 128 + threadIdx.x;
     if (b >= n) return;
     const uint8_t* r = rec + (size_t)order[b] * S6_BYTES;
     e6_encode_position(r, r + AZ_LANDS, r[S6_CUR], r[S6_PHASE], r[S6_ATTACKS], r[S6_ALLOW_DRAW], x + (size_t)b * AZ_INPUT_FLOATS);
     const float* f = (const float*)r;                       // records are 4-byte aligned (288-byte stride)
-    tv[b] = f[S6_VALUE / 4];
+    if (vo == 1) tv[b] = f[S6_VALUE / 4];
+    else for (int k = 0; k < vo; ++k) tv[(size_t)b * vo + k] = s6_value((int8_t)r[S6_STATUS], (r[S6_CUR] + (uint32_t)k) % E6_PLAYERS);
     for (int i = 0; i < AZ_MOVES; ++i) tp[(size_t)b * AZ_MOVES + i] = f[S6_PI / 4 + i];
 }
 
@@ -842,7 +860,7 @@ static int train_reserve(az_nn* nn, AzTrainState* t, int n)
     AZ_CUDA(cudaMalloc(&t->d_x, sizeof(float) * (size_t)n * 42 * AZ_NN_IN_CH));
     AZ_CUDA(cudaMalloc(&t->d_hz, sizeof(float) * (size_t)n * 42 * 4)); AZ_CUDA(cudaMalloc(&t->d_hg, sizeof(float) * (size_t)n * 42 * 4));
     AZ_CUDA(cudaMalloc(&t->d_hfeat, sizeof(float) * (size_t)n * HF_STRIDE));
-    AZ_CUDA(cudaMalloc(&t->d_tp, sizeof(float) * (size_t)n * 43)); AZ_CUDA(cudaMalloc(&t->d_tv, sizeof(float) * (size_t)n));
+    AZ_CUDA(cudaMalloc(&t->d_tp, sizeof(float) * (size_t)n * 43)); AZ_CUDA(cudaMalloc(&t->d_tv, sizeof(float) * (size_t)n * nn->value_outputs));
     {   // GEMM operands of the tensor-core path: A = max(im2col [Mp][9*256], transposed im2col [9*256][Kp]), B = max(weights, dz^T)
         const size_t mp = tr_mp(n * 42), kpw = tr_kp(n * 42);
         const size_t a_elems = (size_t)9 * TR_CH * (mp > kpw ? mp : kpw), b_elems = (size_t)TR_CH * (kpw > (size_t)9 * TR_CH ? kpw : (size_t)9 * TR_CH);
@@ -1003,7 +1021,7 @@ static int train_step_dev(az_nn* nn, const float* d_x, const float* d_tp, const 
                                       dvar(nn, "bn_v/moving_mean"), dvar(nn, "bn_v/moving_variance"), nullptr, nullptr, nullptr, nullptr);
     k_tr_head_board<<<(unsigned)n, 256, 0, s>>>(t->d_hz, hst, hp, d_tp, d_tv, n, t->d_hg, t->d_hfeat);
     // ---- backward: heads
-    k_tr_head_dense_grad<<<(TR_HEAD_DENSE_ELEMS + 255) / 256, 256, 0, s>>>(t->d_hfeat, n, gvar(nn, t, "dense/kernel"), gvar(nn, t, "dense/bias"),
+    k_tr_head_dense_grad<<<(tr_head_dense_elems(hp.vo) + 255) / 256, 256, 0, s>>>(t->d_hfeat, n, hp.vo, gvar(nn, t, "dense/kernel"), gvar(nn, t, "dense/bias"),
                                                                            gvar(nn, t, "dense_1/kernel"), gvar(nn, t, "dense_1/bias"),
                                                                            gvar(nn, t, "dense_2/kernel"), gvar(nn, t, "dense_2/bias"), t->d_loss);
     k_tr_head_stats<<<1, 256, 0, s>>>(t->d_hz, t->d_hg, rows, 1, hst, nullptr, nullptr, nullptr, nullptr,
@@ -1054,7 +1072,7 @@ extern "C" int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_targ
     int rc = train_reserve(nn, t, n); if (rc) return rc;
     AZ_CUDA(cudaMemcpyAsync(t->d_x, h_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaMemcpyAsync(t->d_tp, h_target_policy, sizeof(float) * (size_t)n * 43, cudaMemcpyHostToDevice, s));
-    AZ_CUDA(cudaMemcpyAsync(t->d_tv, h_target_value, sizeof(float) * (size_t)n, cudaMemcpyHostToDevice, s));
+    AZ_CUDA(cudaMemcpyAsync(t->d_tv, h_target_value, sizeof(float) * (size_t)n * nn->value_outputs, cudaMemcpyHostToDevice, s));
     float loss[2] = { 0.0f, 0.0f };
     rc = train_step_dev(nn, t->d_x, t->d_tp, t->d_tv, n, loss, s); if (rc) return rc;
     if (loss_policy) *loss_policy = loss[0];
@@ -1063,14 +1081,15 @@ extern "C" int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_targ
 }
 
 // the record -> (input planes, targets) step of a training loop: batch b of an epoch unpacks the n records order[0..n) of d_rec
-typedef void (*TrUnpack)(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s);
-static void tr_unpack_samples(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s)
+// (tv holds vo values per record)
+typedef void (*TrUnpack)(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, cudaStream_t s);
+static void tr_unpack_samples(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int, cudaStream_t s)
 {
     k_tr_unpack_samples<<<(unsigned)n, 64, 0, s>>>(d_rec, d_order, n, x, tp, tv);
 }
-static void tr_unpack_samples6(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, cudaStream_t s)
+static void tr_unpack_samples6(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, cudaStream_t s)
 {
-    k_tr_unpack_samples6<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv);
+    k_tr_unpack_samples6<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv, vo);
 }
 
 // AlphaZeroNN::train (alphazero_nn.cpp:351-410): `epochs` passes over the samples in shuffled order, whole batches of batch_size only
@@ -1104,7 +1123,7 @@ static int train_records(az_nn* nn, const char* who, const uint8_t* h_records, s
         // the batches of an epoch are enqueued back to back; the losses are accumulated on the device and read once per epoch
         if (ce == cudaSuccess) ce = cudaMemsetAsync(d_acc, 0, 2 * sizeof(double), s);
         for (size_t b = 0; b < batches && ce == cudaSuccess && rc == AZ_OK; ++b) {
-            unpack(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv, s);
+            unpack(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv, nn->value_outputs, s);
             rc = train_step_dev(nn, t->d_x, t->d_tp, t->d_tv, batch_size, nullptr, s);
             if (rc == AZ_OK) k_tr_loss_accum<<<1, 32, 0, s>>>(t->d_loss, d_acc);
         }
@@ -1127,6 +1146,7 @@ extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records
     AZ_REQUIRE(nn && h_records, "NULL argument");
     AZ_REQUIRE(epochs >= 1 && batch_size >= 2, "epochs must be >= 1 and batch_size >= 2");
     AZ_REQUIRE(n_records >= (size_t)batch_size, "fewer samples than one batch");
+    AZ_REQUIRE(nn->value_outputs == 1, "az_nn_train: two-player records hold one value target; the network has six value outputs");
     AzDeviceGuard guard(nn->device);
     return train_records(nn, "az_nn_train", h_records, n_records, AZ_SAMPLE_BYTES, tr_unpack_samples, epochs, batch_size, seed,
                          h_epoch_loss_policy, h_epoch_loss_value, (cudaStream_t)stream);

@@ -166,8 +166,13 @@ typedef struct az_nn az_nn;
 /* the conv ResNet of /root/reference/python/src/build_graph.py:54-90 with `blocks` residual blocks
    (BLOCKS: 5 = shipped GraphDefs python/model/model_*_5.pb, 20 = CMake default) */
 AZ_API int az_nn_create(int blocks, int device, az_nn** out);
+/* the same network with value_outputs (1 or 6) value outputs: dense_2/kernel [256][value_outputs], dense_2/bias [value_outputs], each
+   output through tanh.  6 = the six-seat value vector of SIXPLAYER.md §2: output k is the value of seat (cur + k) % 6, cur = the seat
+   to move in the encoded position.  az_nn_create is value_outputs = 1, the reference graph */
+AZ_API int az_nn_create_value(int blocks, int value_outputs, int device, az_nn** out);
 AZ_API int az_nn_destroy(az_nn* nn);
 AZ_API int az_nn_blocks(const az_nn* nn);
+AZ_API int az_nn_value_outputs(const az_nn* nn);
 AZ_API int az_nn_num_vars(const az_nn* nn);
 AZ_API size_t az_nn_num_params(const az_nn* nn);
 /* i-th variable: TF variable name (e.g. "res0a_branch2a/kernel"), element count, rank, shape (HWIO kernels) */
@@ -182,7 +187,7 @@ AZ_API int az_nn_import_blob(az_nn* nn, const float* h_in, size_t count);
 AZ_API int az_nn_init_random(az_nn* nn, uint64_t seed);
 AZ_API int az_nn_finalize(az_nn* nn);
 /* AlphaZeroNN::predict / processBatchPrediction (alphazero_nn.cpp:236-267, 333-349):
-   x fp32 [n][7][6][13] -> policy [n][43] (softmax), value [n] (tanh) */
+   x fp32 [n][7][6][13] -> policy [n][43] (softmax), value [n][value_outputs] (tanh; [n] for the one-output graph) */
 AZ_API int az_nn_forward(az_nn* nn, const float* h_x, int n, float* h_policy, float* h_value, int precision, void* stream);
 AZ_API int az_nn_forward_dev(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, int precision, void* stream);
 
@@ -190,11 +195,13 @@ AZ_API int az_nn_forward_dev(az_nn* nn, const float* d_x, int n, float* d_policy
 /* One run of the graph's "optimize" op (AlphaZeroNN::train inner loop, neural_network/alphazero_nn.cpp:389-390;
    python/src/build_graph.py:92-106): training-mode forward (batch statistics, moving averages updated with momentum 0.99), softmax
    cross-entropy + mean squared error + 0.001 * L2 of the kernels, Adam(0.001, 0.9, 0.999, 1e-8).  x [n][7][6][13], target policy
-   [n][43], target value [n]; returns the batch's two losses (TF_OUTPUT_LOSS_POLICY / _VALUE).  fp32 on CUDA cores, deterministic. */
+   [n][43], target value [n][value_outputs]; returns the batch's two losses (TF_OUTPUT_LOSS_POLICY / _VALUE; the value loss is the
+   mean over all n * value_outputs squared errors).  fp32 on CUDA cores, deterministic. */
 AZ_API int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_target_policy, const float* h_target_value, int n,
                             float* loss_policy, float* loss_value, void* stream);
 /* AlphaZeroNN::train (alphazero_nn.cpp:351-410) on packed sample records (az_selfplay_samples / the reference's sample files):
-   `epochs` shuffled passes, whole batches of batch_size (SETTINGS.BATCH_SIZE = 512) only; per-epoch mean losses (may be NULL) */
+   `epochs` shuffled passes, whole batches of batch_size (SETTINGS.BATCH_SIZE = 512) only; per-epoch mean losses (may be NULL).
+   Rejects a network with six value outputs (a two-player record holds one value target) */
 AZ_API int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                        float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
 /* AZ_NN_FP32 (default, the parity path) or AZ_NN_BF16: the three convolution-shaped contractions of the step (forward, data gradient,
@@ -236,10 +243,12 @@ typedef struct az_mcts az_mcts;
 #define AZ_EVAL_NN 0        /* leaf evaluation by the network (az_nn) */
 #define AZ_EVAL_PSEUDO 1    /* include/az_pseudo_net.h: exactly representable outputs, for bit-exact search parity tests */
 #define AZ_EVAL_UNIFORM 2   /* uniform prior, value 0 ("null evaluator": tree + env cost only) */
+#define AZ_EVAL_PSEUDO6 3   /* six-player search only: AZ_EVAL_PSEUDO's policy with the six-seat value vector az_pn_value6 (SIXPLAYER.md §2) */
 
 /* one search tree (transposition table) per game of `env`; hyper-parameters come from the env's az_rules
    (mcts_simulations, threads_per_mcts -> sims - sims % t, cpuct, dir_noise_*, temperature_threshold).
-   Replaces AlphaZeroMCTS (player/alpha_zero/alphazero_mcts.h:75-94) with THREADS_PER_MCTS = 1 semantics. */
+   Replaces AlphaZeroMCTS (player/alpha_zero/alphazero_mcts.h:75-94) with THREADS_PER_MCTS = 1 semantics.  Evaluators AZ_EVAL_NN,
+   _PSEUDO, _UNIFORM; a network with six value outputs is rejected. */
 AZ_API int az_mcts_create(az_env* env, az_nn* nn, int evaluator, int precision, az_mcts** out);
 AZ_API int az_mcts_destroy(az_mcts* mcts);
 /* node-pool occupancy: the fullest pool any game had at the end of a search since the counters were reset, the capacity of a pool
@@ -344,7 +353,10 @@ AZ_API int az_env6_encode(az_env6* env, float* h_x, void* stream);
    max(1, concurrent_descents) descents per tree per leaf batch under the reference's active_N rule, the two-player lockstep schedule
    (SIXPLAYER.md §2; K = 1 by default = THREADS_PER_MCTS = 1 semantics), hyper-parameters from the env's az_rules, evaluators and
    precisions as az_mcts_create.  az_mcts6_create rejects K > 16 and a simulation count (mcts_simulations - mcts_simulations %
-   threads_per_mcts) that K does not divide.  Self-play, both pick modes, sample recording and the arena use the env's K. */
+   threads_per_mcts) that K does not divide.  Self-play, both pick modes, sample recording and the arena use the env's K.
+   With a six-seat value vector (evaluator AZ_EVAL_NN over a network with six value outputs, or AZ_EVAL_PSEUDO6) a leaf's v[6] is
+   relative to its seat to move L and a path node whose mover is s receives v[(s - L + 6) % 6]; a finished game backs up as above,
+   and the node's stored value (root statistics) is component 0.  A one-output network keeps the scalar rule bit for bit. */
 typedef struct az_mcts6 az_mcts6;
 AZ_API int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int precision, az_mcts6** out);
 AZ_API int az_mcts6_destroy(az_mcts6* mcts);
@@ -356,6 +368,7 @@ AZ_API int az_mcts6_counters(az_mcts6* mcts, az_counters6* h_out, uint64_t* h_si
    AZ_SAMPLE6_BYTES per sample, every field 4-byte aligned:
      bytes 0..107    the root position BEFORE the move as its AZ_ENV6_IMAGE_BYTES image (az_env6_export's bytes; seat to move = byte 98)
      bytes 108..111  float value target: 1 when the seat to move won, 0 after a draw, -1/5 (the search's -v / 5 with v = 1) otherwise
+                     (the format is the same for both value widths: a six-output network's targets are derived from the status)
      bytes 112..283  float policy target[43]: the search's pi for that move (az_mcts6_search's h_pi), bit for bit
      byte  284       int8 final status of the game (winner seat 0..5 or AZ_STATUS_DRAW); bytes 285..287 zero */
 #define AZ_SAMPLE6_BYTES 288
@@ -368,7 +381,9 @@ AZ_API int az_selfplay6_record(az_mcts6* mcts, size_t capacity_samples, int max_
 /* drains the six-player queue: the calling convention of az_selfplay_samples with AZ_SAMPLE6_BYTES records */
 AZ_API int az_selfplay6_samples(az_mcts6* mcts, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream);
 /* az_nn_train on AZ_SAMPLE6_BYTES records: the same shuffled epochs, whole batches, per-epoch mean losses and training precisions; the
-   input planes are the six-seat encoding of az_env6_encode, built on the device from each record's image */
+   input planes are the six-seat encoding of az_env6_encode, built on the device from each record's image.  With six value outputs
+   target k of a record is the value rule above for seat (cur + k) % 6 (1 for the winner, -1/5 for another seat, 0 after a draw);
+   component 0 is the stored float */
 AZ_API int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                         float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
 /* ---- six-player arena (SIXPLAYER.md §4): seat-rotated matches between searchers and the uniform-random player over one env6.

@@ -55,4 +55,13 @@ AZ_PN_HD float az_pn_value(uint64_t key)
     return (float)((int)((m >> 7) & 255u) - 128) * (1.0f / 128.0f);
 }
 
+/* component k (0..5) of the six-seat value vector (SIXPLAYER.md §2): the value of seat (cur + k) % 6.  Component 0 is
+   az_pn_value; the others come from their own mix, dyadic like the rest, and their sum is not constrained. */
+AZ_PN_HD float az_pn_value6(uint64_t key, int k)
+{
+    if (k == 0) return az_pn_value(key);
+    uint64_t m = az_pn_mix((key ^ 0xD6E8FEB86659FD93ull) + 0xA0761D6478BD642Full * (uint64_t)k);
+    return (float)((int)((m >> 7) & 255u) - 128) * (1.0f / 128.0f);
+}
+
 #endif /* AZ_PSEUDO_NET_H */
