@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(PKG, "libaz_b200.so")
 
 LANDS, MOVES, SKIP, NONE = 42, 43, 42, 43
 DATA_BYTES, INPUT_FLOATS = 160, 546
+INPUT6_FLOATS = 672     # [7][6][16]: the six-player seat planes (AZ_INPUT6_FLOATS, Net(input_planes=16))
 STATUS_RUNNING, STATUS_DRAW, STATUS_ILLEGAL, STATUS_OVER = -1, -2, -3, -4
 
 
@@ -77,6 +78,9 @@ def lib():
         L.az_nn_create_value.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
         L.az_nn_value_outputs.argtypes = [vp]
         L.az_nn_value_outputs.restype = C.c_int
+        L.az_nn_create_planes.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
+        L.az_nn_input_planes.argtypes = [vp]
+        L.az_nn_input_planes.restype = C.c_int
         L.az_nn_destroy.argtypes = [vp]
         L.az_nn_blocks.argtypes = [vp]
         L.az_nn_num_vars.argtypes = [vp]
@@ -145,6 +149,7 @@ def lib():
         L.az_env6_import.argtypes = [vp, vp, vp]
         L.az_env6_counters.argtypes = [vp, C.POINTER(AzCounters6), C.c_int, vp]
         L.az_env6_encode.argtypes = [vp, vp, vp]
+        L.az_env6_encode_planes.argtypes = [vp, C.c_int, vp, vp]
         L.az_mcts6_create.argtypes = [vp, vp, C.c_int, C.c_int, C.POINTER(vp)]
         L.az_mcts6_destroy.argtypes = [vp]
         L.az_mcts6_search.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, vp, vp]
@@ -307,14 +312,16 @@ FP32, BF16 = 0, 1
 
 class Net:
     """the policy/value conv ResNet (az_nn_*); weights keyed by the reference graph's TF variable names.  value_outputs = 6: the
-    six-seat value vector of SIXPLAYER.md §2 (output k = the value of seat (cur + k) % 6); 1 = the reference graph"""
+    six-seat value vector of SIXPLAYER.md §2 (output k = the value of seat (cur + k) % 6); 1 = the reference graph.  input_planes = 16:
+    the six-player seat planes of SIXPLAYER.md §2 (inputs [n, 42 * 16], Env6.encode(planes=16)); 13 = the reference graph"""
 
-    def __init__(self, blocks=5, device=0, seed=None, value_outputs=1):
+    def __init__(self, blocks=5, device=0, seed=None, value_outputs=1, input_planes=13):
         self.L = lib()
         h = C.c_void_p()
-        check(self.L.az_nn_create_value(int(blocks), int(value_outputs), device, C.byref(h)))
+        check(self.L.az_nn_create_planes(int(blocks), int(value_outputs), int(input_planes), device, C.byref(h)))
         self.h, self.blocks, self.device = h, int(blocks), device
         self.value_outputs = int(self.L.az_nn_value_outputs(h))
+        self.input_planes = int(self.L.az_nn_input_planes(h))
         if seed is not None:
             self.init_random(seed)
 
@@ -364,8 +371,8 @@ class Net:
         check(self.L.az_nn_finalize(self.h))
 
     def forward(self, x, precision=FP32, stream=None):
-        """(policy [n, 43], value [n] with one value output, [n, 6] with six)"""
-        a = np.ascontiguousarray(x, np.float32).reshape(-1, INPUT_FLOATS)
+        """x [n, 42 * input_planes] (any shape of that size) -> (policy [n, 43], value [n] with one value output, [n, 6] with six)"""
+        a = np.ascontiguousarray(x, np.float32).reshape(-1, 42 * self.input_planes)
         n = a.shape[0]
         pol = np.empty((n, MOVES), np.float32)
         val = np.empty(n, np.float32) if self.value_outputs == 1 else np.empty((n, self.value_outputs), np.float32)
@@ -377,8 +384,9 @@ class Net:
 
     # ---- training step and checkpoints (AlphaZeroNN::train / saveCheckpoint / loadCheckpoint)
     def train_step(self, x, target_policy, target_value, stream=None):
-        """one optimizer step on a batch; target_value [n] (one value output) or [n, 6] (six); returns (policy loss, value loss)"""
-        a = np.ascontiguousarray(x, np.float32).reshape(-1, INPUT_FLOATS)
+        """one optimizer step on a batch x [n, 42 * input_planes]; target_value [n] (one value output) or [n, 6] (six); returns (policy
+        loss, value loss)"""
+        a = np.ascontiguousarray(x, np.float32).reshape(-1, 42 * self.input_planes)
         tp = np.ascontiguousarray(target_policy, np.float32).reshape(-1, MOVES)
         tv = np.ascontiguousarray(target_value, np.float32)
         assert tv.shape == ((a.shape[0],) if self.value_outputs == 1 else (a.shape[0], self.value_outputs)), tv.shape
@@ -769,9 +777,10 @@ class Env6:
         check(self.L.az_env6_counters(self.h, C.byref(c), int(reset), stream))
         return dict(steps=int(c.steps), games=int(c.games), draws=int(c.draws), wins=[int(c.wins[i]) for i in range(6)])
 
-    def encode(self, stream=None):
-        a = np.empty((self.n, 7, 6, 13), np.float32)
-        check(self.L.az_env6_encode(self.h, _ptr(a), stream))
+    def encode(self, planes=13, stream=None):
+        """the network input of every game, [n, 7, 6, planes]: 13 = the two-player planes read for six seats, 16 = the seat planes"""
+        a = np.empty((self.n, 7, 6, int(planes)), np.float32)
+        check(self.L.az_env6_encode_planes(self.h, int(planes), _ptr(a), stream))
         return a
 
 

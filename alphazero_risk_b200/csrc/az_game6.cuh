@@ -272,9 +272,13 @@ __device__ __forceinline__ void e6_new_game(E6Ctx& c, uint64_t seed, uint32_t ga
 // the six-seat network input of one position (SIXPLAYER.md; r6_encode of the oracle, same expressions): the reference's [7][6][13]
 // planes with "enemy" = the seat that moves next and "neutral" = every other seat.  One thread writes the position's
 // AZ_INPUT_FLOATS floats; shared by the search's leaf batches (k_env6_encode) and the training unpack of six-player records.
+// P = 16: the seat planes (SIXPLAYER.md §2; r6_encode16 of the oracle), AZ_INPUT6_FLOATS floats — plane k (k = 0..5) holds the armies
+// of seat (cur + k) % 6, planes 6..15 are planes 3..12 of the 13-plane form.
+template <int P = 13>
 __device__ __forceinline__ void e6_encode_position(const uint8_t* army, const uint8_t* owner, uint32_t cur, uint32_t phase, uint32_t attacks,
                                                    uint32_t allow_draw, float* __restrict__ out)
 {
+    static_assert(P == 13 || P == 16, "13 or 16 input planes");
     uint64_t own[E6_PLAYERS] = { 0, 0, 0, 0, 0, 0 };
     int own_total = 0, other_total = 0;
     for (int i = 0; i < AZ_LANDS; ++i) {
@@ -290,12 +294,18 @@ __device__ __forceinline__ void e6_encode_position(const uint8_t* army, const ui
     const float reinf_share = __fdiv_rn(ref, __fadd_rn(ref, oref));
     float att = __fdiv_rn((float)attacks, 8.0f); att = att > 1.0f ? 1.0f : att;
     for (int i = 0; i < AZ_LANDS; ++i) {
-        float* f = out + i * 13;
+        float* f = out + i * P;
         const float a = __fdiv_rn((float)army[i], 32.0f);
-        f[0] = owner[i] == cur ? a : 0.0f;
-        f[1] = (owner[i] == nx && nx != cur) ? a : 0.0f;
-        f[2] = (owner[i] != cur && owner[i] != nx) ? a : 0.0f;
-        f[3] = army_share; f[4] = reinf_share; f[5] = att; f[6] = allow_draw ? 1.0f : 0.0f;
-        for (uint32_t k = 0; k < 6; ++k) f[7 + k] = phase == k ? 1.0f : 0.0f;
+        if constexpr (P == 13) {
+            f[0] = owner[i] == cur ? a : 0.0f;
+            f[1] = (owner[i] == nx && nx != cur) ? a : 0.0f;
+            f[2] = (owner[i] != cur && owner[i] != nx) ? a : 0.0f;
+            f[3] = army_share; f[4] = reinf_share; f[5] = att; f[6] = allow_draw ? 1.0f : 0.0f;
+            for (uint32_t k = 0; k < 6; ++k) f[7 + k] = phase == k ? 1.0f : 0.0f;
+        } else {
+            for (uint32_t k = 0; k < E6_PLAYERS; ++k) f[k] = owner[i] == (cur + k) % E6_PLAYERS ? a : 0.0f;
+            f[6] = army_share; f[7] = reinf_share; f[8] = att; f[9] = allow_draw ? 1.0f : 0.0f;
+            for (uint32_t k = 0; k < 6; ++k) f[10 + k] = phase == k ? 1.0f : 0.0f;
+        }
     }
 }

@@ -489,31 +489,34 @@ __global__ void __launch_bounds__(M6_WARPS * 32) k_mcts6_rec_end(Mcts6Dev m)
     if (lane == 0) { m.rec_len[gi] = 0; m.rec_end[gi] = AZ_STATUS_RUNNING; }
 }
 
-// the six-seat network input (SIXPLAYER.md, e6_encode_position) of column i of the SoA state st [28][stride]
+// the six-seat network input (SIXPLAYER.md, e6_encode_position) of column i of the SoA state st [28][stride], P = 13 or 16 planes
+template <int P>
 __device__ __forceinline__ void m6_encode_game(const uint32_t* __restrict__ st, int stride, int i, float* __restrict__ out)
 {
     uint32_t row[E6_WORDS];
     for (int w = 0; w < E6_WORDS; ++w) row[w] = st[(size_t)w * stride + i];
     const uint32_t cur = (row[24] >> 16) & 0xffu, phase = (row[25] >> 8) & 0xffu, attacks = (row[23] >> 24) & 0xffu, allow = (row[23] >> 16) & 0xffu;
-    e6_encode_position((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, out);
+    e6_encode_position<P>((const uint8_t*)row, (const uint8_t*)(row + 11), cur, phase, attacks, allow, out);
 }
 // one thread per position: columns 0..count-1 of the SoA state st [28][stride]
+template <int P>
 __global__ void __launch_bounds__(128) k_env6_encode(const uint32_t* __restrict__ st, int stride, int count, float* __restrict__ x)
 {
     const int i = blockIdx.x * 128 + threadIdx.x;
     if (i >= count) return;
-    m6_encode_game(st, stride, i, x + (size_t)i * AZ_INPUT_FLOATS);
+    m6_encode_game<P>(st, stride, i, x + (size_t)i * 42 * P);
 }
 
 // arena leaf batches: row j * count + k = the leaf of descent slot j * n + games[k] (games = the games that search this tick, k_used =
 // descent slots per game in the batch, leaf state stride K * n), and the network's outputs (policy [43], value [vo]) back to those slots
+template <int P>
 __global__ void __launch_bounds__(128) k_env6_encode_list(const uint32_t* __restrict__ st, int stride, int n, const int32_t* __restrict__ games,
                                                           int count, int k_used, float* __restrict__ x)
 {
     const int i = blockIdx.x * 128 + threadIdx.x;
     if (i >= count * k_used) return;
     const int j = i / count, k = i - j * count;
-    m6_encode_game(st, stride, j * n + games[k], x + (size_t)i * AZ_INPUT_FLOATS);
+    m6_encode_game<P>(st, stride, j * n + games[k], x + (size_t)i * 42 * P);
 }
 __global__ void __launch_bounds__(256) k_mcts6_scatter_evals(const float* __restrict__ pol_c, const float* __restrict__ val_c,
                                                              const int32_t* __restrict__ games, int count, int n, int k_used, int vo,
@@ -592,7 +595,7 @@ extern "C" int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int preci
     rc |= m6_alloc(mc, &d.out_p, n * AZ_MOVES); rc |= m6_alloc(mc, &d.out_move, n); rc |= m6_alloc(mc, &d.out_status, n);
     rc |= m6_alloc(mc, &d.out_sumn, n); rc |= m6_alloc(mc, &d.out_table, n);
     rc |= m6_alloc(mc, &d.counters, (size_t)M6C_N);
-    if (evaluator == M6_EVAL_NN) rc |= m6_alloc(mc, &mc->d_x, ns * AZ_INPUT_FLOATS);
+    if (evaluator == M6_EVAL_NN) rc |= m6_alloc(mc, &mc->d_x, ns * 42 * (size_t)nn->input_planes);
     if (rc) { for (void* p : mc->allocs) cudaFree(p); delete mc; return AZ_ERR_CUDA; }
     d.root_state = az_env6_state_ptr(env);
     d.c1 = 1.0f - r->dir_noise_epsi; d.c2 = r->dir_noise_epsi * r->dir_noise_value; d.cpuct = r->cpuct;
@@ -618,9 +621,11 @@ static int m6_evaluate(az_mcts6* mc, cudaStream_t s, int k_used)
     if (mc->evaluator != M6_EVAL_NN) return AZ_OK;
     Mcts6Dev& d = mc->d;
     const int ns = d.K * d.n;                            // the stride of the SoA leaf state
+    const bool seat_planes = mc->nn->input_planes == AZ_NN_IN_CH6;   // the leaves are encoded with the network's plane count
     if (mc->eval_count > 0 && mc->eval_count < d.n) {
         const int c = mc->eval_count, m = c * k_used;
-        k_env6_encode_list<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, d.n, mc->eval_games, c, k_used, mc->d_x);
+        if (seat_planes) k_env6_encode_list<AZ_NN_IN_CH6><<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, d.n, mc->eval_games, c, k_used, mc->d_x);
+        else k_env6_encode_list<AZ_NN_IN_CH><<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, d.n, mc->eval_games, c, k_used, mc->d_x);
         AZ_CUDA(cudaGetLastError());
         int rc = az_nn_forward_dev(mc->nn, mc->d_x, m, mc->eval_pol, mc->eval_val, mc->precision, s); if (rc) return rc;
         k_mcts6_scatter_evals<<<(m * (AZ_MOVES + d.vo) + 255) / 256, 256, 0, s>>>(mc->eval_pol, mc->eval_val, mc->eval_games, c, d.n, k_used,
@@ -629,7 +634,8 @@ static int m6_evaluate(az_mcts6* mc, cudaStream_t s, int k_used)
         return AZ_OK;
     }
     const int m = d.n * k_used;                          // slots j * n + game: the first k_used * n of them
-    k_env6_encode<<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, m, mc->d_x);
+    if (seat_planes) k_env6_encode<AZ_NN_IN_CH6><<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, m, mc->d_x);
+    else k_env6_encode<AZ_NN_IN_CH><<<(m + 127) / 128, 128, 0, s>>>(d.leaf_state, ns, m, mc->d_x);
     AZ_CUDA(cudaGetLastError());
     return az_nn_forward_dev(mc->nn, mc->d_x, m, d.nn_policy, d.nn_value, mc->precision, s);
 }
@@ -768,22 +774,26 @@ extern "C" int az_mcts6_counters(az_mcts6* mc, az_counters6* h_out, uint64_t* h_
     return AZ_OK;
 }
 
-extern "C" int az_env6_encode(az_env6* e, float* h_x, void* stream)
+extern "C" int az_env6_encode_planes(az_env6* e, int input_planes, float* h_x, void* stream)
 {
     AZ_REQUIRE(e && h_x, "NULL argument");
+    AZ_REQUIRE(input_planes == AZ_NN_IN_CH || input_planes == AZ_NN_IN_CH6, "input_planes must be 13 or 16");
     AzDeviceGuard guard(az_env6_device(e));
     cudaStream_t s = (cudaStream_t)stream;
     const int n = az_env6_n(e);
+    const size_t floats = (size_t)n * 42 * input_planes;
     float* d_x = nullptr;
-    AZ_CUDA(cudaMalloc(&d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS));
-    k_env6_encode<<<(n + 127) / 128, 128, 0, s>>>(az_env6_state_ptr(e), n, n, d_x);
+    AZ_CUDA(cudaMalloc(&d_x, sizeof(float) * floats));
+    if (input_planes == AZ_NN_IN_CH6) k_env6_encode<AZ_NN_IN_CH6><<<(n + 127) / 128, 128, 0, s>>>(az_env6_state_ptr(e), n, n, d_x);
+    else k_env6_encode<AZ_NN_IN_CH><<<(n + 127) / 128, 128, 0, s>>>(az_env6_state_ptr(e), n, n, d_x);
     cudaError_t ce = cudaGetLastError();
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(h_x, d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS, cudaMemcpyDeviceToHost, s);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(h_x, d_x, sizeof(float) * floats, cudaMemcpyDeviceToHost, s);
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
     cudaFree(d_x);
     if (ce != cudaSuccess) { az_set_error("az_env6_encode: %s", cudaGetErrorString(ce)); return AZ_ERR_CUDA; }
     return AZ_OK;
 }
+extern "C" int az_env6_encode(az_env6* e, float* h_x, void* stream) { return az_env6_encode_planes(e, AZ_NN_IN_CH, h_x, stream); }
 
 // ---------------------------------------------------------------- six-player arena (SIXPLAYER.md §4)
 // k_arena6_advance (az_env6.cu) tallies, deals and plays the random player's plies; each tick then runs one search per searcher

@@ -6,7 +6,7 @@
 // BLOCKS x {conv3x3, BN(256), ReLU, conv3x3, BN(256), +skip, ReLU} -> policy head conv1x1->2, BN,
 // ReLU, flatten(84, NHWC order), dense 43 + bias, softmax ; value head conv1x1->1, BN, ReLU,
 // flatten(42), dense 256 + bias, ReLU, dense 1 + bias, tanh (dense value_outputs = 6 for the six-seat value vector of
-// SIXPLAYER.md §2, each output through tanh).  Inference BN:
+// SIXPLAYER.md §2, each output through tanh; 16 input planes instead of 13 for its seat planes, az_nn_create_planes).  Inference BN:
 // y = (x - moving_mean) * (gamma * rsqrt(moving_variance + 0.001)) + beta.
 // Replaces the TensorFlow session->Run of neural_network/alphazero_nn.cpp:247-248, :339-340.
 #include <cmath>
@@ -43,7 +43,7 @@ static float glorot(int fan_in, int fan_out) { return sqrtf(6.0f / (float)(fan_i
 // limits reproduce the initializers recorded there (stem 0.049783, tower 0.036084, pi 0.152499, ...)
 static void build_inventory(az_nn* nn)
 {
-    add_var(nn, "conv/kernel", { 3, 3, AZ_NN_IN_CH, AZ_NN_CH }, glorot(9 * AZ_NN_IN_CH, 9 * AZ_NN_CH), 0.0f);
+    add_var(nn, "conv/kernel", { 3, 3, nn->input_planes, AZ_NN_CH }, glorot(9 * nn->input_planes, 9 * AZ_NN_CH), 0.0f);
     add_bn(nn, "conv_bn", 7);
     for (int i = 0; i < nn->blocks; ++i) {
         std::string s = std::to_string(i) + block_letter(i);
@@ -74,26 +74,28 @@ const float* az_nn_host_var(const az_nn* nn, const std::string& name)
 // neighbour of board cell p for tap t (ky*3+kx), -1 outside the 7x6 board (padding SAME)
 __constant__ int8_t c_nb[42 * 9];
 
-// stem: conv3x3 13->256 + row-indexed BN + ReLU.  One block per board, thread = output channel.
-__global__ void __launch_bounds__(256) k_nn_stem_fp32(const float* __restrict__ x, int n, const float* __restrict__ w /*[9][13][256]*/,
+// stem: conv3x3 P->256 + row-indexed BN + ReLU.  One block per board, thread = output channel.  P = input planes: 13 (the reference
+// graph), 16 (the six-player seat planes)
+template <int P>
+__global__ void __launch_bounds__(256) k_nn_stem_fp32(const float* __restrict__ x, int n, const float* __restrict__ w /*[9][P][256]*/,
                                                        const float* __restrict__ bn /*[4][7]: gamma,beta,mean,var*/,
                                                        float* __restrict__ out /*[n][42][256]*/)
 {
-    __shared__ float s_in[43 * AZ_NN_IN_CH];
+    __shared__ float s_in[43 * P];
     int b = blockIdx.x, co = threadIdx.x;
-    for (int i = threadIdx.x; i < 42 * AZ_NN_IN_CH; i += 256) s_in[i] = x[(size_t)b * 42 * AZ_NN_IN_CH + i];
-    if (threadIdx.x < AZ_NN_IN_CH) s_in[42 * AZ_NN_IN_CH + threadIdx.x] = 0.0f;
+    for (int i = threadIdx.x; i < 42 * P; i += 256) s_in[i] = x[(size_t)b * 42 * P + i];
+    if (threadIdx.x < P) s_in[42 * P + threadIdx.x] = 0.0f;
     __syncthreads();
-    float wr[9 * AZ_NN_IN_CH];
+    float wr[9 * P];
 #pragma unroll
-    for (int i = 0; i < 9 * AZ_NN_IN_CH; ++i) wr[i] = w[i * AZ_NN_CH + co];
+    for (int i = 0; i < 9 * P; ++i) wr[i] = w[i * AZ_NN_CH + co];
     for (int p = 0; p < 42; ++p) {
         float acc = 0.0f;
 #pragma unroll
         for (int t = 0; t < 9; ++t) {
             int q = c_nb[p * 9 + t]; q = q < 0 ? 42 : q;
 #pragma unroll
-            for (int ci = 0; ci < AZ_NN_IN_CH; ++ci) acc = fmaf(s_in[q * AZ_NN_IN_CH + ci], wr[t * AZ_NN_IN_CH + ci], acc);
+            for (int ci = 0; ci < P; ++ci) acc = fmaf(s_in[q * P + ci], wr[t * P + ci], acc);
         }
         int y = p / 6;
         float sc = bn[y] * rsqrtf(bn[21 + y] + AZ_NN_BN_EPS);
@@ -256,18 +258,19 @@ static int upload(float** d, const float* h, size_t count)
     return AZ_OK;
 }
 
-extern "C" int az_nn_create_value(int blocks, int value_outputs, int device, az_nn** out)
+extern "C" int az_nn_create_planes(int blocks, int value_outputs, int input_planes, int device, az_nn** out)
 {
     AZ_REQUIRE(out != nullptr, "out is NULL");
     AZ_REQUIRE(blocks >= 1 && blocks <= 26, "blocks must be in [1, 26]");
     AZ_REQUIRE(value_outputs == 1 || value_outputs == 6, "value_outputs must be 1 or 6");
+    AZ_REQUIRE(input_planes == AZ_NN_IN_CH || input_planes == AZ_NN_IN_CH6, "input_planes must be 13 or 16");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); az_set_error("no CUDA device: libaz_b200 has no CPU fallback"); return AZ_ERR_NO_DEVICE; }
     AZ_REQUIRE(device >= 0 && device < ndev, "device index out of range");
     AzDeviceGuard guard(device);
     az_nn* nn = new (std::nothrow) az_nn();
     AZ_REQUIRE(nn != nullptr, "out of host memory");
-    nn->blocks = blocks; nn->device = device; nn->value_outputs = value_outputs;
+    nn->blocks = blocks; nn->device = device; nn->value_outputs = value_outputs; nn->input_planes = input_planes;
     build_inventory(nn);
     int8_t nb[42 * 9];
     for (int p = 0; p < 42; ++p)
@@ -282,6 +285,10 @@ extern "C" int az_nn_create_value(int blocks, int value_outputs, int device, az_
     return AZ_OK;
 }
 
+extern "C" int az_nn_create_value(int blocks, int value_outputs, int device, az_nn** out)
+{
+    return az_nn_create_planes(blocks, value_outputs, AZ_NN_IN_CH, device, out);
+}
 extern "C" int az_nn_create(int blocks, int device, az_nn** out) { return az_nn_create_value(blocks, 1, device, out); }
 
 extern "C" int az_nn_destroy(az_nn* nn)
@@ -300,6 +307,7 @@ extern "C" int az_nn_num_vars(const az_nn* nn) { return nn ? (int)nn->vars.size(
 extern "C" size_t az_nn_num_params(const az_nn* nn) { return nn ? nn->blob.size() : 0; }
 extern "C" int az_nn_blocks(const az_nn* nn) { return nn ? nn->blocks : 0; }
 extern "C" int az_nn_value_outputs(const az_nn* nn) { return nn ? nn->value_outputs : 0; }
+extern "C" int az_nn_input_planes(const az_nn* nn) { return nn ? nn->input_planes : 0; }
 
 extern "C" int az_nn_var_info(const az_nn* nn, int i, const char** name, size_t* count, int* rank, int* shape4)
 {
@@ -414,7 +422,7 @@ int az_nn_reserve(az_nn* nn, int n)
     cudaFree(nn->d_x); cudaFree(nn->d_policy); cudaFree(nn->d_value);
     nn->d_x = nullptr; nn->d_policy = nullptr; nn->d_value = nullptr;
     for (int i = 0; i < 3; ++i) AZ_CUDA(cudaMalloc(&nn->d_act[i], sizeof(float) * (size_t)n * 42 * AZ_NN_CH));
-    AZ_CUDA(cudaMalloc(&nn->d_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS));
+    AZ_CUDA(cudaMalloc(&nn->d_x, sizeof(float) * (size_t)n * 42 * nn->input_planes));
     AZ_CUDA(cudaMalloc(&nn->d_policy, sizeof(float) * (size_t)n * 43));
     AZ_CUDA(cudaMalloc(&nn->d_value, sizeof(float) * (size_t)n * nn->value_outputs));
     nn->cap = n;
@@ -437,7 +445,9 @@ static int forward_fp32(az_nn* nn, const float* d_x, int n, float* d_policy, flo
 {
     float* buf[3] = { nn->d_act[0], nn->d_act[1], nn->d_act[2] };
     int cur = 0, tmp = 1, nxt = 2;
-    k_nn_stem_fp32<<<n, 256, 0, s>>>(d_x, n, az_nn_dev_var(nn, "conv/kernel"), az_nn_dev_var(nn, "conv_bn/gamma"), buf[cur]);
+    if (nn->input_planes == AZ_NN_IN_CH6)
+        k_nn_stem_fp32<AZ_NN_IN_CH6><<<n, 256, 0, s>>>(d_x, n, az_nn_dev_var(nn, "conv/kernel"), az_nn_dev_var(nn, "conv_bn/gamma"), buf[cur]);
+    else k_nn_stem_fp32<AZ_NN_IN_CH><<<n, 256, 0, s>>>(d_x, n, az_nn_dev_var(nn, "conv/kernel"), az_nn_dev_var(nn, "conv_bn/gamma"), buf[cur]);
     AZ_CUDA(cudaGetLastError());
     dim3 grid((n + F32_BOARDS - 1) / F32_BOARDS, AZ_NN_CH / F32_CO);
     size_t smem = F32_SMEM_FLOATS * sizeof(float);
@@ -466,6 +476,7 @@ extern "C" int az_nn_forward_dev(az_nn* nn, const float* d_x, int n, float* d_po
     AzDeviceGuard guard(nn->device);
     int rc = finalize(nn); if (rc) return rc;
     rc = az_nn_reserve(nn, n); if (rc) return rc;
+    if (precision == AZ_NN_BF16 && nn->input_planes == AZ_NN_IN_CH6) return az_nn_tc_forward_planes16(nn, d_x, n, d_policy, d_value, (cudaStream_t)stream);
     if (precision == AZ_NN_BF16 && nn->value_outputs == 6) return az_nn_tc_forward_value6(nn, d_x, n, d_policy, d_value, (cudaStream_t)stream);
     if (precision == AZ_NN_BF16) return az_nn_tc_forward(nn, d_x, nullptr, n, d_policy, d_value, (cudaStream_t)stream);
     return forward_fp32(nn, d_x, n, d_policy, d_value, (cudaStream_t)stream);
@@ -479,7 +490,7 @@ extern "C" int az_nn_forward(az_nn* nn, const float* h_x, int n, float* h_policy
     cudaStream_t s = (cudaStream_t)stream;
     int rc = finalize(nn); if (rc) return rc;
     rc = az_nn_reserve(nn, n); if (rc) return rc;
-    AZ_CUDA(cudaMemcpyAsync(nn->d_x, h_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS, cudaMemcpyHostToDevice, s));
+    AZ_CUDA(cudaMemcpyAsync(nn->d_x, h_x, sizeof(float) * (size_t)n * 42 * nn->input_planes, cudaMemcpyHostToDevice, s));
     rc = az_nn_forward_dev(nn, nn->d_x, n, nn->d_policy, nn->d_value, precision, stream);
     if (rc) return rc;
     AZ_CUDA(cudaMemcpyAsync(h_policy, nn->d_policy, sizeof(float) * (size_t)n * 43, cudaMemcpyDeviceToHost, s));

@@ -12,6 +12,7 @@
 
 #define AZ_NN_CH 256          // FILTERS, python/src/build_graph.py:32
 #define AZ_NN_IN_CH 13        // FEATURES (INPUT_VECTOR_TYPE_2), build_graph.py:18
+#define AZ_NN_IN_CH6 16       // the six-player seat planes (SIXPLAYER.md §2, az_nn_create_planes)
 #define AZ_NN_BN_EPS 0.001f   // tf.layers.batch_normalization default epsilon (GraphDef: 0.0010000000474974513)
 
 struct AzVar {
@@ -32,6 +33,7 @@ struct AzTrainState; // az_nn_train.cu
 struct az_nn {
     int blocks = 5, device = 0;
     int value_outputs = 1;            // 1 = the reference graph; 6 = the six-seat value vector (SIXPLAYER.md §2)
+    int input_planes = AZ_NN_IN_CH;   // 13 = the reference graph; 16 = the six-player seat planes (SIXPLAYER.md §2)
     std::vector<AzVar> vars;
     std::map<std::string, int> index;
     std::vector<float> blob;          // every variable, fp32, TF layouts (HWIO kernels), inventory order
@@ -40,7 +42,7 @@ struct az_nn {
     float* d_blob = nullptr;          // device copy of blob
     int cap = 0;                      // positions the work buffers are sized for
     float* d_act[3] = { nullptr, nullptr, nullptr };   // fp32 activations [cap][42][256]
-    float* d_x = nullptr; float* d_policy = nullptr; float* d_value = nullptr;   // staging for host-buffer calls
+    float* d_x = nullptr; float* d_policy = nullptr; float* d_value = nullptr;   // staging for host-buffer calls (d_x: [cap][42][input_planes])
     AzTcState* tc = nullptr;
     AzTrainState* train = nullptr;    // optimizer state + training work buffers, created on first use
 };
@@ -63,6 +65,8 @@ int az_nn_tc_forward(az_nn* nn, const float* d_x, const uint32_t* d_env_state, i
                      int state_stride = 0, int scratch_set = 0, bool shared_device = false);
 // the same forward for a network with six value outputs: value [n][6] (az_nn_tc_value6.cu)
 int az_nn_tc_forward_value6(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, cudaStream_t s);
+// the forward of a network with 16 input planes, x fp32 [n][7][6][16], one or six value outputs (az_nn_tc_value6.cu)
+int az_nn_tc_forward_planes16(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, cudaStream_t s);
 
 // raw 3x3 convolution of the training step on the tower kernel (az_nn_tc.cu): fp32 [n * 42][256] in, fp32 HWIO device weights
 // [9][256][256] (flip = 1: the data gradient's kernel), fp32 [n * 42][256] out; bf16 operands, fp32 accumulation

@@ -1,12 +1,14 @@
 // az_nn_tc_value6.cu — the translation unit of the bf16 tensor-core forward: az_nn_tc.cu itself (included byte for byte: the ncu capture
 // of its tower kernel in profiles/traffic.json is keyed by that file's hash) plus the value tail of a network with six value outputs
-// (SIXPLAYER.md §2, az_nn_create_value).
+// (SIXPLAYER.md §2, az_nn_create_value) and the input side of a network with 16 input planes (the seat planes, az_nn_create_planes).
 //
 // A six-output network shares everything with the one-output graph up to dense_1: the same tower, the same 1x1 head convolutions (whose
 // per-cell sums the last tower layer's epilogue writes to d_head_z) and the same policy head.  So its forward is az_nn_tc_forward
 // unchanged — policy bit for bit what a one-output network with the same shared weights gives — followed by k_nn_value6_tail, which
 // reads d_head_z again and writes value [n][6] over the scalar the one-output tail left in the first n entries.
+#define az_nn_tc_prepare az_nn_tc_prepare_13
 #include "az_nn_tc.cu"
+#undef az_nn_tc_prepare
 
 // value [n][6] for HB boards per block: BatchNorm + ReLU of the v channel, dense 42 -> 256 + ReLU, dense 256 -> 6, tanh; the
 // arithmetic of k_nn_heads_tail's value head, once per output column
@@ -54,5 +56,86 @@ int az_nn_tc_forward_value6(az_nn* nn, const float* d_x, int n, float* d_policy,
     if (rc) return rc;
     k_nn_value6_tail<<<(n + HB - 1) / HB, 256, 0, s>>>(nn->tc->scratch[0].d_head_z, n, az_nn_head_params(nn), d_value);
     AZ_CUDA(cudaGetLastError());
+    return AZ_OK;
+}
+
+// ---------------------------------------------------------------- 16 input planes (SIXPLAYER.md §2, "seat planes")
+// The stem's bf16 operand has two chunks of 8 channels whatever the plane count: 13 planes leave channels 13..15 zero, 16 planes fill
+// them.  So a 16-plane network runs the same stem kernel (k_nn_conv_tc<2, true, 3>), tower and heads; only its weight stages and its
+// input packing differ.
+
+// finalize's bf16 preparation: az_nn_tc.cu packs the stem as [3][3][13][256] (channels 13..15 zero); a 16-plane network's stem stages
+// are packed again from all 16 channels before anything reads them
+int az_nn_tc_prepare(az_nn* nn)
+{
+    int rc = az_nn_tc_prepare_13(nn);
+    if (rc || nn->input_planes == AZ_NN_IN_CH) return rc;
+    std::vector<uint8_t> packed((size_t)TC_STEM_BYTES);
+    pack_conv(az_nn_host_var(nn, "conv/kernel"), AZ_NN_IN_CH6, 2, reinterpret_cast<__nv_bfloat16*>(packed.data()));
+    AZ_CUDA(cudaMemcpy(nn->tc->d_wpacked, packed.data(), packed.size(), cudaMemcpyHostToDevice));
+    return AZ_OK;
+}
+
+// fp32 [n][42][16] -> bf16 [2 chunks][r_alloc][8], every channel data (no zero padding); thread = board cell.  The three copies
+// var_stride elements apart (plain, x = 5 cells zeroed, x = 0 cells zeroed) as k_nn_pack_input_tc writes them
+__global__ void __launch_bounds__(256) k_nn_pack_input16_tc(const float* __restrict__ x, int n, __nv_bfloat16* __restrict__ out, int r_alloc,
+                                                             size_t var_stride)
+{
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n * 42) return;
+    const int b = i / 42, p = i - b * 42;
+    const float* src = x + (size_t)i * AZ_NN_IN_CH6;
+    const int row = b * TC_RPB + p;
+    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        uint4 o;
+        __nv_bfloat162* o2 = reinterpret_cast<__nv_bfloat162*>(&o);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) o2[e] = __floats2bfloat162_rn(src[c * 8 + 2 * e], src[c * 8 + 2 * e + 1]);
+        const size_t at = ((size_t)c * r_alloc + TC_HALO + row) * 8;
+        *reinterpret_cast<uint4*>(out + at) = o;
+        *reinterpret_cast<uint4*>(out + var_stride + at) = (p % 6) == 5 ? zero : o;
+        *reinterpret_cast<uint4*>(out + 2 * var_stride + at) = (p % 6) == 0 ? zero : o;
+    }
+}
+
+// the bf16 forward of a 16-plane network (one or six value outputs): k_nn_pack_input16_tc, then the stem, the tower and the heads tail
+// launched exactly as az_nn_tc_forward launches them, then k_nn_value6_tail for six outputs.  The layer loop repeats
+// az_nn_tc_forward's because that function packs its input itself and az_nn_tc.cu cannot change (its hash keys the ncu captures).
+int az_nn_tc_forward_planes16(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, cudaStream_t s)
+{
+    AzTcState* st = nn->tc;
+    if (!st || !st->d_wpacked) { az_set_error("network not finalized"); return AZ_ERR_NOT_READY; }
+    AzTcScratch* tc = &st->scratch[0];
+    int rc = tc_reserve(tc, n); if (rc) return rc;
+    const int tiles = (n * TC_RPB + TC_TILE_ROWS - 1) / TC_TILE_ROWS;
+    const int grid = tiles < st->n_sm ? tiles : st->n_sm;
+    const int layers = 2 * nn->blocks;
+    int cur = 0, tmp = 1, nxt = 2;
+    k_nn_pack_input16_tc<<<(n * 42 + 255) / 256, 256, 0, s>>>(d_x, n, tc->d_in, tc->r_alloc, tc->in_var_stride);
+    AZ_CUDA(cudaGetLastError());
+    AZ_CUDA((launch_conv<2, true, 3>(grid, s, tc->d_in, st->d_wpacked, st->d_scale + layers * 256, st->d_shift + layers * 256, nullptr, tc->d_act[cur], n,
+                                     tc->r_alloc, tiles, tc->in_var_stride * 2)));
+    const int pitems = (tiles + 1) / 2;
+    const int pgrid = 2 * (pitems < st->max_pairs ? pitems : st->max_pairs);
+    for (int i = 0; i < nn->blocks; ++i) {
+        for (int h = 0; h < 2; ++h) {                        // branch2a: cur -> tmp; branch2b: tmp (+ cur as the residual) -> nxt
+            const int L = 2 * i + h;
+            const __nv_bfloat16* src = h ? tc->d_act[tmp] : tc->d_act[cur];
+            const __nv_bfloat16* res = h ? tc->d_act[cur] : nullptr;
+            __nv_bfloat16* dst = h ? tc->d_act[nxt] : tc->d_act[tmp];
+            const bool last = L == layers - 1;              // the last layer feeds the heads directly: no activation store
+            AZ_CUDA(launch_conv_pair3(pgrid, s, src, st->d_wpacked3 + (size_t)L * TC_LAYER_BYTES, st->d_scale + L * 256, st->d_shift + L * 256, res, dst, n,
+                                      tc->r_alloc, tiles, last ? st->d_head_w : nullptr, last ? tc->d_head_z : nullptr));
+        }
+        int o = cur; cur = nxt; nxt = o;
+    }
+    k_nn_heads_tail<<<(n + HB - 1) / HB, 256, 0, s>>>(tc->d_head_z, n, az_nn_head_params(nn), d_policy, d_value);
+    AZ_CUDA(cudaGetLastError());
+    if (nn->value_outputs == 6) {
+        k_nn_value6_tail<<<(n + HB - 1) / HB, 256, 0, s>>>(tc->d_head_z, n, az_nn_head_params(nn), d_value);
+        AZ_CUDA(cudaGetLastError());
+    }
     return AZ_OK;
 }

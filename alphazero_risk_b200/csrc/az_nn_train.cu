@@ -68,7 +68,7 @@ struct AzTrainState {
     bool slots_on_device = false, host_slots_stale = false;
     float beta1_power = TR_BETA1, beta2_power = TR_BETA2;
     uint64_t steps = 0;
-    float* d_x = nullptr;                              // [cap][42][13]
+    float* d_x = nullptr;                              // [cap][42][input_planes]
     std::vector<float*> z, a;                          // per conv layer (0 = stem, 1 + 2i / 2 + 2i = block i): raw output, activation
     float* d_stats = nullptr;                          // [layers + 2][4][256]: mean, invstd, c1 = sum(g)/N, c2 = sum(g*xhat)/N
     double* d_part = nullptr;                          // [TR_STAT_CHUNKS][256][2]
@@ -766,14 +766,15 @@ __global__ void __launch_bounds__(64) k_tr_unpack_samples(const uint8_t* __restr
 
 // six-player records (az_samples6.cuh) -> the six-seat input planes of each record's image (e6_encode_position, the encoding the
 // six-player search evaluates its leaves with) + value and policy targets; one thread per sample.  vo = 6: tv [n][6], target k =
-// s6_value(status, (cur + k) % 6) (component 0 is the record's stored value)
+// s6_value(status, (cur + k) % 6) (component 0 is the record's stored value).  P = the network's input planes (13, or 16 seat planes)
+template <int P>
 __global__ void __launch_bounds__(128) k_tr_unpack_samples6(const uint8_t* __restrict__ rec, const uint32_t* __restrict__ order, int n,
                                                             float* __restrict__ x, float* __restrict__ tp, float* __restrict__ tv, int vo)
 {
     const int b = blockIdx.x * 128 + threadIdx.x;
     if (b >= n) return;
     const uint8_t* r = rec + (size_t)order[b] * S6_BYTES;
-    e6_encode_position(r, r + AZ_LANDS, r[S6_CUR], r[S6_PHASE], r[S6_ATTACKS], r[S6_ALLOW_DRAW], x + (size_t)b * AZ_INPUT_FLOATS);
+    e6_encode_position<P>(r, r + AZ_LANDS, r[S6_CUR], r[S6_PHASE], r[S6_ATTACKS], r[S6_ALLOW_DRAW], x + (size_t)b * 42 * P);
     const float* f = (const float*)r;                       // records are 4-byte aligned (288-byte stride)
     if (vo == 1) tv[b] = f[S6_VALUE / 4];
     else for (int k = 0; k < vo; ++k) tv[(size_t)b * vo + k] = s6_value((int8_t)r[S6_STATUS], (r[S6_CUR] + (uint32_t)k) % E6_PLAYERS);
@@ -857,7 +858,7 @@ static int train_reserve(az_nn* nn, AzTrainState* t, int n)
     t->d_x = t->d_hz = t->d_hg = t->d_hfeat = t->d_tp = t->d_tv = nullptr; t->cap = 0;
     for (int L = 0; L < layers; ++L) { AZ_CUDA(cudaMalloc(&t->z[(size_t)L], sizeof(float) * act)); AZ_CUDA(cudaMalloc(&t->a[(size_t)L], sizeof(float) * act)); }
     for (int i = 0; i < 3; ++i) AZ_CUDA(cudaMalloc(&t->d_g[i], sizeof(float) * act));
-    AZ_CUDA(cudaMalloc(&t->d_x, sizeof(float) * (size_t)n * 42 * AZ_NN_IN_CH));
+    AZ_CUDA(cudaMalloc(&t->d_x, sizeof(float) * (size_t)n * 42 * nn->input_planes));
     AZ_CUDA(cudaMalloc(&t->d_hz, sizeof(float) * (size_t)n * 42 * 4)); AZ_CUDA(cudaMalloc(&t->d_hg, sizeof(float) * (size_t)n * 42 * 4));
     AZ_CUDA(cudaMalloc(&t->d_hfeat, sizeof(float) * (size_t)n * HF_STRIDE));
     AZ_CUDA(cudaMalloc(&t->d_tp, sizeof(float) * (size_t)n * 43)); AZ_CUDA(cudaMalloc(&t->d_tv, sizeof(float) * (size_t)n * nn->value_outputs));
@@ -896,7 +897,7 @@ static int conv_any(az_nn* nn, AzTrainState* t, const float* in, int n, int cin,
         if (!flip && in_rpb) return az_tc_conv_raw_rpb(&t->conv, in_rpb, n, w, 0, out, s);
         return az_tc_conv_raw(&t->conv, in, n, w, flip, out, s);
     }
-    if (t->precision == AZ_NN_BF16) {                       // the 13-channel stem: chunked im2col + k_tc_gemm
+    if (t->precision == AZ_NN_BF16) {                       // the 13- or 16-channel stem: chunked im2col + k_tc_gemm
         const int rows = n * 42, mp = (int)tr_mp(rows), cpad = (cin + 7) / 8 * 8, kp = (int)tr_kp(9 * cpad);
         int rc = az_tg_im2col(in, rows, cin, cpad, mp, kp, t->d_src16, t->d_colA, s); if (rc) return rc;
         rc = az_tg_weights(w, cin, cpad, kp, flip, t->d_colB, s); if (rc) return rc;
@@ -1006,7 +1007,7 @@ static int train_step_dev(az_nn* nn, const float* d_x, const float* d_tp, const 
     const size_t total = (size_t)rows * TR_CH;
     const unsigned egrid = (unsigned)((total + 255) / 256);
     // ---- forward
-    rc = conv_any(nn, t, d_x, n, AZ_NN_IN_CH, dvar(nn, "conv/kernel"), 0, t->z[0], s); if (rc) return rc;
+    rc = conv_any(nn, t, d_x, n, nn->input_planes, dvar(nn, "conv/kernel"), 0, t->z[0], s); if (rc) return rc;
     rc = bn_forward(nn, t, 0, n, nullptr, s); if (rc) return rc;
     for (int L = 1; L < layers; ++L) {
         rc = conv_any(nn, t, t->a[(size_t)L - 1], n, TR_CH, dvar(nn, tr_conv_name(L) + "/kernel"), 0, t->z[(size_t)L], s,
@@ -1044,7 +1045,7 @@ static int train_step_dev(az_nn* nn, const float* d_x, const float* d_tp, const 
         float* tmp = G0; G0 = G2; G2 = tmp;
     }
     rc = bn_backward(nn, t, 0, n, G0, G1, s); if (rc) return rc;
-    rc = conv_wgrad(nn, t, 0, n, d_x, AZ_NN_IN_CH, G1, s); if (rc) return rc;
+    rc = conv_wgrad(nn, t, 0, n, d_x, nn->input_planes, G1, s); if (rc) return rc;
     // ---- Adam
     const float lr_t = (float)((double)TR_LR * sqrt(1.0 - (double)t->beta2_power) / (1.0 - (double)t->beta1_power));
     const size_t np = nn->blob.size();
@@ -1070,7 +1071,7 @@ extern "C" int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_targ
     AzTrainState* t = train_state(nn);
     AZ_REQUIRE(t != nullptr, "out of host memory");
     int rc = train_reserve(nn, t, n); if (rc) return rc;
-    AZ_CUDA(cudaMemcpyAsync(t->d_x, h_x, sizeof(float) * (size_t)n * AZ_INPUT_FLOATS, cudaMemcpyHostToDevice, s));
+    AZ_CUDA(cudaMemcpyAsync(t->d_x, h_x, sizeof(float) * (size_t)n * 42 * nn->input_planes, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaMemcpyAsync(t->d_tp, h_target_policy, sizeof(float) * (size_t)n * 43, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaMemcpyAsync(t->d_tv, h_target_value, sizeof(float) * (size_t)n * nn->value_outputs, cudaMemcpyHostToDevice, s));
     float loss[2] = { 0.0f, 0.0f };
@@ -1081,15 +1082,17 @@ extern "C" int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_targ
 }
 
 // the record -> (input planes, targets) step of a training loop: batch b of an epoch unpacks the n records order[0..n) of d_rec
-// (tv holds vo values per record)
-typedef void (*TrUnpack)(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, cudaStream_t s);
-static void tr_unpack_samples(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int, cudaStream_t s)
+// (tv holds vo values per record, x `planes` input planes per board cell)
+typedef void (*TrUnpack)(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, int planes, cudaStream_t s);
+static void tr_unpack_samples(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int, int, cudaStream_t s)
 {
     k_tr_unpack_samples<<<(unsigned)n, 64, 0, s>>>(d_rec, d_order, n, x, tp, tv);
 }
-static void tr_unpack_samples6(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, cudaStream_t s)
+static void tr_unpack_samples6(const uint8_t* d_rec, const uint32_t* d_order, int n, float* x, float* tp, float* tv, int vo, int planes,
+                               cudaStream_t s)
 {
-    k_tr_unpack_samples6<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv, vo);
+    if (planes == AZ_NN_IN_CH6) k_tr_unpack_samples6<AZ_NN_IN_CH6><<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv, vo);
+    else k_tr_unpack_samples6<AZ_NN_IN_CH><<<(unsigned)((n + 127) / 128), 128, 0, s>>>(d_rec, d_order, n, x, tp, tv, vo);
 }
 
 // AlphaZeroNN::train (alphazero_nn.cpp:351-410): `epochs` passes over the samples in shuffled order, whole batches of batch_size only
@@ -1123,7 +1126,7 @@ static int train_records(az_nn* nn, const char* who, const uint8_t* h_records, s
         // the batches of an epoch are enqueued back to back; the losses are accumulated on the device and read once per epoch
         if (ce == cudaSuccess) ce = cudaMemsetAsync(d_acc, 0, 2 * sizeof(double), s);
         for (size_t b = 0; b < batches && ce == cudaSuccess && rc == AZ_OK; ++b) {
-            unpack(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv, nn->value_outputs, s);
+            unpack(d_rec, d_order + b * (size_t)batch_size, batch_size, t->d_x, t->d_tp, t->d_tv, nn->value_outputs, nn->input_planes, s);
             rc = train_step_dev(nn, t->d_x, t->d_tp, t->d_tv, batch_size, nullptr, s);
             if (rc == AZ_OK) k_tr_loss_accum<<<1, 32, 0, s>>>(t->d_loss, d_acc);
         }
@@ -1147,12 +1150,14 @@ extern "C" int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records
     AZ_REQUIRE(epochs >= 1 && batch_size >= 2, "epochs must be >= 1 and batch_size >= 2");
     AZ_REQUIRE(n_records >= (size_t)batch_size, "fewer samples than one batch");
     AZ_REQUIRE(nn->value_outputs == 1, "az_nn_train: two-player records hold one value target; the network has six value outputs");
+    AZ_REQUIRE(nn->input_planes == AZ_NN_IN_CH, "az_nn_train: two-player records encode 13 input planes; the network has 16 (the six-player seat planes)");
     AzDeviceGuard guard(nn->device);
     return train_records(nn, "az_nn_train", h_records, n_records, AZ_SAMPLE_BYTES, tr_unpack_samples, epochs, batch_size, seed,
                          h_epoch_loss_policy, h_epoch_loss_value, (cudaStream_t)stream);
 }
 
-// The same loop on six-player records (az_selfplay6_samples); the input planes are the six-seat encoding of each record's image.
+// The same loop on six-player records (az_selfplay6_samples); the input planes are the six-seat encoding of each record's image, with
+// the network's plane count.
 extern "C" int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                             float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream)
 {

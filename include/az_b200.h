@@ -39,6 +39,7 @@ extern "C" {
 #define AZ_NONE 43             /* LandIndex::None */
 #define AZ_DATA_BYTES 160      /* sizeof(Data), state/state.h:86-105 */
 #define AZ_INPUT_FLOATS 546    /* [7][6][13], neural_network/alphazero_nn_data.h:66 (INPUT_VECTOR_TYPE_2) */
+#define AZ_INPUT6_FLOATS 672   /* [7][6][16]: the six-player seat planes (SIXPLAYER.md §2, az_nn_create_planes) */
 #define AZ_STATE_WORDS 16      /* device SoA: 32-bit words per game (see DESIGN.md) */
 
 typedef enum az_error {
@@ -170,9 +171,16 @@ AZ_API int az_nn_create(int blocks, int device, az_nn** out);
    output through tanh.  6 = the six-seat value vector of SIXPLAYER.md §2: output k is the value of seat (cur + k) % 6, cur = the seat
    to move in the encoded position.  az_nn_create is value_outputs = 1, the reference graph */
 AZ_API int az_nn_create_value(int blocks, int value_outputs, int device, az_nn** out);
+/* the same network with input_planes (13 or 16) input planes: conv/kernel [3][3][input_planes][256], everything else unchanged.
+   16 = the six-player seat planes of SIXPLAYER.md §2 (AZ_INPUT6_FLOATS per position): plane k (k = 0..5) holds army / 32 on the lands
+   of seat (cur + k) % 6, planes 6..15 are planes 3..12 of the 13-plane encoding.  Such a network takes [n][7][6][16] in az_nn_forward,
+   az_nn_train_step, az_nn_train6 and the six-player search; the two-player search and az_nn_train reject it.  az_nn_create_value is
+   input_planes = 13 */
+AZ_API int az_nn_create_planes(int blocks, int value_outputs, int input_planes, int device, az_nn** out);
 AZ_API int az_nn_destroy(az_nn* nn);
 AZ_API int az_nn_blocks(const az_nn* nn);
 AZ_API int az_nn_value_outputs(const az_nn* nn);
+AZ_API int az_nn_input_planes(const az_nn* nn);
 AZ_API int az_nn_num_vars(const az_nn* nn);
 AZ_API size_t az_nn_num_params(const az_nn* nn);
 /* i-th variable: TF variable name (e.g. "res0a_branch2a/kernel"), element count, rank, shape (HWIO kernels) */
@@ -187,21 +195,22 @@ AZ_API int az_nn_import_blob(az_nn* nn, const float* h_in, size_t count);
 AZ_API int az_nn_init_random(az_nn* nn, uint64_t seed);
 AZ_API int az_nn_finalize(az_nn* nn);
 /* AlphaZeroNN::predict / processBatchPrediction (alphazero_nn.cpp:236-267, 333-349):
-   x fp32 [n][7][6][13] -> policy [n][43] (softmax), value [n][value_outputs] (tanh; [n] for the one-output graph) */
+   x fp32 [n][7][6][input_planes] -> policy [n][43] (softmax), value [n][value_outputs] (tanh; [n] for the one-output graph) */
 AZ_API int az_nn_forward(az_nn* nn, const float* h_x, int n, float* h_policy, float* h_value, int precision, void* stream);
 AZ_API int az_nn_forward_dev(az_nn* nn, const float* d_x, int n, float* d_policy, float* d_value, int precision, void* stream);
 
 /* ---------------------------------------------------------------- training step and TensorFlow checkpoints (SURVEY.md §8f N4) */
 /* One run of the graph's "optimize" op (AlphaZeroNN::train inner loop, neural_network/alphazero_nn.cpp:389-390;
    python/src/build_graph.py:92-106): training-mode forward (batch statistics, moving averages updated with momentum 0.99), softmax
-   cross-entropy + mean squared error + 0.001 * L2 of the kernels, Adam(0.001, 0.9, 0.999, 1e-8).  x [n][7][6][13], target policy
+   cross-entropy + mean squared error + 0.001 * L2 of the kernels, Adam(0.001, 0.9, 0.999, 1e-8).  x [n][7][6][input_planes], target policy
    [n][43], target value [n][value_outputs]; returns the batch's two losses (TF_OUTPUT_LOSS_POLICY / _VALUE; the value loss is the
    mean over all n * value_outputs squared errors).  fp32 on CUDA cores, deterministic. */
 AZ_API int az_nn_train_step(az_nn* nn, const float* h_x, const float* h_target_policy, const float* h_target_value, int n,
                             float* loss_policy, float* loss_value, void* stream);
 /* AlphaZeroNN::train (alphazero_nn.cpp:351-410) on packed sample records (az_selfplay_samples / the reference's sample files):
    `epochs` shuffled passes, whole batches of batch_size (SETTINGS.BATCH_SIZE = 512) only; per-epoch mean losses (may be NULL).
-   Rejects a network with six value outputs (a two-player record holds one value target) */
+   Rejects a network with six value outputs (a two-player record holds one value target) or 16 input planes (two-player records
+   encode 13) */
 AZ_API int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                        float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
 /* AZ_NN_FP32 (default, the parity path) or AZ_NN_BF16: the three convolution-shaped contractions of the step (forward, data gradient,
@@ -209,7 +218,7 @@ AZ_API int az_nn_train(az_nn* nn, const uint8_t* h_records, size_t n_records, in
 AZ_API int az_nn_train_precision(az_nn* nn, int precision);
 /* AlphaZeroNNGroup::train's hand-off to the group's copies on the other GPUs (alphazero_gpu_cluster.cpp:221-231 saves a temporary
    checkpoint and reloads it): every variable, the Adam slots and the beta powers from src to dst, device to device (peer copy over
-   NVLink) when the state lives on the device.  Same architecture required; synchronises `stream` */
+   NVLink) when the state lives on the device.  Same architecture (blocks, value outputs, input planes) required; synchronises `stream` */
 AZ_API int az_nn_copy_state(az_nn* dst, az_nn* src, void* stream);
 /* introspection for the parity tests: gradient of the total loss from the last step; Adam slots (which: 0 = m, 1 = v); beta powers */
 AZ_API int az_nn_train_get_grad(az_nn* nn, const char* name, float* h_out, size_t count);
@@ -248,7 +257,7 @@ typedef struct az_mcts az_mcts;
 /* one search tree (transposition table) per game of `env`; hyper-parameters come from the env's az_rules
    (mcts_simulations, threads_per_mcts -> sims - sims % t, cpuct, dir_noise_*, temperature_threshold).
    Replaces AlphaZeroMCTS (player/alpha_zero/alphazero_mcts.h:75-94) with THREADS_PER_MCTS = 1 semantics.  Evaluators AZ_EVAL_NN,
-   _PSEUDO, _UNIFORM; a network with six value outputs is rejected. */
+   _PSEUDO, _UNIFORM; a network with six value outputs or 16 input planes is rejected. */
 AZ_API int az_mcts_create(az_env* env, az_nn* nn, int evaluator, int precision, az_mcts** out);
 AZ_API int az_mcts_destroy(az_mcts* mcts);
 /* node-pool occupancy: the fullest pool any game had at the end of a search since the counters were reset, the capacity of a pool
@@ -348,6 +357,8 @@ AZ_API int az_env6_counters(az_env6* env, az_counters6* h_out, int reset, void* 
 /* the six-seat network input: the reference's [n][7][6][13] tensor with "enemy" = the seat that moves next, "neutral" = every other
    seat (SIXPLAYER.md), so the same tower evaluates it */
 AZ_API int az_env6_encode(az_env6* env, float* h_x, void* stream);
+/* the same with input_planes = 13 (az_env6_encode) or 16: [n][7][6][16], the seat planes of az_nn_create_planes */
+AZ_API int az_env6_encode_planes(az_env6* env, int input_planes, float* h_x, void* stream);
 /* the six-player SEARCH of SIXPLAYER.md: the reference's MCTS with the table cleared before every search and the six-seat value rule
    (a leaf's value belongs to the seat to move there: +v for that seat's nodes on the path, -v / 5 for the others); K =
    max(1, concurrent_descents) descents per tree per leaf batch under the reference's active_N rule, the two-player lockstep schedule
@@ -356,7 +367,8 @@ AZ_API int az_env6_encode(az_env6* env, float* h_x, void* stream);
    threads_per_mcts) that K does not divide.  Self-play, both pick modes, sample recording and the arena use the env's K.
    With a six-seat value vector (evaluator AZ_EVAL_NN over a network with six value outputs, or AZ_EVAL_PSEUDO6) a leaf's v[6] is
    relative to its seat to move L and a path node whose mover is s receives v[(s - L + 6) % 6]; a finished game backs up as above,
-   and the node's stored value (root statistics) is component 0.  A one-output network keeps the scalar rule bit for bit. */
+   and the node's stored value (root statistics) is component 0.  A one-output network keeps the scalar rule bit for bit.  Leaves are
+   encoded with the network's input planes (13, or the 16 seat planes). */
 typedef struct az_mcts6 az_mcts6;
 AZ_API int az_mcts6_create(az_env6* env, az_nn* nn, int evaluator, int precision, az_mcts6** out);
 AZ_API int az_mcts6_destroy(az_mcts6* mcts);
@@ -381,7 +393,8 @@ AZ_API int az_selfplay6_record(az_mcts6* mcts, size_t capacity_samples, int max_
 /* drains the six-player queue: the calling convention of az_selfplay_samples with AZ_SAMPLE6_BYTES records */
 AZ_API int az_selfplay6_samples(az_mcts6* mcts, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream);
 /* az_nn_train on AZ_SAMPLE6_BYTES records: the same shuffled epochs, whole batches, per-epoch mean losses and training precisions; the
-   input planes are the six-seat encoding of az_env6_encode, built on the device from each record's image.  With six value outputs
+   input planes are the six-seat encoding of az_env6_encode_planes with the network's plane count, built on the device from each
+   record's image.  With six value outputs
    target k of a record is the value rule above for seat (cur + k) % 6 (1 for the winner, -1/5 for another seat, 0 after a draw);
    component 0 is the stored float */
 AZ_API int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
