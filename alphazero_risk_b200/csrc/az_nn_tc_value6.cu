@@ -1,6 +1,7 @@
 // az_nn_tc_value6.cu — the translation unit of the bf16 tensor-core forward: az_nn_tc.cu itself (included byte for byte: the ncu capture
 // of its tower kernel in profiles/traffic.json is keyed by that file's hash) plus the value tail of a network with six value outputs
-// (SIXPLAYER.md §2, az_nn_create_value) and the input side of a network with 16 input planes (the seat planes, az_nn_create_planes).
+// (SIXPLAYER.md §2, az_nn_create_value) and the input side of a network with 16 input planes (the seat planes, az_nn_create_planes),
+// and the test entries that read the forward's work buffers (AzTcState and AzTcScratch are defined only in az_nn_tc.cu).
 //
 // A six-output network shares everything with the one-output graph up to dense_1: the same tower, the same 1x1 head convolutions (whose
 // per-cell sums the last tower layer's epilogue writes to d_head_z) and the same policy head.  So its forward is az_nn_tc_forward
@@ -9,6 +10,7 @@
 #define az_nn_tc_prepare az_nn_tc_prepare_13
 #include "az_nn_tc.cu"
 #undef az_nn_tc_prepare
+#include "az_tc_gemm.cuh"
 
 // value [n][6] for HB boards per block: BatchNorm + ReLU of the v channel, dense 42 -> 256 + ReLU, dense 256 -> 6, tanh; the
 // arithmetic of k_nn_heads_tail's value head, once per output column
@@ -138,4 +140,85 @@ int az_nn_tc_forward_planes16(az_nn* nn, const float* d_x, int n, float* d_polic
         AZ_CUDA(cudaGetLastError());
     }
     return AZ_OK;
+}
+
+// ---------------------------------------------------------------- test introspection (tests/test_tc_operands_gpu.py)
+// The work buffers of the bf16 forward and the training step's tensor-core contractions, for tests that check every contraction on the
+// operands it actually read against an fp64 reference.  Neither entry changes what a production call computes.
+
+// one buffer of scratch set `s` as of the last bf16 forward that used it: which = 0 the stem operand d_in (bf16 bits, [3 copies][2 chunks]
+// [r_alloc][8]), 1..3 d_act[0..2] (bf16 bits, [32][r_alloc][8], halos and padding rows included), 4 d_head_z (float4 [n][42]).
+// h_out == NULL with bytes == 0 only reports r_alloc (0 before the first forward).
+extern "C" int az_nn_tc_probe(az_nn* nn, int s, int which, int n, void* h_out, size_t bytes, int* r_alloc)
+{
+    AZ_REQUIRE(nn && nn->tc, "no bf16 forward state on this network");
+    AZ_REQUIRE(s >= 0 && s < AZ_TC_SCRATCH_SETS, "scratch set out of range");
+    AZ_REQUIRE(which >= 0 && which <= 4, "which must be 0 (input), 1..3 (activation buffers) or 4 (head sums)");
+    const AzTcScratch& tc = nn->tc->scratch[s];
+    if (r_alloc) *r_alloc = tc.r_alloc;
+    if (!h_out && bytes == 0) return AZ_OK;
+    AZ_REQUIRE(h_out != nullptr, "h_out is NULL");
+    AZ_REQUIRE(tc.cap_boards > 0, "no bf16 forward has run on this scratch set");
+    AZ_REQUIRE(n >= 1 && n <= tc.cap_boards, "n out of range");
+    const void* src = which == 0 ? (const void*)tc.d_in : which == 4 ? (const void*)tc.d_head_z : (const void*)tc.d_act[which - 1];
+    const size_t want = which == 0 ? (size_t)3 * 2 * tc.r_alloc * 16 : which == 4 ? sizeof(float4) * (size_t)n * 42 : (size_t)TC_CHUNKS * tc.r_alloc * 16;
+    AZ_REQUIRE(bytes == want, "byte count does not match the buffer");
+    AzDeviceGuard guard(nn->device);
+    AZ_CUDA(cudaDeviceSynchronize());
+    AZ_CUDA(cudaMemcpy(h_out, src, bytes, cudaMemcpyDeviceToHost));
+    return AZ_OK;
+}
+
+// The training step's tensor-core contractions through their production functions on fp32 host arrays (rounded to bf16 on the device):
+//   mode 0: out[n * 42][256] = conv(a[n * 42][256], w = b[9][256][256] HWIO)          az_tc_conv_raw, flip = 0
+//   mode 1: out[n * 42][256] = data gradient of dz = a through w = b                   az_tc_dz_prepare + az_tc_dgrad_prepared
+//   mode 2: out[9][256][256] = weight gradient of activation a with dz = b [n * 42][256]  az_tc_dz_prepare + az_tc_wgrad_prepared
+//           (at most max_splits K splits) + az_tg_reduce
+// n_warm > n first runs the same mode at n_warm boards with other data on the same scratch, so the measured call reuses buffers a larger
+// batch left dirty (and mode 1 / 2 take the n < dz_boards clearing path).
+extern "C" int az_tc_conv_test(int mode, const float* h_a, const float* h_b, int n, int n_warm, int max_splits, float* h_out)
+{
+    AZ_REQUIRE(h_a && h_b && h_out, "NULL argument");
+    AZ_REQUIRE(mode >= 0 && mode <= 2, "mode must be 0 (forward), 1 (data gradient) or 2 (weight gradient)");
+    AZ_REQUIRE(n >= 1 && n_warm >= 0 && max_splits >= 1 && max_splits <= 64, "bad argument");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); az_set_error("no CUDA device: libaz_b200 has no CPU fallback"); return AZ_ERR_NO_DEVICE; }
+    const int n_max = n_warm > n ? n_warm : n;
+    const size_t rows_max = (size_t)n_max * 42 * 256, wsz = (size_t)9 * 256 * 256;
+    const size_t b_elems = mode == 2 ? rows_max : wsz, out_elems = mode == 2 ? wsz : rows_max;
+    AzTcConvScratch sc;
+    float *d_a = nullptr, *d_b = nullptr, *d_out = nullptr, *d_part = nullptr;
+    int rc = AZ_OK;
+    cudaError_t ce = cudaMalloc(&d_a, rows_max * sizeof(float));
+    if (ce == cudaSuccess) ce = cudaMalloc(&d_b, b_elems * sizeof(float));
+    if (ce == cudaSuccess) ce = cudaMalloc(&d_out, out_elems * sizeof(float));
+    if (ce == cudaSuccess && mode == 2) ce = cudaMalloc(&d_part, (size_t)max_splits * wsz * sizeof(float));
+    auto run = [&](int nb) -> int {
+        if (mode == 0) return az_tc_conv_raw(&sc, d_a, nb, d_b, 0, d_out, 0);
+        int r = az_tc_dz_prepare(&sc, mode == 1 ? d_a : d_b, nb, 0); if (r) return r;
+        if (mode == 1) return az_tc_dgrad_prepared(&sc, nb, d_b, d_out, 0);
+        int splits = 0;
+        r = az_tc_wgrad_prepared(&sc, d_a, nb, d_part, max_splits, &splits, 0); if (r) return r;
+        return az_tg_reduce(d_part, splits, 9 * 256, 9 * 256, d_out, 0);
+    };
+    if (ce == cudaSuccess && n_warm > n) {
+        // other data, exact in bf16: small multiples of 1/64 from a multiplicative hash of the index
+        std::vector<float> wa(rows_max), wb(b_elems);
+        for (size_t i = 0; i < wa.size(); ++i) wa[i] = (float)((uint32_t)(i * 2654435761u) >> 26) / 64.0f - 0.5f;
+        for (size_t i = 0; i < wb.size(); ++i) wb[i] = mode == 2 ? (float)((uint32_t)(i * 2246822519u) >> 26) / 64.0f - 0.5f : h_b[i];
+        ce = cudaMemcpy(d_a, wa.data(), wa.size() * sizeof(float), cudaMemcpyHostToDevice);
+        if (ce == cudaSuccess) ce = cudaMemcpy(d_b, wb.data(), wb.size() * sizeof(float), cudaMemcpyHostToDevice);
+        if (ce == cudaSuccess) rc = run(n_warm);
+        if (ce == cudaSuccess && rc == AZ_OK) ce = cudaDeviceSynchronize();
+    }
+    const size_t a_elems = (size_t)n * 42 * 256;
+    if (ce == cudaSuccess && rc == AZ_OK) ce = cudaMemcpy(d_a, h_a, a_elems * sizeof(float), cudaMemcpyHostToDevice);
+    if (ce == cudaSuccess && rc == AZ_OK) ce = cudaMemcpy(d_b, h_b, (mode == 2 ? a_elems : wsz) * sizeof(float), cudaMemcpyHostToDevice);
+    if (ce == cudaSuccess && rc == AZ_OK) rc = run(n);
+    if (ce == cudaSuccess && rc == AZ_OK) ce = cudaDeviceSynchronize();
+    if (ce == cudaSuccess && rc == AZ_OK) ce = cudaMemcpy(h_out, d_out, (mode == 2 ? wsz : a_elems) * sizeof(float), cudaMemcpyDeviceToHost);
+    az_tc_conv_raw_release(&sc);
+    cudaFree(d_a); cudaFree(d_b); cudaFree(d_out); cudaFree(d_part);
+    if (ce != cudaSuccess) { az_set_error("az_tc_conv_test: %s", cudaGetErrorString(ce)); cudaGetLastError(); return AZ_ERR_CUDA; }
+    return rc;
 }

@@ -223,6 +223,15 @@ AZ_API int az_nn_copy_state(az_nn* dst, az_nn* src, void* stream);
 /* introspection for the parity tests: gradient of the total loss from the last step; Adam slots (which: 0 = m, 1 = v); beta powers */
 AZ_API int az_nn_train_get_grad(az_nn* nn, const char* name, float* h_out, size_t count);
 AZ_API int az_nn_train_get_layer(az_nn* nn, int layer, int which /* 0 = convolution output, 1 = activation */, float* h_out, size_t count);
+/* test introspection of the bf16 tensor-core path.  az_nn_tc_probe: one work buffer of scratch set s as of the last bf16 forward that
+   used it — which = 0 the stem operand (bf16 bits, [3 copies][2 chunks][r_alloc][8]), 1..3 the activation buffers (bf16 bits,
+   [32 chunks][r_alloc][8], halo and padding rows included), 4 the per-cell head sums (float4 [n][42]); bytes must be the buffer's size
+   (h_out = NULL with bytes = 0 reports r_alloc only).  az_tc_conv_test: the training step's contractions through their production
+   functions — mode 0 forward conv(a [n*42][256], b = w [9][256][256] HWIO), mode 1 data gradient of dz = a through w = b, mode 2
+   weight gradient [9][256][256] of activation a with dz = b [n*42][256] in at most max_splits K splits; n_warm > n first runs the same
+   mode at n_warm boards with other data on the same scratch */
+AZ_API int az_nn_tc_probe(az_nn* nn, int s, int which, int n, void* h_out, size_t bytes, int* r_alloc);
+AZ_API int az_tc_conv_test(int mode, const float* h_a, const float* h_b, int n, int n_warm, int max_splits, float* h_out);
 AZ_API int az_nn_optimizer_get(az_nn* nn, const char* name, int which, float* h_out, size_t count);
 AZ_API int az_nn_optimizer_powers(az_nn* nn, float* beta1_power, float* beta2_power, uint64_t* steps);
 /* AlphaZeroNN::saveCheckpoint / loadCheckpoint (alphazero_nn.cpp:189-214): TensorFlow V2 checkpoint bundle <prefix>.index +
