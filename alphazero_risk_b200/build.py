@@ -21,7 +21,7 @@ COMMON = ["-std=c++17", "-O3", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler",
 # A unit may include another .cu whose bytes must stay as they are (profiles/traffic.json keys its ncu captures by source hashes):
 # INCLUDED lists those files, so that a change to them rebuilds the unit.
 UNITS = {
-    "az_env.cu": ["-fmad=false"],
+    "az_env_rollout.cu": ["-fmad=false"],    # az_env.cu (included unchanged) + the rollout with the land bytes kept in the pool slot
     "az_mcts_value6.cu": ["-fmad=false"],    # az_mcts.cu (included unchanged) + az_mcts_create's six-output check
     "az_nn.cu": [],
     "az_nn_tc_value6.cu": [],                # az_nn_tc.cu (included unchanged) + the six-output value tail
@@ -34,7 +34,7 @@ UNITS = {
 }
 
 
-INCLUDED = {"az_mcts_value6.cu": ["az_mcts.cu"], "az_nn_tc_value6.cu": ["az_nn_tc.cu"]}
+INCLUDED = {"az_env_rollout.cu": ["az_env.cu"], "az_mcts_value6.cu": ["az_mcts.cu"], "az_nn_tc_value6.cu": ["az_nn_tc.cu"]}
 
 
 def _newer(src_files, target):
