@@ -145,6 +145,7 @@ def lib():
         L.az_env6_last_kernel_ms.argtypes = [vp, C.POINTER(C.c_float)]
         L.az_env6_step.argtypes = [vp, vp, vp, vp]
         L.az_env6_query.argtypes = [vp, vp, vp, vp]
+        L.az_env6_script_actions.argtypes = [vp, vp, vp]
         L.az_env6_export.argtypes = [vp, vp, vp]
         L.az_env6_import.argtypes = [vp, vp, vp]
         L.az_env6_counters.argtypes = [vp, C.POINTER(AzCounters6), C.c_int, vp]
@@ -160,6 +161,7 @@ def lib():
         L.az_selfplay6_samples.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_uint64), vp]
         L.az_nn_train6.argtypes = [vp, vp, C.c_size_t, C.c_int, C.c_int, C.c_uint64, vp, vp, vp]
         L.az_arena6_create.argtypes = [vp, C.POINTER(vp), C.c_int, vp, C.c_int, C.POINTER(vp)]
+        L.az_arena6_create_agents.argtypes = [vp, C.POINTER(vp), vp, C.c_int, vp, C.c_int, C.POINTER(vp)]
         L.az_arena6_destroy.argtypes = [vp]
         L.az_arena6_play.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(AzArena6Results), vp, vp, vp]
         L.az_arena6_active_slots.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t)]
@@ -762,6 +764,12 @@ class Env6:
         check(self.L.az_env6_query(self.h, _ptr(v), _ptr(st), stream))
         return v, st
 
+    def script_actions(self, stream=None):
+        """the scripted agent's action (SIXPLAYER.md §5) for every game's position, uint8 [n]; 0xff for a finished game"""
+        a = np.empty(self.n, np.uint8)
+        check(self.L.az_env6_script_actions(self.h, _ptr(a), stream))
+        return a
+
     def export(self, stream=None):
         a = np.empty((self.n, ENV6_IMAGE_BYTES), np.uint8)
         check(self.L.az_env6_export(self.h, _ptr(a), stream))
@@ -851,18 +859,33 @@ class AzArena6Results(C.Structure):
                     errors=int(self.errors))
 
 
+# agent kinds of az_arena6_create_agents (include/az_b200.h)
+AGENT6_SEARCHER, AGENT6_RANDOM, AGENT6_SCRIPT = 0, 1, 2
+
+
+class _Script6:
+    def __repr__(self):
+        return "SCRIPT6"
+
+
+# the scripted six-player agent (SIXPLAYER.md §5) as an Arena6 agent, next to Mcts6 handles and None (the uniform-random player)
+SCRIPT6 = _Script6()
+
+
 class Arena6:
-    """six-player matches on the device (az_arena6_*, SIXPLAYER.md §4): `agents` are Mcts6 handles over `env` or None (the
-    uniform-random player), seat_agent[s] = the agent index that holds seat s; with rotate_seats the six games of a group share
-    one deal and rotate the seats"""
+    """six-player matches on the device (az_arena6_*, SIXPLAYER.md §4): `agents` are Mcts6 handles over `env`, None (the
+    uniform-random player) or SCRIPT6 (the scripted agent, SIXPLAYER.md §5), seat_agent[s] = the agent index that holds seat s;
+    with rotate_seats the six games of a group share one deal and rotate the seats"""
 
     def __init__(self, env, agents, seat_agent, rotate_seats=True):
         self.L, self.env, self.agents = lib(), env, list(agents)
-        hs = (C.c_void_p * max(1, len(self.agents)))(*[a.h if a is not None else None for a in self.agents])
+        kinds = [AGENT6_RANDOM if a is None else AGENT6_SCRIPT if a is SCRIPT6 else AGENT6_SEARCHER for a in self.agents]
+        hs = (C.c_void_p * max(1, len(self.agents)))(*[a.h if k == AGENT6_SEARCHER else None for a, k in zip(self.agents, kinds)])
+        ks = np.ascontiguousarray(kinds if kinds else [0], np.int32)
         seats = np.ascontiguousarray(seat_agent, np.uint8)
         assert seats.shape == (6,)
         h = C.c_void_p()
-        check(self.L.az_arena6_create(env.h, hs, len(self.agents), _ptr(seats), int(rotate_seats), C.byref(h)))
+        check(self.L.az_arena6_create_agents(env.h, hs, _ptr(ks), len(self.agents), _ptr(seats), int(rotate_seats), C.byref(h)))
         self.h = h
 
     def close(self):

@@ -52,7 +52,8 @@ struct Arena6Dev {
     uint32_t* out_plies;        // [n_games]  and its plies
     unsigned long long* res;    // [A6_N]
     uint32_t seat_agent;        // agent index of seat s in bits 4s .. 4s + 3
-    uint8_t searcher;           // bit a: agent a is a searcher (else the uniform-random player)
+    uint8_t searcher;           // bit a: agent a is a searcher
+    uint8_t script;             // bit a: agent a is the scripted agent (SIXPLAYER.md §5); neither bit: the uniform-random player
     uint8_t rotate;
 };
 

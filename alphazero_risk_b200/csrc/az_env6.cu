@@ -20,6 +20,7 @@
 
 #define E6_BLOCK 128                    // configs[3] has 16384 games per GPU: 128 blocks = four warps on 128 of the 148 SMs (256: 64 SMs)
 #include "az_game6.cuh"
+#include "az_script6.cuh"
 
 struct E6Smem {
     uint64_t tab[AZ_TABLE_U64];
@@ -138,6 +139,18 @@ __global__ void __launch_bounds__(E6_BLOCK) k_env6_query(const uint32_t* __restr
     if (status) status[gi] = (int8_t)e6_status(c.g, rules);
 }
 
+// the scripted action of every game (SIXPLAYER.md §5), 0xff for a finished game
+__global__ void __launch_bounds__(E6_BLOCK) k_env6_script(const uint32_t* __restrict__ st, int n, const uint64_t* __restrict__ g_tab,
+                                                         AzRulesDev rules, uint8_t* __restrict__ action)
+{
+    __shared__ E6Smem sm;
+    const AzTables T = e6_stage(sm, g_tab);
+    const int gi = blockIdx.x * E6_BLOCK + threadIdx.x;
+    if (gi >= n) return;
+    E6Ctx c; e6_load(c, sm, st, n, gi);
+    action[gi] = e6_status(c.g, rules) != AZ_STATUS_RUNNING ? (uint8_t)0xff : (uint8_t)e6_script_action(c, T, rules);
+}
+
 // 108-byte host image (== r6_state of the oracle): army[42], owner[42], cards[6], pool[6], round u16, cur, card_sets, reinf,
 // phase, mob_from, mob_to, allow_draw, attacks, 2 pad bytes
 __global__ void __launch_bounds__(E6_BLOCK) k_env6_export(const uint32_t* __restrict__ st, int n, uint8_t* __restrict__ img)
@@ -181,14 +194,14 @@ __global__ void __launch_bounds__(E6_BLOCK) k_env6_import(uint32_t* __restrict__
 
 // ---------------------------------------------------------------- six-player arena (SIXPLAYER.md §4): everything between two searches
 // One thread per slot: tally the slot's finished game (per-game status and plies on the device), claim the next match game from
-// the shared counter and deal it (deal of game id g - g % 6 with rotation, else g; ply 0), play the uniform-random player's plies
-// (az_env6_rollout's rule keyed by the match game id), and stop when a searcher's seat is to move: to_move = that agent.  At most
-// 64 iterations per launch, like k_arena_advance.  res[A6_ACTIVE] counts the slots that hold a game afterwards, res[A6_WAIT0 + a]
-// those waiting for agent a's search.
+// the shared counter and deal it (deal of game id g - g % 6 with rotation, else g; ply 0), play the plies of the uniform-random player
+// (az_env6_rollout's rule keyed by the match game id) and of the scripted agent (e6_script_action, SIXPLAYER.md §5; the same dice),
+// and stop when a searcher's seat is to move: to_move = that agent.  At most 64 iterations per launch, like k_arena_advance.
+// res[A6_ACTIVE] counts the slots that hold a game afterwards, res[A6_WAIT0 + a] those waiting for agent a's search.
 __global__ void __launch_bounds__(E6_BLOCK) k_arena6_advance(Arena6Dev a, const uint64_t* __restrict__ g_tab, AzRulesDev rules)
 {
     __shared__ E6Smem sm;
-    __shared__ unsigned s_cnt[1 + 2 * E6_PLAYERS];    // active slots, waiting slots per agent, random plies per agent
+    __shared__ unsigned s_cnt[1 + 2 * E6_PLAYERS];    // active slots, waiting slots per agent, random / scripted plies per agent
     if (threadIdx.x < 1 + 2 * E6_PLAYERS) s_cnt[threadIdx.x] = 0;
     const AzTables T = e6_stage(sm, g_tab);           // (its barrier also orders the zeroing above)
     const int gi = blockIdx.x * E6_BLOCK + threadIdx.x;
@@ -227,9 +240,13 @@ __global__ void __launch_bounds__(E6_BLOCK) k_arena6_advance(Arena6Dev a, const 
             }
             const uint32_t agent = (a.seat_agent >> (4 * ((c.g.cur + r) % E6_PLAYERS))) & 0xfu;
             if ((a.searcher >> agent) & 1u) { wait = (int)agent; break; }
-            const uint64_t valid = e6_valid(c.g, T, rules);
             const az_u32x4 blk = az_rng_block(a.seed, game, c.ply, AZ_STREAM_REAL, 0);
-            const int action = az_nth_set_bit(valid, az_mulhi32(blk.y, (uint32_t)__popcll(valid)));
+            int action;
+            if ((a.script >> agent) & 1u) action = e6_script_action(c, T, rules);
+            else {
+                const uint64_t valid = e6_valid(c.g, T, rules);
+                action = az_nth_set_bit(valid, az_mulhi32(blk.y, (uint32_t)__popcll(valid)));
+            }
             { E6DiceWord dice; dice.w = blk.x; e6_move(c, T, rules, action, dice); }
             c.ply++;
             atomicAdd(&s_cnt[1 + E6_PLAYERS + agent], 1u);
@@ -388,6 +405,18 @@ extern "C" int az_env6_query(az_env6* e, uint64_t* h_valid, int8_t* h_status, vo
     AZ_CUDA(cudaGetLastError());
     if (h_valid) AZ_CUDA(cudaMemcpyAsync(h_valid, e->d_valid, sizeof(uint64_t) * (size_t)e->n, cudaMemcpyDeviceToHost, s));
     if (h_status) AZ_CUDA(cudaMemcpyAsync(h_status, e->d_status, (size_t)e->n, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
+    return AZ_OK;
+}
+
+extern "C" int az_env6_script_actions(az_env6* e, uint8_t* h_action, void* stream)
+{
+    AZ_REQUIRE(e && h_action, "NULL argument");
+    AzDeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    k_env6_script<<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, az_device_tables(), e6_rules(e->rules), e->d_action);
+    AZ_CUDA(cudaGetLastError());
+    AZ_CUDA(cudaMemcpyAsync(h_action, e->d_action, (size_t)e->n, cudaMemcpyDeviceToHost, s));
     AZ_CUDA(cudaStreamSynchronize(s));
     return AZ_OK;
 }

@@ -796,12 +796,12 @@ extern "C" int az_env6_encode_planes(az_env6* e, int input_planes, float* h_x, v
 extern "C" int az_env6_encode(az_env6* e, float* h_x, void* stream) { return az_env6_encode_planes(e, AZ_NN_IN_CH, h_x, stream); }
 
 // ---------------------------------------------------------------- six-player arena (SIXPLAYER.md §4)
-// k_arena6_advance (az_env6.cu) tallies, deals and plays the random player's plies; each tick then runs one search per searcher
+// k_arena6_advance (az_env6.cu) tallies, deals and plays the random and scripted agents' plies; each tick then runs one search per searcher
 // restricted to the slots waiting for it (Mcts6Dev::sel over to_move), with the slots' match game ids as the search's game ids, and
 // its leaf batches compacted to those slots.  A searcher's move can hand the turn to another agent: that slot waits for the next tick.
 struct az_arena6 {
     az_env6* env = nullptr;
-    az_mcts6* agent[E6_PLAYERS] = {};    // NULL = the uniform-random player
+    az_mcts6* agent[E6_PLAYERS] = {};    // NULL = the uniform-random player or the scripted agent (Arena6Dev::script)
     int n_agents = 0;
     Arena6Dev a;
     int32_t* d_list = nullptr;           // slots waiting for the searcher of this search (leaf-batch compaction)
@@ -826,10 +826,17 @@ template <class T> static int a6_alloc(az_arena6* ar, T** p, size_t count)
     return AZ_OK;
 }
 
-extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_agents, const uint8_t* seat_agent, int rotate_seats, az_arena6** out)
+extern "C" int az_arena6_create_agents(az_env6* env, az_mcts6* const* agents, const int* kinds, int n_agents, const uint8_t* seat_agent,
+                                       int rotate_seats, az_arena6** out)
 {
-    AZ_REQUIRE(env && agents && seat_agent && out, "NULL argument");
+    AZ_REQUIRE(env && agents && kinds && seat_agent && out, "NULL argument");
     AZ_REQUIRE(n_agents >= 1 && n_agents <= E6_PLAYERS, "n_agents must be in 1..6");
+    for (int i = 0; i < n_agents; ++i) {
+        AZ_REQUIRE(kinds[i] == AZ_AGENT6_SEARCHER || kinds[i] == AZ_AGENT6_RANDOM || kinds[i] == AZ_AGENT6_SCRIPT,
+                   "unknown agent kind (AZ_AGENT6_SEARCHER, AZ_AGENT6_RANDOM or AZ_AGENT6_SCRIPT)");
+        AZ_REQUIRE((kinds[i] == AZ_AGENT6_SEARCHER) == (agents[i] != nullptr),
+                   "agents[i] must be an az_mcts6 handle for a searcher and NULL for the random or scripted agent");
+    }
     for (int i = 0; i < n_agents; ++i) {
         if (!agents[i]) continue;
         AZ_REQUIRE(agents[i]->env == env, "every searcher must be built over the arena's env (the agents share its game states)");
@@ -849,7 +856,11 @@ extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_age
     memset(&a, 0, sizeof a);
     a.n = az_env6_n(env); a.state = az_env6_state_ptr(env); a.rotate = rotate_seats ? 1 : 0;
     for (int s = 0; s < E6_PLAYERS; ++s) a.seat_agent |= (uint32_t)seat_agent[s] << (4 * s);
-    for (int i = 0; i < n_agents; ++i) { ar->agent[i] = agents[i]; if (agents[i]) a.searcher |= (uint8_t)(1u << i); }
+    for (int i = 0; i < n_agents; ++i) {
+        ar->agent[i] = agents[i];
+        if (kinds[i] == AZ_AGENT6_SEARCHER) a.searcher |= (uint8_t)(1u << i);
+        if (kinds[i] == AZ_AGENT6_SCRIPT) a.script |= (uint8_t)(1u << i);
+    }
     const size_t n = (size_t)a.n;
     size_t ns = n, nv = n;                                              // the largest compacted leaf batch: K * n, and its values K * n * vo
     for (int i = 0; i < n_agents; ++i) if (agents[i]) {
@@ -863,6 +874,15 @@ extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_age
     if (rc) { for (void* p : ar->allocs) cudaFree(p); delete ar; return AZ_ERR_CUDA; }
     *out = ar;
     return AZ_OK;
+}
+
+extern "C" int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_agents, const uint8_t* seat_agent, int rotate_seats, az_arena6** out)
+{
+    AZ_REQUIRE(agents != nullptr, "NULL argument");
+    AZ_REQUIRE(n_agents >= 1 && n_agents <= E6_PLAYERS, "n_agents must be in 1..6");
+    int kinds[E6_PLAYERS];
+    for (int i = 0; i < n_agents; ++i) kinds[i] = agents[i] ? AZ_AGENT6_SEARCHER : AZ_AGENT6_RANDOM;
+    return az_arena6_create_agents(env, agents, kinds, n_agents, seat_agent, rotate_seats, out);
 }
 
 extern "C" int az_arena6_destroy(az_arena6* ar)

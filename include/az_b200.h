@@ -408,9 +408,13 @@ AZ_API int az_selfplay6_samples(az_mcts6* mcts, uint8_t* h_records, size_t max_r
    component 0 is the stored float */
 AZ_API int az_nn_train6(az_nn* nn, const uint8_t* h_records, size_t n_records, int epochs, int batch_size, uint64_t seed,
                         float* h_epoch_loss_policy, float* h_epoch_loss_value, void* stream);
-/* ---- six-player arena (SIXPLAYER.md §4): seat-rotated matches between searchers and the uniform-random player over one env6.
-   An agent is an az_mcts6 handle over `env` (argmax play, table cleared per search) or NULL = the uniform-random player
-   (az_env6_rollout's rule).  seat_agent[s] = the agent index that holds seat s; every agent holds at least one seat.  Match game g
+/* the scripted agent's action (SIXPLAYER.md §5) for the current position of every game, one byte per game: a land 0..41 or 42 =
+   skip, always legal; 0xff for a finished game.  A pure function of the position and the env's rules (no randomness, no memory);
+   az_env6_step with these actions plays the scripted agent's ply with the real-move dice, as the arena does. */
+AZ_API int az_env6_script_actions(az_env6* env, uint8_t* h_action, void* stream);
+/* ---- six-player arena (SIXPLAYER.md §4): seat-rotated matches between searchers, the uniform-random player and the scripted agent
+   over one env6.  An agent is an az_mcts6 handle over `env` (argmax play, table cleared per search), the uniform-random player
+   (az_env6_rollout's rule) or the scripted agent (az_env6_script_actions' rule, SIXPLAYER.md §5).  seat_agent[s] = the agent index that holds seat s; every agent holds at least one seat.  Match game g
    (first_game <= g < first_game + n_games) starts from the deal of game id d (e6_new_game(seed, d, 0)) with ply 0; with rotate_seats
    d = g - g % 6 and seat s is played by seat_agent[(s + g % 6) % 6] (the six games of a group share one deal, every agent sits in
    every seat), without it d = g and seat s by seat_agent[s].  All randomness of a ply is keyed by (seed, g, ply), so a game's
@@ -424,8 +428,15 @@ typedef struct az_arena6_results {
     uint64_t moves[6];      /* plies played, by agent index */
     uint64_t sims, evals, ticks, errors;   /* errors = the searchers' overflow counters, must be 0 */
 } az_arena6_results;
-/* agents[i] == NULL: the uniform-random player.  Rejects handles over another env, the same handle twice, n_agents outside 1..6,
+#define AZ_AGENT6_SEARCHER 0
+#define AZ_AGENT6_RANDOM 1
+#define AZ_AGENT6_SCRIPT 2
+/* kinds[i] = the kind of agent i; agents[i] is an az_mcts6 handle for AZ_AGENT6_SEARCHER and NULL for the other kinds.  Rejects
+   unknown kinds, a handle that does not match its kind, handles over another env, the same handle twice, n_agents outside 1..6,
    seat_agent entries >= n_agents and agents without a seat */
+AZ_API int az_arena6_create_agents(az_env6* env, az_mcts6* const* agents, const int* kinds /*[n_agents]*/, int n_agents,
+                                   const uint8_t* seat_agent /*[6]*/, int rotate_seats, az_arena6** out);
+/* az_arena6_create_agents with agents[i] == NULL meaning the uniform-random player and a handle a searcher */
 AZ_API int az_arena6_create(az_env6* env, az_mcts6* const* agents, int n_agents, const uint8_t* seat_agent /*[6]*/,
                             int rotate_seats, az_arena6** out);
 AZ_API int az_arena6_destroy(az_arena6* arena);
