@@ -146,6 +146,9 @@ def lib():
         L.az_env6_step.argtypes = [vp, vp, vp, vp]
         L.az_env6_query.argtypes = [vp, vp, vp, vp]
         L.az_env6_script_actions.argtypes = [vp, vp, vp]
+        L.az_env6_play.argtypes = [vp, vp, C.c_uint32, C.c_int, vp]
+        L.az_env6_record.argtypes = [vp, C.c_size_t, C.c_int]
+        L.az_env6_samples.argtypes = [vp, vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_uint64), vp]
         L.az_env6_export.argtypes = [vp, vp, vp]
         L.az_env6_import.argtypes = [vp, vp, vp]
         L.az_env6_counters.argtypes = [vp, C.POINTER(AzCounters6), C.c_int, vp]
@@ -769,6 +772,34 @@ class Env6:
         a = np.empty(self.n, np.uint8)
         check(self.L.az_env6_script_actions(self.h, _ptr(a), stream))
         return a
+
+    def play(self, seat_kinds, n_plies, record_seats=0, stream=None):
+        """n_plies plies of every game by scripted and uniform-random seats (az_env6_play, SIXPLAYER.md §6): seat_kinds[s] is None
+        (the uniform-random player) or SCRIPT6; bit s of record_seats records the plies of seat s (record() first)"""
+        kinds = list(seat_kinds)
+        assert len(kinds) == 6, "seat_kinds needs six entries"
+        for k in kinds:
+            if k is not None and k is not SCRIPT6:
+                raise AzError("a seat of Env6.play is None (the random player) or SCRIPT6, not %r" % (k,))
+        ks = np.ascontiguousarray([AGENT6_SCRIPT if k is SCRIPT6 else AGENT6_RANDOM for k in kinds], np.int32)
+        seats = int(record_seats)
+        if not 0 <= seats < 64:                  # c_uint32 would wrap a larger value into range
+            raise AzError("record_seats must be in 0..63, not %d" % seats)
+        check(self.L.az_env6_play(self.h, _ptr(ks), C.c_uint32(seats), int(n_plies), stream))
+
+    def record(self, capacity_samples, max_samples_per_game=4096):
+        """enable recording in play() (az_env6_record).  Staging costs 112 bytes x max_samples_per_game per game on the device:
+        about 7.5 GB for 16384 games at the default 4096; a game with more recorded plies is dropped whole and counted"""
+        check(self.L.az_env6_record(self.h, C.c_size_t(int(capacity_samples)), int(max_samples_per_game)))
+
+    def samples(self, stream=None):
+        """records of the finished games of play() as a [k, SAMPLE6_BYTES] uint8 array and the dropped count (az_env6_samples)"""
+        n, dropped = C.c_size_t(0), C.c_uint64(0)
+        check(self.L.az_env6_samples(self.h, None, C.c_size_t(0), C.byref(n), C.byref(dropped), stream))
+        out = np.empty((n.value, SAMPLE6_BYTES), np.uint8)
+        if n.value:          # an empty queue was drained (and its dropped count reset) by the query itself
+            check(self.L.az_env6_samples(self.h, _ptr(out), C.c_size_t(n.value), C.byref(n), C.byref(dropped), stream))
+        return out[:n.value], int(dropped.value)
 
     def export(self, stream=None):
         a = np.empty((self.n, ENV6_IMAGE_BYTES), np.uint8)

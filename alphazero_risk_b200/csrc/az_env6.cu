@@ -21,6 +21,7 @@
 #define E6_BLOCK 128                    // configs[3] has 16384 games per GPU: 128 blocks = four warps on 128 of the 148 SMs (256: 64 SMs)
 #include "az_game6.cuh"
 #include "az_script6.cuh"
+#include "az_samples6.cuh"
 
 struct E6Smem {
     uint64_t tab[AZ_TABLE_U64];
@@ -149,6 +150,106 @@ __global__ void __launch_bounds__(E6_BLOCK) k_env6_script(const uint32_t* __rest
     if (gi >= n) return;
     E6Ctx c; e6_load(c, sm, st, n, gi);
     action[gi] = e6_status(c.g, rules) != AZ_STATUS_RUNNING ? (uint8_t)0xff : (uint8_t)e6_script_action(c, T, rules);
+}
+
+// ---------------------------------------------------------------- generated games (SIXPLAYER.md §6)
+// state words 22..26 of the game's scalars, packed as e6_store packs them (e6_store keeps its own copy: the SASS of the kernels that
+// existed before generated games stays as it was)
+__device__ __forceinline__ void e6_pack_scalars(const AzGame6& g, uint32_t w[5])
+{
+    w[0] = g.cards_lo;
+    w[1] = (g.cards_hi & 0xffffu) | ((g.allow_draw & 0xffu) << 16) | ((g.attacks & 0xffu) << 24);
+    w[2] = (g.round & 0xffffu) | (g.cur << 16) | (g.card_sets << 24);
+    w[3] = (g.reinf & 0xffu) | (g.phase << 8) | (g.mob_from << 16) | (g.mob_to << 24);
+    w[4] = g.pools & 0xffffffu;
+}
+// recording of az_env6_play (az_env6_record): the samples of each slot's running game are staged until the game ends
+struct E6RecDev {
+    uint32_t* stage = nullptr;                  // [n][max][28]  state words 0..26 before the ply, then the played action
+    uint32_t* len = nullptr;                    // [n]           staged samples of the running game (> max = overflowed)
+    uint8_t* out = nullptr;                     // [cap][288]    records of finished games
+    unsigned long long* count = nullptr;        // [2]           records in out, samples dropped (staging or queue full)
+    int max = 0;
+    unsigned long long cap = 0;
+};
+#define E6_STAGE_WORDS 28
+
+// the `len` staged samples of slot gi's game, which ended with `status` -> one contiguous block of records (az_rec_reserve: a game
+// that overflowed its staging or does not fit is dropped whole and counted).  The game's own thread writes its block, 16 bytes a store.
+__device__ __noinline__ void e6_rec_flush(E6RecDev r, int gi, uint32_t len, int status)
+{
+    unsigned long long base = 0;
+    if (!az_rec_reserve(r.count, r.cap, len, len <= (uint32_t)r.max, &base)) return;
+    const uint4* src = (const uint4*)(r.stage + (size_t)gi * r.max * E6_STAGE_WORDS);
+    uint4* dst = (uint4*)(r.out + base * S6_BYTES);
+    for (uint32_t i = 0; i < len; ++i, src += E6_STAGE_WORDS / 4, dst += S6_BYTES / 16) {
+        uint32_t w[E6_STAGE_WORDS];
+#pragma unroll
+        for (int q = 0; q < E6_STAGE_WORDS / 4; ++q) { const uint4 v = src[q]; w[4 * q] = v.x; w[4 * q + 1] = v.y; w[4 * q + 2] = v.z; w[4 * q + 3] = v.w; }
+        const int action = (int)w[E6_STAGE_WORDS - 1];
+#pragma unroll
+        for (int q = 0; q < S6_BYTES / 16; ++q)
+            dst[q] = make_uint4(s6_onehot_record_word(w, action, status, 4 * q), s6_onehot_record_word(w, action, status, 4 * q + 1),
+                                s6_onehot_record_word(w, action, status, 4 * q + 2), s6_onehot_record_word(w, action, status, 4 * q + 3));
+    }
+}
+
+// n_plies plies of every game, the seat to move playing by `script` (bit s set: seat s is the scripted agent, e6_script_action; clear:
+// the uniform-random player, k_env6_rollout's rule), both with the real-move dice of (seed, game, ply); finished games are counted
+// and re-dealt in place on k_env6_rollout's schedule, so six random seats are k_env6_rollout bit for bit.  REC: every ply of a seat
+// in `record_seats` stages (state before the ply, action); a game's samples become records by the end of the call in which it ends.
+template <bool REC>
+__global__ void __launch_bounds__(E6_BLOCK) k_env6_play(uint32_t* __restrict__ st, int n, const uint64_t* __restrict__ g_tab, int n_plies,
+                                                       uint64_t seed, uint32_t first_game, AzRulesDev rules, uint32_t script,
+                                                       uint32_t record_seats, E6RecDev rec, unsigned long long* __restrict__ counters)
+{
+    __shared__ E6Smem sm;
+    const AzTables T = e6_stage(sm, g_tab);
+    const int gi = blockIdx.x * E6_BLOCK + threadIdx.x;
+    if (gi >= n) return;
+    E6Ctx c; e6_load(c, sm, st, n, gi);
+    const uint32_t game = first_game + (uint32_t)gi;
+    unsigned games = 0, draws = 0;
+    uint32_t len = REC ? rec.len[gi] : 0u;
+    for (int s = 0; s < n_plies; ++s) {
+        const int stt = e6_status(c.g, rules);
+        if (stt != AZ_STATUS_RUNNING) {
+            games++;
+            if (stt == AZ_STATUS_DRAW) draws++; else atomicAdd(&counters[3 + stt], 1ull);
+            if (REC && len) { e6_rec_flush(rec, gi, len, stt); len = 0; }
+            e6_new_game(c, seed, game, c.ply);
+        }
+        const az_u32x4 blk = az_rng_block(seed, game, c.ply, AZ_STREAM_REAL, 0);
+        int action;
+        if ((script >> c.g.cur) & 1u) action = e6_script_action(c, T, rules);
+        else {
+            const uint64_t valid = e6_valid(c.g, T, rules);
+            action = az_nth_set_bit(valid, az_mulhi32(blk.y, (uint32_t)__popcll(valid)));
+        }
+        if (REC && ((record_seats >> c.g.cur) & 1u)) {
+            if (len < (uint32_t)rec.max) {
+                uint32_t w[E6_STAGE_WORDS];
+#pragma unroll
+                for (int k = 0; k < 22; ++k) w[k] = sm.col[k * E6_BLOCK + threadIdx.x];
+                e6_pack_scalars(c.g, w + 22);
+                w[E6_STAGE_WORDS - 1] = (uint32_t)action;
+                uint4* d = (uint4*)(rec.stage + ((size_t)gi * rec.max + len) * E6_STAGE_WORDS);
+#pragma unroll
+                for (int q = 0; q < E6_STAGE_WORDS / 4; ++q) d[q] = make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
+            }
+            len++;
+        }
+        { E6DiceWord dice; dice.w = blk.x; e6_move(c, T, rules, action, dice); }
+        c.ply++;
+    }
+    if (REC) {
+        if (len && e6_status(c.g, rules) != AZ_STATUS_RUNNING) { e6_rec_flush(rec, gi, len, e6_status(c.g, rules)); len = 0; }
+        rec.len[gi] = len;
+    }
+    e6_store(c, sm, st, n, gi);
+    atomicAdd(&counters[0], (unsigned long long)n_plies);
+    if (games) atomicAdd(&counters[1], (unsigned long long)games);
+    if (draws) atomicAdd(&counters[2], (unsigned long long)draws);
 }
 
 // 108-byte host image (== r6_state of the oracle): army[42], owner[42], cards[6], pool[6], round u16, cur, card_sets, reinf,
@@ -280,6 +381,7 @@ struct az_env6 {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool timed = false;
     uint64_t generation = 0;    // bumped by reset / import: a search's staged samples of the games before it are abandoned
+    E6RecDev rec;               // recording of az_env6_play (az_env6_record); enabled iff rec.out != NULL
 };
 
 // accessors for az_mcts6.cu
@@ -340,6 +442,7 @@ extern "C" int az_env6_destroy(az_env6* e)
     if (!e) return AZ_OK;
     AzDeviceGuard guard(e->device);
     cudaFree(e->d_state); cudaFree(e->d_counters); cudaFree(e->d_img); cudaFree(e->d_action); cudaFree(e->d_status); cudaFree(e->d_valid); cudaFree(e->d_bad);
+    cudaFree(e->rec.stage); cudaFree(e->rec.len); cudaFree(e->rec.out); cudaFree(e->rec.count);
     if (e->ev0) cudaEventDestroy(e->ev0);
     if (e->ev1) cudaEventDestroy(e->ev1);
     delete e;
@@ -352,6 +455,7 @@ extern "C" int az_env6_reset(az_env6* e, uint64_t seed, void* stream)
     AzDeviceGuard guard(e->device);
     e->seed = seed;
     e->generation++;
+    if (e->rec.out) AZ_CUDA(cudaMemsetAsync(e->rec.len, 0, sizeof(uint32_t) * (size_t)e->n, (cudaStream_t)stream));   // staged samples go
     k_env6_reset<<<e6_grid(e->n), E6_BLOCK, 0, (cudaStream_t)stream>>>(e->d_state, e->n, seed, e->first_game);
     AZ_CUDA(cudaGetLastError());
     return AZ_OK;
@@ -441,6 +545,7 @@ extern "C" int az_env6_import(az_env6* e, const uint8_t* h_images, void* stream)
     AZ_CUDA(cudaMemcpyAsync(e->d_img, h_images, (size_t)e->n * E6_IMG, cudaMemcpyHostToDevice, s));
     AZ_CUDA(cudaMemsetAsync(e->d_bad, 0, sizeof(int), s));
     e->generation++;
+    if (e->rec.out) AZ_CUDA(cudaMemsetAsync(e->rec.len, 0, sizeof(uint32_t) * (size_t)e->n, s));                       // staged samples go
     k_env6_import<<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, e->d_img, e->d_bad);
     AZ_CUDA(cudaGetLastError());
     int bad = 0;
@@ -461,5 +566,84 @@ extern "C" int az_env6_counters(az_env6* e, az_counters6* h_out, int reset, void
     AZ_CUDA(cudaStreamSynchronize(s));
     h_out->steps = h[0]; h_out->games = h[1]; h_out->draws = h[2];
     for (int p = 0; p < E6_PLAYERS; ++p) h_out->wins[p] = h[3 + p];
+    return AZ_OK;
+}
+
+// ---- generated games (SIXPLAYER.md §6)
+extern "C" int az_env6_play(az_env6* e, const int* seat_kind, uint32_t record_seats, int n_plies, void* stream)
+{
+    AZ_REQUIRE(e != nullptr, "env is NULL");
+    AZ_REQUIRE(seat_kind != nullptr, "seat_kind is NULL");
+    AZ_REQUIRE(n_plies >= 0, "n_plies must be >= 0");
+    AZ_REQUIRE(record_seats < (1u << E6_PLAYERS), "record_seats has a bit above seat 5");
+    AZ_REQUIRE(record_seats == 0 || e->rec.out != nullptr, "record_seats != 0 needs az_env6_record first");
+    uint32_t script = 0;
+    for (int p = 0; p < E6_PLAYERS; ++p) {
+        AZ_REQUIRE(seat_kind[p] == AZ_AGENT6_RANDOM || seat_kind[p] == AZ_AGENT6_SCRIPT,
+                   "seat_kind entries must be AZ_AGENT6_RANDOM or AZ_AGENT6_SCRIPT (a searcher cannot play here)");
+        if (seat_kind[p] == AZ_AGENT6_SCRIPT) script |= 1u << p;
+    }
+    AzDeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    AZ_CUDA(cudaEventRecord(e->ev0, s));
+    // With recording enabled every call runs the recording kernel, record_seats == 0 included: a game with samples staged by an
+    // earlier call may end in this one, and its block must be queued (and its staging cleared) before the re-deal.
+    if (e->rec.out)
+        k_env6_play<true><<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, az_device_tables(), n_plies, e->seed, e->first_game,
+                                                           e6_rules(e->rules), script, record_seats, e->rec, e->d_counters);
+    else if (script == 0)                                // six random seats, nothing staged: exactly the rollout, at its speed
+        k_env6_rollout<<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, az_device_tables(), n_plies, e->seed, e->first_game,
+                                                         e6_rules(e->rules), e->d_counters);
+    else
+        k_env6_play<false><<<e6_grid(e->n), E6_BLOCK, 0, s>>>(e->d_state, e->n, az_device_tables(), n_plies, e->seed, e->first_game,
+                                                            e6_rules(e->rules), script, 0u, E6RecDev(), e->d_counters);
+    AZ_CUDA(cudaGetLastError());
+    AZ_CUDA(cudaEventRecord(e->ev1, s));
+    e->timed = true;
+    return AZ_OK;
+}
+
+extern "C" int az_env6_record(az_env6* e, size_t capacity_samples, int max_samples_per_game)
+{
+    AZ_REQUIRE(e != nullptr, "env is NULL");
+    AZ_REQUIRE(capacity_samples > 0 && max_samples_per_game > 0, "capacity_samples and max_samples_per_game must be positive");
+    AZ_REQUIRE(e->rec.out == nullptr, "recording is already enabled on this env");
+    AzDeviceGuard guard(e->device);
+    const size_t n = (size_t)e->n;
+    E6RecDev r;
+    cudaError_t ce = cudaMalloc(&r.stage, sizeof(uint32_t) * n * (size_t)max_samples_per_game * E6_STAGE_WORDS);
+    if (ce == cudaSuccess) ce = cudaMalloc(&r.len, sizeof(uint32_t) * n);
+    if (ce == cudaSuccess) ce = cudaMemset(r.len, 0, sizeof(uint32_t) * n);
+    if (ce == cudaSuccess) ce = cudaMalloc(&r.count, 2 * sizeof(unsigned long long));
+    if (ce == cudaSuccess) ce = cudaMemset(r.count, 0, 2 * sizeof(unsigned long long));
+    if (ce == cudaSuccess) ce = cudaMalloc(&r.out, capacity_samples * (size_t)S6_BYTES);
+    if (ce != cudaSuccess) {
+        cudaFree(r.stage); cudaFree(r.len); cudaFree(r.count); cudaFree(r.out);
+        az_set_error("az_env6_record: %s", cudaGetErrorString(ce));
+        return AZ_ERR_CUDA;
+    }
+    r.max = max_samples_per_game; r.cap = capacity_samples;
+    e->rec = r;                                        // rec.out != NULL: recording enabled
+    return AZ_OK;
+}
+
+extern "C" int az_env6_samples(az_env6* e, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream)
+{
+    AZ_REQUIRE(e && n_out, "NULL argument");
+    AZ_REQUIRE(e->rec.out != nullptr, "az_env6_record has not been called");
+    AzDeviceGuard guard(e->device);
+    cudaStream_t s = (cudaStream_t)stream;
+    unsigned long long h[2];
+    AZ_CUDA(cudaMemcpyAsync(h, e->rec.count, sizeof h, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
+    AZ_REQUIRE(h[0] <= e->rec.cap, "sample queue corrupted: committed count exceeds the capacity");
+    const size_t have = (size_t)h[0];                  // committed records: az_rec_reserve never reserves past the capacity
+    if (h_dropped) *h_dropped = h[1];
+    *n_out = have;
+    if (!h_records && have) return AZ_OK;              // size query; with an empty queue the call drains (resets the dropped count)
+    AZ_REQUIRE(max_records >= have, "h_records is too small: query the size with h_records = NULL first");
+    if (have) AZ_CUDA(cudaMemcpyAsync(h_records, e->rec.out, have * (size_t)S6_BYTES, cudaMemcpyDeviceToHost, s));
+    AZ_CUDA(cudaMemsetAsync(e->rec.count, 0, sizeof h, s));
+    AZ_CUDA(cudaStreamSynchronize(s));
     return AZ_OK;
 }

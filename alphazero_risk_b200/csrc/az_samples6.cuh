@@ -1,5 +1,5 @@
 // az_samples6.cuh — the six-player training-sample record (include/az_b200.h AZ_SAMPLE6_BYTES), shared by the recorder of the
-// six-player search (az_mcts6.cu) and the training unpack (az_nn_train.cu).  A format of this project: every field is 4-byte aligned,
+// six-player search (az_mcts6.cu), the recorder of generated games (az_env6.cu) and the training unpack (az_nn_train.cu).  A format of this project: every field is 4-byte aligned,
 // so both sides move whole 32-bit words.
 //   bytes 0..107    the position before the move as its 108-byte image (k_env6_export's layout; seat to move = byte 98)
 //   bytes 108..111  float value target of the seat to move there
@@ -60,4 +60,11 @@ __device__ __forceinline__ uint32_t s6_record_word(const uint32_t* __restrict__ 
     if (k == S6_VALUE / 4) return __float_as_uint(s6_value(status, (st[24] >> 16) & 0xffu));
     if (k < S6_STATUS / 4) return __float_as_uint(pi[k - S6_PI / 4]);
     return (uint32_t)(uint8_t)(int8_t)status;
+}
+
+// the same word for a sample whose policy target is one-hot at the played `action` (the generated games of az_env6_play)
+__device__ __forceinline__ uint32_t s6_onehot_record_word(const uint32_t* __restrict__ st, int action, int status, int k)
+{
+    if (k >= S6_PI / 4 && k < S6_STATUS / 4) return k - S6_PI / 4 == action ? __float_as_uint(1.0f) : 0u;
+    return s6_record_word(st, nullptr, status, k);
 }

@@ -447,6 +447,28 @@ AZ_API int az_arena6_play(az_arena6* arena, uint64_t first_game, uint64_t n_game
                           int8_t* h_status, uint32_t* h_plies, void* stream);
 /* the number of slots that held a game at each tick of the last az_arena6_play (*n_out = its ticks; h_active = NULL: size query) */
 AZ_API int az_arena6_active_slots(az_arena6* arena, uint32_t* h_active, size_t max_ticks, size_t* n_out);
+/* ---- six-player generated games (SIXPLAYER.md §6): scripted and random play recorded on the device as training records.
+   az_env6_play plays n_plies plies of every game with no host synchronisation: the seat to move, cur, plays by seat_kind[cur]
+   (AZ_AGENT6_RANDOM = az_env6_rollout's rule, AZ_AGENT6_SCRIPT = az_env6_script_actions' rule), both with the real-move dice of
+   (seed, first_game_id + slot, ply).  Finished games are counted and re-dealt in place on az_env6_rollout's schedule and the env
+   counters accumulate as there, so six random seats without recording are az_env6_rollout bit for bit.  Bit s of record_seats
+   (< 64) records every ply seat s plays, forced plies included: the image before the ply and the played action, staged per slot
+   until the game ends.  When a game ends, in any call on a recording env (record_seats = 0 included), its samples become
+   AZ_SAMPLE6_BYTES records (value target as above for the final status, policy target 1.0f at the played action and 0 elsewhere)
+   in one contiguous block of the queue, within the call in which it ended;
+   a game that is still running keeps its staged samples for the next call.  Recording changes no state, dice or counter.  Rejects
+   a seat_kind entry that is not RANDOM or SCRIPT, seat_kind == NULL, n_plies < 0, record_seats >= 64 and record_seats != 0 without
+   az_env6_record.  Only az_env6_play's own plies are staged: if az_env6_step, az_env6_rollout or a search moves the games in
+   between, a game's block holds only the plies az_env6_play played.  az_env6_reset and az_env6_import (so az_arena6_play too)
+   discard the staged samples.  Timed by az_env6_last_kernel_ms. */
+AZ_API int az_env6_play(az_env6* env, const int* seat_kind /*[6]*/, uint32_t record_seats, int n_plies, void* stream);
+/* enable recording in az_env6_play: max_samples_per_game staged samples per slot on the device (112 bytes each), an output queue of
+   capacity_samples records.  A game with more samples, or one that does not fit the queue, is dropped whole and counted.  Rejects
+   capacity_samples == 0, max_samples_per_game <= 0 and a second call */
+AZ_API int az_env6_record(az_env6* env, size_t capacity_samples, int max_samples_per_game);
+/* drains the queue of az_env6_play: the calling convention of az_selfplay6_samples (h_records = NULL: size query; a drain resets the
+   dropped count).  Rejected before az_env6_record */
+AZ_API int az_env6_samples(az_env6* env, uint8_t* h_records, size_t max_records, size_t* n_out, uint64_t* h_dropped, void* stream);
 
 /* ---------------------------------------------------------------- multi-GPU (SURVEY.md 8e): NCCL over NVLink / NVSwitch, never inside a search
    Games shard over GPUs by contiguous global id (first_game_id of az_env_create) and never migrate; every GPU holds a full copy of
